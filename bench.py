@@ -20,6 +20,8 @@ One "step" = one pass of the hot path over a batch of `--frames` synthetic frame
                         sample of the same frames, frame-parallel over the host cores (rank 0, N=1 only), and the
                         north_star acceptance list checked on one frame of the run (parity_check)
 `--impl reference` times only that CPU path (all host threads, bounded sample per step).
+`--dump-outputs DIR` writes what the device-resident arm computed in its last timed step as DIR/<name>.npy (see
+dump_outputs); the inputs depend only on the arguments, so two builds can be compared output for output.
 """
 import argparse
 import json
@@ -339,6 +341,31 @@ def single_frame_latency(ctx, pair, maps, K, Q, reps=10):
     return out
 
 
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(out_dir, fp, counts):
+    """`--dump-outputs`: the results of the pipeline's last run, as a caller of the timed path receives them, in float32
+    (images, depth, disparity, Steger centres) or float64 (counts, Simple centres, 3D points) .npy files under out_dir:
+      counts.npy                  3D points of every frame slot of the run
+      frameNNN_<key>.npy          FramePipeline.fetch(NNN): left_rect, depth, disp16 (int16 fixed point x16 as stored),
+                                  points_2d, points_3d
+    The full per-frame outputs of a whole step exceed 64 MB at the larger configs, so the frame slots are a fixed seeded
+    sample (the same for every run with the same arguments), as many as fit in 64 MB.  A c5 step runs the job as several
+    pipeline runs (chunks of --frames frames, all on the same resident inputs); the pipeline keeps only the last one, so
+    for c5 the files hold that last chunk, not the whole job."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = len(counts)
+    per_frame = (3 + 1 + 1) * 4 * W * H + (2 + 3) * 8 * MAX_POINTS + 5 * 128  # upper bound, .npy headers included
+    k = max(1, min(n, (DUMP_BYTES - 8 * n - 128) // per_frame))
+    slots = np.sort(np.random.default_rng(0).choice(n, size=k, replace=False))
+    np.save(os.path.join(out_dir, "counts.npy"), np.asarray(counts, np.float64))
+    for f in slots:
+        for key, a in fp.fetch(int(f)).items():
+            a = a if a.dtype in (np.float32, np.float64) else a.astype(np.float32)
+            np.save(os.path.join(out_dir, "frame%03d_%s.npy" % (f, key)), a)
+
+
 def run_gpu(args, rank, world, local_rank):
     import torch
     import torch.distributed as dist
@@ -432,6 +459,8 @@ def run_gpu(args, rank, world, local_rank):
         dist.all_reduce(nl, op=dist.ReduceOp.SUM)
     elapsed_ms, wall_max = float(el[0]), float(el[1])
     launches = int(nl[0])  # kernels of libl3d.so launched inside the timed region, summed over ranks
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, fp, counts)
 
     # ---- end-to-end arm (host buffers through the C ABI) ----------------------------------------
     for _ in range(2):
@@ -558,7 +587,13 @@ def main():
     ap.add_argument("--distinct", type=int, default=8, help="distinct synthetic frames rendered per rank")
     ap.add_argument("--lanes", type=int, default=0, help="frames in flight per GPU (streams; default per config: 28 = four lane sets of 7 frames)")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the outputs of the last timed step (rank 0, GPU arm) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU arm's outputs; the reference arm keeps none")
     select_config(args.config)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

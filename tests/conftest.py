@@ -23,9 +23,24 @@ def golden_synth():
     return dict(np.load(os.path.join(GOLDEN, "synth_c1.npz")))
 
 
+def _load_golden(*names):
+    """one dict of every array in tests/golden/<name>.npz (the real pairs are stored one per file)"""
+    out = {}
+    for n in names:
+        out.update(np.load(os.path.join(GOLDEN, n + ".npz")))
+    return out
+
+
 @pytest.fixture(scope="session")
 def golden_real():
-    return dict(np.load(os.path.join(GOLDEN, "real_pair.npz")))
+    """the shipped calibration of the real rig and two of its pairs (a, b) in full"""
+    return _load_golden("real_rig", "real_pair_a", "real_pair_b")
+
+
+@pytest.fixture(scope="session")
+def golden_real_more():
+    """four more real pairs (c-f): inputs, int16 disparity, CRC32s of the rectified views and the depth image"""
+    return _load_golden("real_pair_c", "real_pair_d", "real_pair_e", "real_pair_f")
 
 
 @pytest.fixture(scope="session")

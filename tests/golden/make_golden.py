@@ -120,8 +120,12 @@ def main():
             dep[dep < 0] = 0; dep[dep > 10] = 0; dep[dispf <= 0] = 0
         real.update({"frame_" + tag: combined, "lrect_" + tag: lrect, "rrect_" + tag: rrect, "disp16_" + tag: d16,
                      "depth_" + tag: dep})
-    np.savez_compressed(os.path.join(HERE, "real_pair.npz"), **real)
-    for f in ("synth_c1.npz", "real_pair.npz"):
+    # one file per pair (and the calibration apart) keeps every golden file under 1 MB
+    files = {"real_pair_" + t + ".npz": {k: v for k, v in real.items() if k.endswith("_" + t)} for t in ("a", "b")}
+    files["real_rig.npz"] = {k: v for k, v in real.items() if not k.endswith(("_a", "_b"))}
+    for f, arrays in files.items():
+        np.savez_compressed(os.path.join(HERE, f), **arrays)
+    for f in ["synth_c1.npz"] + sorted(files):
         print(f, os.path.getsize(os.path.join(HERE, f)) // 1024, "KiB")
 
 

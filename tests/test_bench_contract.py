@@ -49,6 +49,49 @@ def test_reference_arm_line_matches_the_gpu_arm():
     assert ref["cpu_baseline"]["value"] == ref["value"] and ref["gpu_launches"] == 0
 
 
+@pytest.mark.parametrize("config", ["c1", "c4"])
+def test_dump_outputs_within_budget(tmp_path, config):
+    """--dump-outputs with every frame at max_points (a stand-in for the pipeline whose values depend on the frame slot):
+    float32 / float64 files only, at most 64 MB in all, the same frame sample on every run, counts.npy the counts handed
+    in, and frameNNN_<key>.npy the values fetch(NNN) returned for <key>."""
+    import re
+    import numpy as np
+    import bench
+
+    class Pipe:
+        def fetch(self, f):
+            W, H, m = bench.W, bench.H, bench.MAX_POINTS
+            i = np.arange(W * H, dtype=np.int64).reshape(H, W)
+            xy = np.arange(2 * m).reshape(m, 2) * 0.25 + f
+            return dict(left_rect=((i[..., None] * 3 + np.arange(3) + f) % 256).astype(np.uint8),
+                        depth=(i % 977 + f).astype(np.float32) / 7, disp16=((i * 37 + f) % 65536 - 32768).astype(np.int16),
+                        points_2d=xy if config == "c1" else xy.astype(np.float32),   # Simple: float64, Steger: float32
+                        points_3d=np.arange(3 * m).reshape(m, 3) * 0.125 - f)
+
+    bench.select_config(config)
+    counts = (np.arange(bench.CFG["frames"]) * 7919 % 20001).astype(np.int32)
+    listings = []
+    for run in ("a", "b"):
+        d = tmp_path / run
+        bench.dump_outputs(str(d), Pipe(), counts)
+        files = sorted(os.listdir(d))
+        assert sum(os.path.getsize(d / f) for f in files) <= 64 * 10 ** 6
+        assert np.array_equal(np.load(d / "counts.npy"), counts) and np.load(d / "counts.npy").dtype == np.float64
+        slots = set()
+        for f in files:
+            if f == "counts.npy":
+                continue
+            m = re.fullmatch(r"frame(\d{3})_(\w+)\.npy", f)
+            assert m, f
+            slots.add(int(m.group(1)))
+            got, want = np.load(d / f), Pipe().fetch(int(m.group(1)))[m.group(2)]
+            assert got.dtype == (np.float64 if want.dtype == np.float64 else np.float32), f
+            assert got.shape == want.shape and np.array_equal(got, want), f
+        assert slots and len(files) == 1 + 5 * len(slots)
+        listings.append(files)
+    assert listings[0] == listings[1]
+
+
 def test_reference_arm_other_ranks_exit_quietly():
     env = dict(os.environ, RANK="1", LOCAL_RANK="1", WORLD_SIZE="2", MASTER_ADDR="127.0.0.1", MASTER_PORT="29533")
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2", "--steps", "1",

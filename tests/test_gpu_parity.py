@@ -93,13 +93,12 @@ def test_colour_arithmetic_full_cube(ctx):
         eq(ctx.colour_mask(img, boxes[0][0], boxes[0][1], 200), want, "config.py colour + brightness mask")
 
 
-def test_sgbm_more_real_pairs(ctx, golden_real):
-    """Four more of the reference's 28 calibration pairs (tests/golden/real_pairs.npz from the REAL camera class): the
+def test_sgbm_more_real_pairs(ctx, golden_real, golden_real_more):
+    """Four more of the reference's 28 calibration pairs (tests/golden/real_pair_[c-f].npz from the REAL camera class): the
     rectified views (CRC32 of cv2.remap's output), the as-constructed 3WAY matcher's int16 disparity and the depth image."""
-    import os
     import zlib
     g = golden_real
-    more = dict(np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "real_pairs.npz")))
+    more = golden_real_more
     size = (320, 240)
     R1, R2, P1, P2, Q, _, _ = cv2.stereoRectify(g["K_left"], g["dist_left"], g["K_right"], g["dist_right"], size,
                                                 g["R"], g["T"], flags=cv2.CALIB_ZERO_DISPARITY, alpha=0)

@@ -1,7 +1,6 @@
 """Pin the oracle's C restatement (oracle/csrc) against the installed cv2 binary -- the library the
 reference calls on its hot path (SURVEY 8c).  Bit-exact for every integer stage."""
 import cv2
-import os
 
 import numpy as np
 import pytest
@@ -245,48 +244,41 @@ def test_wls_oracle_variants_switch_one_point_each():
     assert not np.array_equal(outs[2], outs[8])
 
 
-REF_IMAGES = "/root/reference/calibration_images"
-
-
-@pytest.mark.skipif(not os.path.isdir(REF_IMAGES), reason="the reference tree is only present in the build container")
-def test_oracle_on_all_28_real_pairs(golden_real):
-    """SURVEY 8c pin (ii): every one of the reference's 28 calibration pairs, rectified with the shipped calibration -- the
-    oracle's remap / gray / StereoSGBM restatements against the cv2 binary (as constructed: SGBM_3WAY, 64 / 5; and the
-    WLS-mutated left + right matcher pair in MODE_HH on every fourth pair), and the committed goldens against what the
-    REAL camera class produces today."""
-    import sys
+def test_oracle_on_stored_real_pairs(golden_real, golden_real_more):
+    """SURVEY 8c pin (ii): the six of the reference's 28 calibration pairs the goldens store (real_pair_[a-f].npz),
+    rectified with the shipped calibration -- the oracle's remap / gray / StereoSGBM restatements against the cv2 binary
+    (as constructed: SGBM_3WAY, 64 / 5; and the WLS-mutated left + right matcher pair in MODE_HH), and the goldens the
+    REAL camera class produced against what the same cv2 calls produce today."""
     import zlib
-    from oracle import cref, ref_ops
     g = golden_real
     size = (320, 240)
     R1, R2, P1, P2, Q, _, _ = cv2.stereoRectify(g["K_left"], g["dist_left"], g["K_right"], g["dist_right"], size,
                                                 g["R"], g["T"], flags=cv2.CALIB_ZERO_DISPARITY, alpha=0)
     mlx, mly = cv2.initUndistortRectifyMap(g["K_left"], g["dist_left"], R1, P1, size, cv2.CV_32FC1)
     mrx, mry = cv2.initUndistortRectifyMap(g["K_right"], g["dist_right"], R2, P2, size, cv2.CV_32FC1)
-    names = sorted(os.listdir(os.path.join(REF_IMAGES, "left")))
-    assert len(names) == 28
     base, mut, right = ref_ops.sgbm_param_sets(64, 5, 2)
     _, mut_hh, right_hh = ref_ops.sgbm_param_sets(64, 5, 1)
-    more = dict(np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "real_pairs.npz")))
-    by_index = {int(more["index_" + t]): t for t in ("c", "d", "e", "f")}
-    for i, name in enumerate(names):
-        l = cv2.imread(os.path.join(REF_IMAGES, "left", name))
-        r = cv2.imread(os.path.join(REF_IMAGES, "right", name.replace("left_", "right_")))
+    more = golden_real_more
+    for t in ("a", "b", "c", "d", "e", "f"):
+        src = g if t in ("a", "b") else more
+        frame = src["frame_" + t]
+        l, r = np.ascontiguousarray(frame[:, :320]), np.ascontiguousarray(frame[:, 320:])
         lrect, rrect = cv2.remap(l, mlx, mly, cv2.INTER_LINEAR), cv2.remap(r, mrx, mry, cv2.INTER_LINEAR)
-        assert np.array_equal(cref.remap_bilinear(l, mlx, mly), lrect), name
-        assert np.array_equal(cref.remap_bilinear(r, mrx, mry), rrect), name
+        assert np.array_equal(cref.remap_bilinear(l, mlx, mly), lrect), t
+        assert np.array_equal(cref.remap_bilinear(r, mrx, mry), rrect), t
         lg, rg = cv2.cvtColor(lrect, cv2.COLOR_BGR2GRAY), cv2.cvtColor(rrect, cv2.COLOR_BGR2GRAY)
-        assert np.array_equal(cref.bgr2gray(lrect), lg)
+        assert np.array_equal(cref.bgr2gray(lrect), lg) and np.array_equal(cref.bgr2gray(rrect), rg), t
         want = cv2.StereoSGBM_create(**base).compute(lg, rg)
-        assert np.array_equal(cref.sgbm_compute(lg, rg, **base), want), name
-        if i % 4 == 0:
-            assert np.array_equal(cref.sgbm_compute(lg, rg, **mut_hh), cv2.StereoSGBM_create(**mut_hh).compute(lg, rg)), name
-            assert np.array_equal(cref.sgbm_compute(rg, lg, **right_hh), cv2.StereoSGBM_create(**right_hh).compute(rg, lg)), name
-        if i in by_index:  # the committed golden of this pair is what the pipeline above produces
-            t = by_index[i]
-            assert np.array_equal(more["frame_" + t], np.hstack([l, r]))
-            assert np.array_equal(more["disp16_" + t], want)
-            assert int(more["lrect_crc_" + t]) == zlib.crc32(lrect.tobytes())
+        assert np.array_equal(cref.sgbm_compute(lg, rg, **base), want), t
+        assert np.array_equal(cref.sgbm_compute(lg, rg, **mut_hh), cv2.StereoSGBM_create(**mut_hh).compute(lg, rg)), t
+        assert np.array_equal(cref.sgbm_compute(rg, lg, **right_hh), cv2.StereoSGBM_create(**right_hh).compute(rg, lg)), t
+        # the stored golden of this pair is what the calls above produce
+        assert np.array_equal(src["disp16_" + t], want), t
+        if t in ("a", "b"):
+            assert np.array_equal(src["lrect_" + t], lrect) and np.array_equal(src["rrect_" + t], rrect), t
+        else:
+            assert int(src["lrect_crc_" + t]) == zlib.crc32(lrect.tobytes()), t
+            assert int(src["rrect_crc_" + t]) == zlib.crc32(rrect.tobytes()), t
 
 
 def test_stereo_rectify_vs_cv2(golden_real):
