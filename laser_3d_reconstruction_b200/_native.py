@@ -74,7 +74,7 @@ RECON_PLANE, RECON_DEPTH, RECON_DISPARITY, RECON_DISPARITY_MEDIAN = 0, 1, 2, 3
 EXPORTS = (
     "l3d_ctx_create l3d_ctx_destroy l3d_last_error l3d_sync l3d_device_count l3d_version l3d_launch_count "
     "l3d_set_rectify_maps l3d_init_undistort_rectify_map l3d_remap_gray l3d_bgr2gray l3d_sgbm_compute l3d_sgbm_compute_pair l3d_sgbm_debug l3d_sgbm_volume_rows "
-    "l3d_sgbm_vgroup_time l3d_bm_compute l3d_median3_s16 l3d_filter_speckles l3d_wls_filter l3d_disp_to_depth l3d_compute_depth "
+    "l3d_sgbm_vgroup_time l3d_bm_compute l3d_median3_s16 l3d_filter_speckles l3d_wls_filter l3d_fgs_solve l3d_disp_to_depth l3d_compute_depth "
     "l3d_simple_extract l3d_colour_mask l3d_steger_extract l3d_reconstruct l3d_laser_depth_map l3d_voxel_downsample l3d_statistical_outlier_removal l3d_pipeline_create l3d_pipeline_destroy "
     "l3d_pipeline_set_maps l3d_pipeline_run_dev l3d_pipeline_run_host l3d_pipeline_fetch l3d_pipeline_fetch_points l3d_pipeline_points_needed "
     "l3d_pipeline_pack_points_dev l3d_pipeline_launch_count l3d_pipeline_graph_replays l3d_pipeline_last_ms l3d_pipeline_set_timing l3d_pipeline_kernel_time "
@@ -321,6 +321,19 @@ class Context:
         self.check(self.lib.l3d_wls_filter(self.h, C.byref(params), _ptr(dl), _ptr(dr), _ptr(guide), W, H, _ptr(out),
                                            _ptr(conf)), "l3d_wls_filter")
         return (out, conf) if want_conf else out
+
+    def fgs_solve(self, num, den, ch, cv, lam=8000.0, iters=3, variant=0, solver=WLS_SOLVER_PARALLEL):
+        """The FGS passes of wls_filter alone (include/l3d.h: l3d_fgs_solve) on h x w float32 planes: num / den solved
+        with row weights ch and column weights cv.  -> (num, den, parallel_used)"""
+        num, den = _arr(num, np.float32).copy(), _arr(den, np.float32).copy()
+        ch, cv = _arr(ch, np.float32), _arr(cv, np.float32)
+        if num.ndim != 2 or not (num.shape == den.shape == ch.shape == cv.shape):
+            raise ValueError("fgs_solve expects four float32 planes of equal 2-D shape")
+        H, W = num.shape
+        par = C.c_int(-1)
+        self.check(self.lib.l3d_fgs_solve(self.h, int(solver), int(variant), C.c_double(lam), int(iters), _ptr(ch), _ptr(cv),
+                                          W, H, _ptr(num), _ptr(den), C.byref(par)), "l3d_fgs_solve")
+        return num, den, bool(par.value)
 
     def disp_to_depth(self, disp16, Q=None):
         disp16 = _arr(disp16, np.int16)

@@ -498,6 +498,31 @@ int l3d_wls_filter(l3d_ctx* ctx, const l3d_wls_params* p, const int16_t* dl, con
     API_END(ctx)
 }
 
+int l3d_fgs_solve(l3d_ctx* ctx, int solver, int variant, double lambda, int iters, const float* ch, const float* cv,
+                  int w, int h, float* num, float* den, int* parallel_used) {
+    API_BEGIN(ctx)
+    NEED(ctx, ch && cv && num && den && w > 0 && h > 0, "fgs arguments");
+    NEED(ctx, iters >= 1 && iters <= 3, "fgs iters (1..3)");
+    CK(ctx, cudaSetDevice(ctx->device));
+    Lane& L = ctx->lane;
+    size_t n = (size_t)w * h;
+    // the planes dev_wls solves in
+    float *a = L.get<float>(S_WLS_A, n), *b = L.get<float>(S_WLS_B, n), *D = L.get<float>(S_WLS_C, n);
+    float *wh = L.get<float>(S_WLS_H, n), *wv = L.get<float>(S_WLS_I, n);
+    RC(h2d(ctx, a, num, n * 4));
+    RC(h2d(ctx, b, den, n * 4));
+    RC(h2d(ctx, wh, ch, n * 4));
+    RC(h2d(ctx, wv, cv, n * 4));
+    bool par = false;
+    RC(dev_fgs(L, solver, variant, lambda, iters, wh, wv, w, h, a, b, D, &par));
+    RC(d2h(ctx, num, a, n * 4));
+    RC(d2h(ctx, den, b, n * 4));
+    RC(finish(ctx));
+    if (parallel_used) *parallel_used = par ? 1 : 0;
+    return L3D_OK;
+    API_END(ctx)
+}
+
 int l3d_disp_to_depth(l3d_ctx* ctx, const int16_t* disp16, int W, int H, const double* Q, float* depth) {
     API_BEGIN(ctx)
     NEED(ctx, disp16 && depth && W > 0 && H > 0, "depth arguments");

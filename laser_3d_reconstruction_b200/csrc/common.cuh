@@ -160,6 +160,9 @@ int dev_speckles(Lane& L, int16_t* img, int W, int H, int newVal, int maxSize, i
 
 int dev_wls(Lane& L, const l3d_wls_params& p, const int16_t* dl, const int16_t* dr,
             const uint8_t* guide, int W, int H, int16_t* out, float* conf_out);
+// the FGS passes of dev_wls: `iters` x (row solves weighted by ch, column solves weighted by cv) on num/den in place
+int dev_fgs(Lane& L, int solver, int variant, double lambda, int iters, const float* ch, const float* cv, int w, int h,
+            float* num, float* den, float* Dscr, bool* parallel_used);
 int dev_depth(Lane& L, const int16_t* disp16, int W, int H, const double* Q, float* depth);
 
 int dev_simple(Lane& L, const uint8_t* bgr, int W, int H, const int* lo, const int* hi, int thr,

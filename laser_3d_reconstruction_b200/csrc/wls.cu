@@ -498,6 +498,33 @@ static int wls_lut(Lane& L, double sigma, float** out) {
     return L3D_OK;
 }
 
+// The FGS passes of the WLS filter (dev_wls; l3d_fgs_solve runs them alone): `iters` iterations of (row solves with
+// weights ch, column solves with weights cv) on num/den in place; Dscr (w x h) is scratch of the serial kernels.
+// solver: 0 = partitioned parallel solves (default), 1 = serial solves in the oracle's operation order (bit-identical
+// to oracle/csrc/orc_wls.c); L3D_FGS_SERIAL=1 forces the serial form everywhere, and so do lines longer than the
+// parallel kernels can stage in shared memory (w > 2552 or h > 1248) or shorter than 2.
+int dev_fgs(Lane& L, int solver, int variant, double lambda, int iters, const float* ch, const float* cv, int w, int h,
+            float* num, float* den, float* Dscr, bool* parallel_used) {
+    float lam = (float)lambda;
+    static const bool force_serial = getenv("L3D_FGS_SERIAL") && atoi(getenv("L3D_FGS_SERIAL")) > 0;
+    const size_t smr = fgsp_smem_bytes(FGSP_ROWS, w), smc = (size_t)FGSP_COLS * 5 * (((h + 31) / 32) * 32 + 4) * sizeof(float);
+    const bool parallel = !force_serial && solver != 1 && smr <= 200 * 1024 && smc <= 200 * 1024 && w >= 2 && h >= 2;
+    *parallel_used = parallel;
+    if (parallel) {
+        L3D_CHECK(L, cudaFuncSetAttribute(fgs_rows_par_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smr));
+        L3D_CHECK(L, cudaFuncSetAttribute(fgs_cols_par_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smc));
+    }
+    for (int it = 0; it < iters; it++) {
+        if (parallel) L3D_LAUNCH(L, fgs_rows_par_kernel, cdiv(h, FGSP_ROWS), FGSP_ROWS * 32, smr, num, den, ch, w, h, lam);
+        else L3D_LAUNCH(L, fgs_rows_kernel, cdiv(h, FGS_LPW), 32, 0, num, den, ch, Dscr, w, h, lam);
+        if (variant & L3D_WLS_LAMBDA_PER_PASS) lam *= 0.25f;
+        if (parallel) L3D_LAUNCH(L, fgs_cols_par_kernel, cdiv(w, FGSP_COLS), FGSP_COLS * 32, smc, num, den, cv, w, h, lam);
+        else L3D_LAUNCH(L, fgs_cols_kernel<FGS_CPW>, cdiv(w, FGS_CPW), 32, 0, num, den, cv, Dscr, w, h, lam);
+        lam *= 0.25f;
+    }
+    return L3D_OK;
+}
+
 int dev_wls(Lane& L, const l3d_wls_params& p, const int16_t* dl, const int16_t* dr, const uint8_t* guide,
             int W, int H, int16_t* out, float* conf_out) {
     int x0 = std::max(0, p.min_disp + p.num_disp);
@@ -524,25 +551,9 @@ int dev_wls(Lane& L, const l3d_wls_params& p, const int16_t* dl, const int16_t* 
     float *num = aL, *den = bL;
     L3D_LAUNCH(L, wls_lrc_kernel, g, 128, 0, dl, dr, guide, lut, W, x0, w, h, p.lrc_thresh, (p.variant & L3D_WLS_LRC_OUTSIDE_ZERO) ? 1 : 0, cl, cr, conf, num, den, ch,
                cv);
-    float lam = (float)p.lambda;
-    float* Dscr = aR;  // aR/bR are free as well: elimination factors of the current pass
-    // solver: 0 = partitioned parallel solves (default), 1 = serial solves in the oracle's operation order (bit-identical
-    // to oracle/csrc/orc_wls.c); L3D_FGS_SERIAL=1 forces the serial form everywhere
-    static const bool force_serial = getenv("L3D_FGS_SERIAL") && atoi(getenv("L3D_FGS_SERIAL")) > 0;
-    const size_t smr = fgsp_smem_bytes(FGSP_ROWS, w), smc = (size_t)FGSP_COLS * 5 * (((h + 31) / 32) * 32 + 4) * sizeof(float);
-    const bool parallel = !force_serial && p.solver != 1 && smr <= 200 * 1024 && smc <= 200 * 1024 && w >= 2 && h >= 2;
-    if (parallel) {
-        L3D_CHECK(L, cudaFuncSetAttribute(fgs_rows_par_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smr));
-        L3D_CHECK(L, cudaFuncSetAttribute(fgs_cols_par_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smc));
-    }
-    for (int it = 0; it < 3; it++) {
-        if (parallel) L3D_LAUNCH(L, fgs_rows_par_kernel, cdiv(h, FGSP_ROWS), FGSP_ROWS * 32, smr, num, den, ch, w, h, lam);
-        else L3D_LAUNCH(L, fgs_rows_kernel, cdiv(h, FGS_LPW), 32, 0, num, den, ch, Dscr, w, h, lam);
-        if (p.variant & L3D_WLS_LAMBDA_PER_PASS) lam *= 0.25f;
-        if (parallel) L3D_LAUNCH(L, fgs_cols_par_kernel, cdiv(w, FGSP_COLS), FGSP_COLS * 32, smc, num, den, cv, w, h, lam);
-        else L3D_LAUNCH(L, fgs_cols_kernel<FGS_CPW>, cdiv(w, FGS_CPW), 32, 0, num, den, cv, Dscr, w, h, lam);
-        lam *= 0.25f;
-    }
+    bool parallel = false;
+    rc = dev_fgs(L, p.solver, p.variant, p.lambda, 3, ch, cv, w, h, num, den, aR, &parallel);  // aR is free as well: scratch D
+    if (rc != L3D_OK) return rc;
     L3D_LAUNCH(L, wls_finalize_kernel, dim3(cdiv(W, 128), H), 128, 0, num, den, conf, W, H, x0, w, outside, out, conf_out);
     L.t_end("wls");
     return L3D_OK;

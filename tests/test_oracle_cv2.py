@@ -395,7 +395,6 @@ def test_wls_solver_against_an_independent_f64_solve():
     weighted graph Laplacian, weights exp(-|dg| / sigma_color), lambda_t = lambda / 4^t) give the oracle's int16 output
     within 1 LSB everywhere and identically on > 99 % of the ROI.  (What stays unpinned is ximgproc's choice of these
     ingredients, not the arithmetic.)"""
-    from scipy.linalg import solve_banded
     W, H, D = 150, 33, 48
     lam0, sigma = 8000.0, 1.5
     for seed in (3, 8):
@@ -406,31 +405,31 @@ def test_wls_solver_against_an_independent_f64_solve():
         wh = np.zeros((h, w)); wv = np.zeros((h, w))
         wh[:, :-1] = np.exp(-np.abs(g[:, :-1] - g[:, 1:]) / sigma)
         wv[:-1, :] = np.exp(-np.abs(g[:-1, :] - g[1:, :]) / sigma)
-
-        def solve_lines(u, wts, lam):   # u: (lines, n), wts[:, j] couples j and j + 1
-            res = np.empty_like(u)
-            n = u.shape[1]
-            for i in range(u.shape[0]):
-                ab = np.zeros((3, n))
-                ab[0, 1:] = -lam * wts[i, :-1]
-                ab[2, :-1] = -lam * wts[i, :-1]
-                ab[1] = 1.0
-                ab[1, :-1] += lam * wts[i, :-1]
-                ab[1, 1:] += lam * wts[i, :-1]
-                res[i] = solve_banded((1, 1), ab, u[i])
-            return res
-
-        def fgs(u):
-            lam = lam0
-            for _ in range(3):
-                u = solve_lines(u, wh, lam)
-                u = solve_lines(u.T.copy(), wv.T.copy(), lam).T.copy()
-                lam *= 0.25
-            return u
         c = conf[:, x0:].astype(np.float64)
-        num, den = fgs(c * dl[:, x0:].astype(np.float64)), fgs(c)
+        num, den = ref_ops.fgs_f64(c * dl[:, x0:].astype(np.float64), c, -wh, -wv, lam0, 3)
         want = np.clip(np.rint(num / (den + 1e-43)), -32768, 32767)
         got = out[:, x0:].astype(np.float64)
         diff = np.abs(got - want)
         assert diff.max() <= 1, diff.max()
         assert (diff == 0).mean() > 0.99, (diff == 0).mean()
+
+
+@pytest.mark.parametrize("variant", [0, 1, 15])
+def test_fgs_f32_restatement_reproduces_the_oracle(variant):
+    """ref_ops.fgs_f32_serial (numpy float32, vectorised over lines) repeats orc_wls.c's fgs_solve operation for operation:
+    fed the oracle's own confidence map and guide weights, it gives the oracle's int16 output bit for bit, under either
+    lambda schedule.  The GPU solver tests measure the serial f32 error with it, so it must not be an unchecked helper."""
+    lam0, sigma = 8000.0, 1.5
+    for (W, H, D), seed in (((150, 33, 48), 3), ((97, 40, 16), 8)):
+        dl, dr, guide = wls_case(W, H, D, seed)
+        out, conf = cref.wls_filter(dl, dr, guide, 0, D, 3, lam0, sigma, want_conf=True, variant=variant)
+        x0 = D
+        c = conf[:, x0:]
+        ch, cv = ref_ops.wls_weights(guide[:, x0:], sigma)
+        num, den = ref_ops.fgs_f32_serial(c * dl[:, x0:].astype(np.float32), c, ch, cv, lam0, 3, variant)
+        with np.errstate(over="ignore", invalid="ignore"):
+            v = num * (np.float32(1) / (den + np.float32(1e-43)))
+        q = np.where(np.abs(v) < np.float32(2 ** 31), np.rint(np.nan_to_num(v)), -32768)
+        got = np.clip(q, -32768, 32767).astype(np.int16)
+        assert np.array_equal(got, out[:, x0:]), "%d of %d pixels differ" % ((got != out[:, x0:]).sum(), got.size)
+        assert (out[:, :x0] == -16).all()
