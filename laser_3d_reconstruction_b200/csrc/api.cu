@@ -577,17 +577,14 @@ static int depth_back(Lane& L, const l3d_depth_config& cfg, DepthRuns& dr, int W
     const uint8_t* gl = L.get<uint8_t>(S_GRAY_L, n);
     int16_t* dl = L.get<int16_t>(S_DISP_L, n);
     RC(sgbm_back(L, dr.left, dl, nullptr));
-    const int16_t* df = dl;
+    const double* Q = cfg.use_Q ? cfg.Q : nullptr;
     if (dr.has_right) {
         int16_t* drr = L.get<int16_t>(S_DISP_R, n);
         RC(sgbm_back(L, dr.right, drr, nullptr));
-        RC(dev_wls(L, cfg.wls, dl, drr, gl, W, H, disp_f, nullptr));
-        df = disp_f;
-    } else {
-        L3D_CHECK(L, cudaMemcpyAsync(disp_f, dl, n * 2, cudaMemcpyDeviceToDevice, L.stream));
+        return dev_wls(L, cfg.wls, dl, drr, gl, W, H, disp_f, nullptr, depth, Q);  // the filter's last kernel writes the depth too
     }
-    RC(dev_depth(L, df, W, H, cfg.use_Q ? cfg.Q : nullptr, depth));
-    return L3D_OK;
+    L3D_CHECK(L, cudaMemcpyAsync(disp_f, dl, n * 2, cudaMemcpyDeviceToDevice, L.stream));
+    return dev_depth(L, dl, W, H, Q, depth);
 }
 
 // get_frames() depth path on device buffers (camera/single_usb_stereo_camera.py:311-359), one frame start to finish

@@ -158,8 +158,9 @@ int dev_bm(Lane& L, const l3d_bm_params& p, const uint8_t* left, const uint8_t* 
 int dev_median3(Lane& L, const int16_t* src, int W, int H, int16_t* dst);
 int dev_speckles(Lane& L, int16_t* img, int W, int H, int newVal, int maxSize, int maxDiff);
 
+// depth != nullptr: the last kernel of the filter also writes the depth of the filtered disparity (dev_depth's arithmetic)
 int dev_wls(Lane& L, const l3d_wls_params& p, const int16_t* dl, const int16_t* dr,
-            const uint8_t* guide, int W, int H, int16_t* out, float* conf_out);
+            const uint8_t* guide, int W, int H, int16_t* out, float* conf_out, float* depth = nullptr, const double* Q = nullptr);
 // the FGS passes of dev_wls: `iters` x (row solves weighted by ch, column solves weighted by cv) on num/den in place
 int dev_fgs(Lane& L, int solver, int variant, double lambda, int iters, const float* ch, const float* cv, int w, int h,
             float* num, float* den, float* Dscr, bool* parallel_used);

@@ -11,7 +11,8 @@
 //   wls_lrc                    LR-consistency confidence, FGS right-hand sides, guide weights
 //   fgs_hpass / fgs_vpass      3 x (row solves, column solves), Thomas algorithm, one line per
 //                              thread, numerator and denominator solved together
-//   wls_finalize               num/(den+eps) -> int16 (half-even, saturated)
+//   fgs_*_par                  the same solves partitioned over the 32 lanes of a warp (default)
+//   wls_finalize               num/(den+eps) -> int16 (half-even, saturated); in the frame pipeline also the depth
 #include "common.cuh"
 
 namespace l3d {
@@ -330,13 +331,17 @@ __global__ void __launch_bounds__(32) fgs_rows_kernel(float* num, float* den, co
 //   reduced system in the chunk ends u_e (one row per lane: row e with u_{s'} of the next chunk replaced by that
 //               chunk's row-s form), solved across the lanes by parallel cyclic reduction with warp shuffles
 //   back sweep  (e-1 .. s): u_j = g_j - AB_j u_{s-1} - D_j u_{j+1}
-// Lines are staged in shared memory (coalesced in and out); a lane walks its chunk with an odd element stride
-// between lanes, so every step of a sweep hits 32 different banks.
-constexpr int FGSP_ROWS = 4;   // lines (= warps) per CTA in the row pass
-constexpr int FGSP_COLS = 8;   // lines per CTA in the column pass: 8 adjacent columns = one 32-byte sector per image row
+// A line lives in shared memory as four planes: weights (overwritten by D in the down sweep), g1, g2 and AB; a lane
+// walks its chunk with an odd element stride between lanes, so every step of a sweep hits 32 different banks.  The
+// kernels stage their lines with asynchronous copies issued all at once (one bulk copy per row plane, or one cp.async
+// per element) instead of a loop of dependent loads: the solves do little arithmetic, and what they cost the frame
+// pipeline is the SMs they hold (an SM that hosts an FGS CTA is closed to the matcher kernels, which each need a whole
+// register file) times how long they hold them.
+constexpr int FGSP_ROWS = 4;        // lines (= warps) per CTA in the row pass
+constexpr int FGSP_W_MAX = 2552;    // longest row / column the parallel kernels solve; longer lines take the serial kernels
+constexpr int FGSP_H_MAX = 1248;
 
-__device__ __forceinline__ void fgsp_solve_line(const float* __restrict__ wgt, float* g1, float* g2, float* Dd, float* AB,
-                                                int n, float lam, int lane) {
+__device__ __forceinline__ void fgsp_solve_line(float* wd, float* g1, float* g2, float* AB, int n, float lam, int lane) {
     int m = (n + 31) / 32;
     if (m < 2) m = 2;
     m |= 1;                                            // odd chunk length: lane stride == m mod 32 is odd
@@ -346,7 +351,7 @@ __device__ __forceinline__ void fgsp_solve_line(const float* __restrict__ wgt, f
     // ---- up sweep: row s in terms of (u_{s-1}, u_s, u_e)
     float E = 0.f, G = -1.f, H1 = 0.f, H2 = 0.f;
     for (int j = e - 1; j >= s && act; j--) {
-        const float c = __fmul_rn(lam, wgt[j]), a = j > 0 ? __fmul_rn(lam, wgt[j - 1]) : 0.f;
+        const float c = __fmul_rn(lam, wd[j]), a = j > 0 ? __fmul_rn(lam, wd[j - 1]) : 0.f;
         const float b = 1.0f - a - c;
         const float ib = __frcp_rn(b - c * E);
         E = a * ib;
@@ -354,17 +359,21 @@ __device__ __forceinline__ void fgsp_solve_line(const float* __restrict__ wgt, f
         H1 = (g1[j] - c * H1) * ib;
         H2 = (g2[j] - c * H2) * ib;
     }
-    // ---- down sweep
+    // ---- down sweep: D_j replaces w_j; a_j = lam w_{j-1} is carried from the previous step.  The first a is the
+    // previous chunk's last weight, which its lane overwrites: read it before any lane writes D.
+    float a = act && s > 0 ? __fmul_rn(lam, wd[s - 1]) : 0.f;
+    __syncwarp();
     float Dp = 0.f, ABp = -1.f, p1 = 0.f, p2 = 0.f;
     for (int j = s; j <= e && act; j++) {
-        const float c = __fmul_rn(lam, wgt[j]), a = j > 0 ? __fmul_rn(lam, wgt[j - 1]) : 0.f;
+        const float c = __fmul_rn(lam, wd[j]);
         const float b = 1.0f - a - c;
         const float ib = __frcp_rn(b - a * Dp);
         Dp = c * ib;
         ABp = -a * ABp * ib;
         p1 = (g1[j] - a * p1) * ib;
         p2 = (g2[j] - a * p2) * ib;
-        Dd[j] = Dp; AB[j] = ABp; g1[j] = p1; g2[j] = p2;
+        wd[j] = Dp; AB[j] = ABp; g1[j] = p1; g2[j] = p2;
+        a = c;
     }
     // ---- reduced system over the chunk ends: A u_e(l-1) + B u_e(l) + C u_e(l+1) = F
     const int ncnt = __shfl_down_sync(0xffffffffu, cnt, 1);
@@ -401,7 +410,7 @@ __device__ __forceinline__ void fgsp_solve_line(const float* __restrict__ wgt, f
         float n1 = ue1, n2 = ue2;
         g1[e] = n1; g2[e] = n2;
         for (int j = e - 1; j >= s; j--) {
-            const float d = Dd[j], ab = AB[j];
+            const float d = wd[j], ab = AB[j];
             n1 = g1[j] - ab * up1 - d * n1;
             n2 = g2[j] - ab * up2 - d * n2;
             g1[j] = n1; g2[j] = n2;
@@ -409,79 +418,172 @@ __device__ __forceinline__ void fgsp_solve_line(const float* __restrict__ wgt, f
     }
 }
 
-static size_t fgsp_smem_bytes(int lines, int len) { return (size_t)lines * 5 * ((size_t)len + 8) * sizeof(float); }
+__device__ __forceinline__ void cp_async4(float* dst, const float* src) {
+    asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"((uint32_t)__cvta_generic_to_shared(dst)), "l"(src) : "memory");
+}
 
-// row pass: warp <-> image row; num / den are solved in place
+// row plane pitch (floats): a multiple of 4 when w is, so that every plane of a line starts 16-byte aligned
+__host__ __device__ inline int fgsp_row_pitch(int w) { return w + 8; }
+static size_t fgsp_rows_smem(int w) { return (size_t)FGSP_ROWS * 4 * fgsp_row_pitch(w) * sizeof(float); }
+
+// row pass: warp <-> image row; num / den are solved in place.  bulk (w % 4 == 0 and 16-byte aligned planes): each
+// plane row moves as one cp.async.bulk (in on an mbarrier, out as a bulk store); otherwise one cp.async per element.
 __global__ void __launch_bounds__(FGSP_ROWS * 32) fgs_rows_par_kernel(float* num, float* den, const float* __restrict__ wgt,
-                                                                     int w, int h, float lam) {
+                                                                     int w, int h, float lam, int bulk) {
     extern __shared__ __align__(16) float fsm[];
-    const int LP = w + 8;
+    __shared__ __align__(8) uint64_t bar[FGSP_ROWS];
+    const int LP = fgsp_row_pitch(w);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int row = blockIdx.x * FGSP_ROWS + warp;
-    float* base = fsm + (size_t)warp * 5 * LP;
-    float *sw = base, *s1 = base + LP, *s2 = base + 2 * LP, *sD = base + 3 * LP, *sA = base + 4 * LP;
-    if (row < h) {
-        const size_t off = (size_t)row * w;
-        for (int i = lane; i < w; i += 32) { sw[i] = wgt[off + i]; s1[i] = num[off + i]; s2[i] = den[off + i]; }
+    if (row >= h) return;  // whole warps; the CTA never synchronises
+    float* base = fsm + (size_t)warp * 4 * LP;
+    float *sw = base, *s1 = base + LP, *s2 = base + 2 * LP, *sA = base + 3 * LP;
+    const size_t off = (size_t)row * w;
+    const uint32_t bytes = (uint32_t)w * 4u;
+    if (bulk) {
+        const uint32_t mb = (uint32_t)__cvta_generic_to_shared(&bar[warp]);
+        if (lane == 0) {
+            asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(mb) : "memory");
+            asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+            asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(mb), "r"(3u * bytes) : "memory");
+            const float* src[3] = {wgt + off, num + off, den + off};
+            float* dst[3] = {sw, s1, s2};
+#pragma unroll
+            for (int i = 0; i < 3; i++)
+                asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
+                             ::"r"((uint32_t)__cvta_generic_to_shared(dst[i])), "l"(src[i]), "r"(bytes), "r"(mb) : "memory");
+        }
+        __syncwarp();
+        asm volatile("{\n\t.reg .pred P1;\n\tWAIT:\n\t"
+                     "mbarrier.try_wait.parity.shared::cta.b64 P1, [%0], 0;\n\t"
+                     "@!P1 bra WAIT;\n\t}" ::"r"(mb) : "memory");
+    } else {
+        for (int i = lane; i < w; i += 32) {
+            cp_async4(sw + i, wgt + off + i); cp_async4(s1 + i, num + off + i); cp_async4(s2 + i, den + off + i);
+        }
+        asm volatile("cp.async.wait_all;" ::: "memory");
+        __syncwarp();
     }
-    __syncwarp();
-    if (row < h) fgsp_solve_line(sw, s1, s2, sD, sA, w, lam, lane);
-    __syncwarp();
-    if (row < h) {
-        const size_t off = (size_t)row * w;
+    fgsp_solve_line(sw, s1, s2, sA, w, lam, lane);
+    if (bulk) {
+        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // the solve's stores, visible to the bulk copy
+        __syncwarp();
+        if (lane == 0) {
+            asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;"
+                         ::"l"(num + off), "r"((uint32_t)__cvta_generic_to_shared(s1)), "r"(bytes) : "memory");
+            asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;"
+                         ::"l"(den + off), "r"((uint32_t)__cvta_generic_to_shared(s2)), "r"(bytes) : "memory");
+            asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+            asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");  // shared memory stays alive until read
+        }
+    } else {
+        __syncwarp();
         for (int i = lane; i < w; i += 32) { num[off + i] = s1[i]; den[off + i] = s2[i]; }
     }
 }
 
-// column pass: a CTA stages FGSP_COLS adjacent columns (32 contiguous bytes per image row), warp <-> column
-__global__ void __launch_bounds__(FGSP_COLS * 32) fgs_cols_par_kernel(float* num, float* den, const float* __restrict__ wgt,
-                                                                     int w, int h, float lam) {
+// column plane pitch (floats): == 32 / NC mod 32, so that a staging request (NC adjacent columns x 32 / NC rows) hits
+// 32 different banks.  Plane p of column c starts at (p * NC + c) * pitch.
+__host__ __device__ inline int fgsp_col_pitch(int h, int nc) { return ((h + 31) / 32) * 32 + 32 / nc; }
+static size_t fgsp_cols_smem(int h, int nc) { return (size_t)nc * 4 * fgsp_col_pitch(h, nc) * sizeof(float); }
+
+// column pass: a CTA stages NC adjacent columns (4 NC contiguous bytes per image row), warp <-> column.  The staging
+// copies are one cp.async per element, all issued before the one wait: a 16-byte copy would span four columns, which
+// live in different planes.
+template <int NC>
+__global__ void __launch_bounds__(NC * 32) fgs_cols_par_kernel(float* num, float* den, const float* __restrict__ wgt,
+                                                              int w, int h, float lam) {
     extern __shared__ __align__(16) float fsm[];
-    const int LP = ((h + 31) / 32) * 32 + 4;  // == 4 mod 32: the 8 columns x 4 rows a warp stages per request hit 32 banks
+    const int LP = fgsp_col_pitch(h, NC);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int col0 = blockIdx.x * FGSP_COLS;
-    const int ncol = min(FGSP_COLS, w - col0);
-    const int tc = threadIdx.x & (FGSP_COLS - 1), tr = threadIdx.x / FGSP_COLS;  // staging role: column, row phase
-    constexpr int RPI = FGSP_COLS * 32 / FGSP_COLS;                               // rows per staging iteration
+    const int col0 = blockIdx.x * NC;
+    const int ncol = min(NC, w - col0);
+    const int tc = threadIdx.x % NC, tr = threadIdx.x / NC;  // staging role: column, row phase (32 phases)
     if (tc < ncol) {
-        float *sw = fsm + (size_t)tc * 5 * LP, *s1 = sw + LP, *s2 = sw + 2 * LP;
-        for (int r = tr; r < h; r += RPI) {
+        for (int r = tr; r < h; r += 32) {
             const size_t g = (size_t)r * w + col0 + tc;
-            sw[r] = wgt[g]; s1[r] = num[g]; s2[r] = den[g];
+            cp_async4(fsm + (size_t)tc * LP + r, wgt + g);
+            cp_async4(fsm + (size_t)(NC + tc) * LP + r, num + g);
+            cp_async4(fsm + (size_t)(2 * NC + tc) * LP + r, den + g);
         }
     }
+    asm volatile("cp.async.wait_all;" ::: "memory");
     __syncthreads();
-    if (warp < ncol) {
-        float* base = fsm + (size_t)warp * 5 * LP;
-        fgsp_solve_line(base, base + LP, base + 2 * LP, base + 3 * LP, base + 4 * LP, h, lam, lane);
-    }
+    if (warp < ncol)
+        fgsp_solve_line(fsm + (size_t)warp * LP, fsm + (size_t)(NC + warp) * LP, fsm + (size_t)(2 * NC + warp) * LP,
+                        fsm + (size_t)(3 * NC + warp) * LP, h, lam, lane);
     __syncthreads();
     if (tc < ncol) {
-        const float *s1 = fsm + (size_t)tc * 5 * LP + LP, *s2 = s1 + LP;
-        for (int r = tr; r < h; r += RPI) {
+        const float *s1 = fsm + (size_t)(NC + tc) * LP, *s2 = fsm + (size_t)(2 * NC + tc) * LP;
+        for (int r = tr; r < h; r += 32) {
             const size_t g = (size_t)r * w + col0 + tc;
             num[g] = s1[r]; den[g] = s2[r];
         }
     }
 }
 
+// ---- K5a: disparity -> depth of one pixel (camera/single_usb_stereo_camera.py:335-357) ------------------------------
+struct QMat { double q[16]; };
+
+__device__ __forceinline__ float depth_q_px(int16_t d16, int x, int y, const QMat& Q) {
+    float disp = __fdiv_rn((float)d16, 16.0f);
+    double d = (double)disp, fx = (double)x, fy = (double)y;
+    // cv2.reprojectImageTo3D (4.13, probed): [X Y Z W]^T = Q [x y d 1]^T in f64, the numerator is
+    // first stored as f32 (Vec3f), then divided by the f64 W and rounded to f32 again
+    double Z = __dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(Q.q[8], fx), __dmul_rn(Q.q[9], fy)), __dmul_rn(Q.q[10], d)), Q.q[11]);
+    double Wh = __dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(Q.q[12], fx), __dmul_rn(Q.q[13], fy)), __dmul_rn(Q.q[14], d)), Q.q[15]);
+    float z = (float)__ddiv_rn((double)(float)Z, Wh);
+    if (z < 0.f) z = 0.f;
+    if (z > 10.f) z = 0.f;
+    if (disp <= 0.f) z = 0.f;
+    return z;
+}
+
+__device__ __forceinline__ float depth_default_px(int16_t d16) {
+    float disp = __fdiv_rn((float)d16, 16.0f);
+    float z = 0.f;
+    if (disp > 0.f) z = __fdiv_rn((float)(0.06 * 350), disp);
+    if (z > 10.f) z = 0.f;
+    return z;
+}
+
+// DEPTH: 0 = the filtered disparity alone; 1 / 2 = also its depth, through Q / the default baseline (dev_depth's two
+// kernels), so the frame pipeline spends no launch and no re-read of the disparity on it
+template <int DEPTH>
 __global__ void wls_finalize_kernel(const float* __restrict__ num, const float* __restrict__ den,
                                     const float* __restrict__ conf, int W, int H, int x0, int w, int outside,
-                                    int16_t* __restrict__ out, float* __restrict__ conf_out) {
+                                    int16_t* __restrict__ out, float* __restrict__ conf_out, QMat Q, float* __restrict__ depth) {
     int x = blockIdx.x * blockDim.x + threadIdx.x;
     int y = blockIdx.y;
     if (x >= W) return;
     size_t o = (size_t)y * W + x;
-    if (x < x0) { out[o] = (int16_t)outside; if (conf_out) conf_out[o] = 0.f; return; }
-    size_t i = (size_t)y * w + (x - x0);
-    float v = __fmul_rn(num[i], __fdiv_rn(1.0f, __fadd_rn(den[i], 1e-43f)));
     int q;
-    if (!(fabsf(v) < 2147483648.f)) q = -32768;  // NaN / |v| >= 2^31: cvRound gives INT_MIN
-    else if (v >= 32767.f) q = 32767;
-    else if (v <= -32768.f) q = -32768;
-    else q = __float2int_rn(v);
+    if (x < x0) {
+        q = outside;
+        if (conf_out) conf_out[o] = 0.f;
+    } else {
+        size_t i = (size_t)y * w + (x - x0);
+        float v = __fmul_rn(num[i], __fdiv_rn(1.0f, __fadd_rn(den[i], 1e-43f)));
+        if (!(fabsf(v) < 2147483648.f)) q = -32768;  // NaN / |v| >= 2^31: cvRound gives INT_MIN
+        else if (v >= 32767.f) q = 32767;
+        else if (v <= -32768.f) q = -32768;
+        else q = __float2int_rn(v);
+        if (conf_out) conf_out[o] = conf[i];
+    }
     out[o] = (int16_t)q;
-    if (conf_out) conf_out[o] = conf[i];
+    if (DEPTH == 1) depth[o] = depth_q_px((int16_t)q, x, y, Q);
+    if (DEPTH == 2) depth[o] = depth_default_px((int16_t)q);
+}
+
+static int wls_finalize(Lane& L, const float* num, const float* den, const float* conf, int W, int H, int x0, int w,
+                        int outside, int16_t* out, float* conf_out, float* depth, const double* Q) {
+    const dim3 g(cdiv(W, 128), H);
+    QMat q{};
+    if (Q) memcpy(q.q, Q, sizeof(q.q));
+    if (!depth) L3D_LAUNCH(L, wls_finalize_kernel<0>, g, 128, 0, num, den, conf, W, H, x0, w, outside, out, conf_out, q, depth);
+    else if (Q) L3D_LAUNCH(L, wls_finalize_kernel<1>, g, 128, 0, num, den, conf, W, H, x0, w, outside, out, conf_out, q, depth);
+    else L3D_LAUNCH(L, wls_finalize_kernel<2>, g, 128, 0, num, den, conf, W, H, x0, w, outside, out, conf_out, q, depth);
+    return L3D_OK;
 }
 
 // exp LUT for the guide weights: lut[k] = -exp(-sqrt(k)/sigma), k = squared grey difference
@@ -501,24 +603,36 @@ static int wls_lut(Lane& L, double sigma, float** out) {
 // The FGS passes of the WLS filter (dev_wls; l3d_fgs_solve runs them alone): `iters` iterations of (row solves with
 // weights ch, column solves with weights cv) on num/den in place; Dscr (w x h) is scratch of the serial kernels.
 // solver: 0 = partitioned parallel solves (default), 1 = serial solves in the oracle's operation order (bit-identical
-// to oracle/csrc/orc_wls.c); L3D_FGS_SERIAL=1 forces the serial form everywhere, and so do lines longer than the
-// parallel kernels can stage in shared memory (w > 2552 or h > 1248) or shorter than 2.
+// to oracle/csrc/orc_wls.c); L3D_FGS_SERIAL=1 forces the serial form everywhere, and so do lines longer than
+// FGSP_W_MAX / FGSP_H_MAX or shorter than 2.
 int dev_fgs(Lane& L, int solver, int variant, double lambda, int iters, const float* ch, const float* cv, int w, int h,
             float* num, float* den, float* Dscr, bool* parallel_used) {
     float lam = (float)lambda;
     static const bool force_serial = getenv("L3D_FGS_SERIAL") && atoi(getenv("L3D_FGS_SERIAL")) > 0;
-    const size_t smr = fgsp_smem_bytes(FGSP_ROWS, w), smc = (size_t)FGSP_COLS * 5 * (((h + 31) / 32) * 32 + 4) * sizeof(float);
-    const bool parallel = !force_serial && solver != 1 && smr <= 200 * 1024 && smc <= 200 * 1024 && w >= 2 && h >= 2;
+    const bool parallel = !force_serial && solver != 1 && w <= FGSP_W_MAX && h <= FGSP_H_MAX && w >= 2 && h >= 2;
     *parallel_used = parallel;
+    const size_t smr = fgsp_rows_smem(w);
+    int nc = 8;  // columns per CTA: 16 where a 16-column CTA fits an SM, else 8
+    const int bulk = w % 4 == 0 && ((uintptr_t)num | (uintptr_t)den | (uintptr_t)ch) % 16 == 0;
     if (parallel) {
+        int dev = 0, optin = 0, fit = 0;
+        L3D_CHECK(L, cudaGetDevice(&dev));
+        L3D_CHECK(L, cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+        if (fgsp_cols_smem(h, 16) <= (size_t)optin) {
+            L3D_CHECK(L, cudaFuncSetAttribute(fgs_cols_par_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fgsp_cols_smem(h, 16)));
+            L3D_CHECK(L, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&fit, fgs_cols_par_kernel<16>, 16 * 32, fgsp_cols_smem(h, 16)));
+        }
+        if (fit >= 1) nc = 16;
+        else L3D_CHECK(L, cudaFuncSetAttribute(fgs_cols_par_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fgsp_cols_smem(h, 8)));
         L3D_CHECK(L, cudaFuncSetAttribute(fgs_rows_par_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smr));
-        L3D_CHECK(L, cudaFuncSetAttribute(fgs_cols_par_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smc));
     }
+    const size_t smc = fgsp_cols_smem(h, nc);
     for (int it = 0; it < iters; it++) {
-        if (parallel) L3D_LAUNCH(L, fgs_rows_par_kernel, cdiv(h, FGSP_ROWS), FGSP_ROWS * 32, smr, num, den, ch, w, h, lam);
+        if (parallel) L3D_LAUNCH(L, fgs_rows_par_kernel, cdiv(h, FGSP_ROWS), FGSP_ROWS * 32, smr, num, den, ch, w, h, lam, bulk);
         else L3D_LAUNCH(L, fgs_rows_kernel, cdiv(h, FGS_LPW), 32, 0, num, den, ch, Dscr, w, h, lam);
         if (variant & L3D_WLS_LAMBDA_PER_PASS) lam *= 0.25f;
-        if (parallel) L3D_LAUNCH(L, fgs_cols_par_kernel, cdiv(w, FGSP_COLS), FGSP_COLS * 32, smc, num, den, cv, w, h, lam);
+        if (parallel && nc == 16) L3D_LAUNCH(L, fgs_cols_par_kernel<16>, cdiv(w, 16), 16 * 32, smc, num, den, cv, w, h, lam);
+        else if (parallel) L3D_LAUNCH(L, fgs_cols_par_kernel<8>, cdiv(w, 8), 8 * 32, smc, num, den, cv, w, h, lam);
         else L3D_LAUNCH(L, fgs_cols_kernel<FGS_CPW>, cdiv(w, FGS_CPW), 32, 0, num, den, cv, Dscr, w, h, lam);
         lam *= 0.25f;
     }
@@ -526,14 +640,13 @@ int dev_fgs(Lane& L, int solver, int variant, double lambda, int iters, const fl
 }
 
 int dev_wls(Lane& L, const l3d_wls_params& p, const int16_t* dl, const int16_t* dr, const uint8_t* guide,
-            int W, int H, int16_t* out, float* conf_out) {
+            int W, int H, int16_t* out, float* conf_out, float* depth, const double* Q) {
     int x0 = std::max(0, p.min_disp + p.num_disp);
     int w = W - x0, h = H;
     int outside = 16 * (p.min_disp - 1);
     if (w <= 0) {
         // nothing inside the ROI: constant output
-        L3D_LAUNCH(L, wls_finalize_kernel, dim3(cdiv(W, 128), H), 128, 0, nullptr, nullptr, nullptr, W, H, W, 0, outside, out, conf_out);
-        return L3D_OK;
+        return wls_finalize(L, nullptr, nullptr, nullptr, W, H, W, 0, outside, out, conf_out, depth, Q);
     }
     L3D_ARG(L, p.dd_radius >= 0 && p.dd_radius < 64, "wls dd_radius");
     size_t n = (size_t)w * h;
@@ -554,40 +667,25 @@ int dev_wls(Lane& L, const l3d_wls_params& p, const int16_t* dl, const int16_t* 
     bool parallel = false;
     rc = dev_fgs(L, p.solver, p.variant, p.lambda, 3, ch, cv, w, h, num, den, aR, &parallel);  // aR is free as well: scratch D
     if (rc != L3D_OK) return rc;
-    L3D_LAUNCH(L, wls_finalize_kernel, dim3(cdiv(W, 128), H), 128, 0, num, den, conf, W, H, x0, w, outside, out, conf_out);
+    rc = wls_finalize(L, num, den, conf, W, H, x0, w, outside, out, conf_out, depth, Q);
     L.t_end("wls");
+    if (rc != L3D_OK) return rc;
     return L3D_OK;
 }
 
-// ---- K5a: disparity -> depth (camera/single_usb_stereo_camera.py:335-357) -------------------
-struct QMat { double q[16]; };
-
+// ---- K5a: disparity -> depth ---------------------------------------------------------------
 __global__ void depth_q_kernel(const int16_t* __restrict__ d16, int W, int H, QMat Q, float* __restrict__ depth) {
     int x = blockIdx.x * blockDim.x + threadIdx.x;
     int y = blockIdx.y;
     if (x >= W) return;
     size_t i = (size_t)y * W + x;
-    float disp = __fdiv_rn((float)d16[i], 16.0f);
-    double d = (double)disp, fx = (double)x, fy = (double)y;
-    // cv2.reprojectImageTo3D (4.13, probed): [X Y Z W]^T = Q [x y d 1]^T in f64, the numerator is
-    // first stored as f32 (Vec3f), then divided by the f64 W and rounded to f32 again
-    double Z = __dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(Q.q[8], fx), __dmul_rn(Q.q[9], fy)), __dmul_rn(Q.q[10], d)), Q.q[11]);
-    double Wh = __dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(Q.q[12], fx), __dmul_rn(Q.q[13], fy)), __dmul_rn(Q.q[14], d)), Q.q[15]);
-    float z = (float)__ddiv_rn((double)(float)Z, Wh);
-    if (z < 0.f) z = 0.f;
-    if (z > 10.f) z = 0.f;
-    if (disp <= 0.f) z = 0.f;
-    depth[i] = z;
+    depth[i] = depth_q_px(d16[i], x, y, Q);
 }
 
 __global__ void depth_default_kernel(const int16_t* __restrict__ d16, size_t n, float* __restrict__ depth) {
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    float disp = __fdiv_rn((float)d16[i], 16.0f);
-    float z = 0.f;
-    if (disp > 0.f) z = __fdiv_rn((float)(0.06 * 350), disp);
-    if (z > 10.f) z = 0.f;
-    depth[i] = z;
+    depth[i] = depth_default_px(d16[i]);
 }
 
 int dev_depth(Lane& L, const int16_t* disp16, int W, int H, const double* Q, float* depth) {
