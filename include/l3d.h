@@ -140,7 +140,7 @@ int l3d_wls_filter(l3d_ctx* ctx, const l3d_wls_params* p, const int16_t* dl, con
  * row weights ch and column weights cv (<= 0, as the LUT makes them). Runs `iters` (1..3)
  * iterations of (row pass, column pass) with the lambda schedule of `variant`. solver: as in
  * l3d_wls_params. *parallel_used = 1 when the partitioned kernels ran, 0 for the serial
- * fallback (gate: solver, L3D_FGS_SERIAL, shared-memory size, w >= 2 && h >= 2). */
+ * fallback (gate: solver, shared-memory size, w >= 2 && h >= 2). */
 int l3d_fgs_solve(l3d_ctx* ctx, int solver, int variant, double lambda, int iters,
                   const float* ch, const float* cv, int w, int h, float* num, float* den, int* parallel_used);
 

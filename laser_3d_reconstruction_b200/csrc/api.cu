@@ -969,9 +969,7 @@ int l3d_pipeline_create(l3d_ctx* ctx, const l3d_pipeline_config* cfg, l3d_pipeli
     // the whole register file); the short back-half kernels come next, the wide front kernels fill the rest.
     int prio_lo = 0, prio_hi = 0;
     CK(ctx, cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi));
-    int prio[3] = {prio_hi, prio_lo, std::max(prio_hi, prio_lo - 2)};  // aggregation, front, back
-    if (const char* e = getenv("L3D_PRIO")) sscanf(e, "%d,%d,%d", &prio[0], &prio[1], &prio[2]);
-    for (int& q : prio) q = std::min(prio_lo, std::max(prio_hi, q));
+    const int prio[3] = {prio_hi, prio_lo, std::max(prio_hi, prio_lo - 2)};  // aggregation, front, back
     CK(ctx, cudaMalloc(&p->flags, 16));
     CK(ctx, cudaMemset(p->flags, 0, 16));
     for (auto& L : p->lanes) {
@@ -1038,13 +1036,9 @@ int l3d_pipeline_set_maps(l3d_pipeline* p, int eye, const float* mapx, const flo
 constexpr int VG_WAVE = 15;
 static int pipe_group_size(const l3d_pipeline* p) {
     const int jobs_per_frame = p->cfg.depth.use_wls ? 2 : 1;
-    static const int forced = getenv("L3D_GROUP") ? atoi(getenv("L3D_GROUP")) : 0;  // experiment: frames per lane set
-    if (forced > 0) return std::min((int)p->lanes.size(), forced);
     return std::min((int)p->lanes.size(), std::max(1, VG_WAVE / jobs_per_frame));
 }
 static bool pipe_grouped(const l3d_pipeline* p) {
-    static const bool off = getenv("L3D_NO_VGROUP") && atoi(getenv("L3D_NO_VGROUP")) > 0;
-    if (off) return false;
     const l3d_pipeline_config& c = p->cfg;
     const int jobs_per_frame = c.depth.use_wls ? 2 : 1;
     if (pipe_group_size(p) * jobs_per_frame < 8 || c.depth.left.mode >= 2) return false;  // 3WAY / HH4: direction-split

@@ -10,16 +10,18 @@
 //
 // Kernels:
 //   sgbm_prefilter_kernel     x-Sobel clip + half-pixel min/max, as pixel-pair operand entries (2 planes x 16 B / pixel)
-//   sgbm_cost_warp_kernel     Birchfield-Tomasi pixel cost -> blockSize^2 box sum -> C (+P2); disparity pairs split over
-//                             the warps, warp-private cost strips and row-sum rings, TMA operand ring, no block barrier
-//   sgbm_cost_kernel          the block-synchronous form (D = 256 and every other geometry)
+//   sgbm_cost_dual_kernel     Birchfield-Tomasi pixel cost -> blockSize^2 box sum -> C (+P2), single-segment volumes at
+//                             block 5 / D 64, block 9 / D 128, block 11 / D 256 (one or both matchers of a frame)
+//   sgbm_cost_warp_kernel     the warp-decoupled single-volume form: SGBM_3WAY's striped volumes at block 5 / D 64 and
+//                             block 9 / D 128
+//   sgbm_cost_kernel          the block-synchronous form: every other geometry, SGBM_3WAY's at block 11 / D 256 among them
 //   sgbm_scan_hpair_kernel    both horizontal paths of a row in one CTA
 //   sgbm_scan_kernel          one SGM path direction per launch, one warp per scan line, path state in registers,
 //                             DPX u16x2 min/add, warp-wide min via CREDUX, C/S streamed through a cp.async ring; the
-//                             last path can run the WTA (SCAN_FINAL)
+//                             last path can run the WTA (SCAN_FINAL; modes SGBM / HH / HH4)
 //   sgbm_vgroup_kernel        (sgbm_vgroup.cu) the three previous-row paths of a pass fused on a thread-block cluster
 //   sgbm_wta_lean_kernel      WTA + uniqueness + disp2 (atomicMax key) + sub-pixel, 32 pixels per warp (modes SGBM / HH / HH4)
-//   sgbm_wta_lean3_kernel     the same walk with SGBM_3WAY's rules; sgbm_wta_kernel is the warp-per-pixel restatement
+//   sgbm_wta_lean3_kernel     the same walk with SGBM_3WAY's rules
 //   sgbm_lrcheck_kernel       left-right consistency
 // Value domain (see DESIGN.md): 0 <= L,S <= 32767 and C >= P2, which holds whenever the block sum
 // does not wrap int16 (always for blockSize <= 9; for 11 unless every pixel of a block mismatches
@@ -103,24 +105,22 @@ int sgbm_volume_rows(const l3d_sgbm_params& p, int W, int H) {
 // ------------------------------------------------------------------------------------------
 // directional aggregation scan
 // ------------------------------------------------------------------------------------------
+// The kernels take ScanArgs and WtaArgs as __grid_constant__: they index the segment tables at run time, and NVVM copies
+// a by-value parameter of up to 128 bytes (the size of both) into a local-memory stack frame to do that unless the
+// parameter is declared read-only.
 struct ScanArgs {
     const int16_t* C; int16_t* S;
     int width1, D, nact, P1, P2;
     uint32_t zero;  // 0, as a value the compiler cannot see (sgm_step.cuh)
-    int hp_mode;    // horizontal pair: 0 = each warp runs on through the other half, 1 = each warp turns round at the middle
     int hp_row0;    // horizontal pair: first volume row of this launch (row waves)
     int kind;   // 0 ->, 1 <-, 2 down, 3 down-right, 4 down-left, 5 up, 6 up-left, 7 up-right
     int store;  // 1: S = L ; 0: S = min(S + L, 32767)
     int HV, nseg;
     int lines_per_seg;  // kinds >= 2: lines per segment (columns, or diagonals)
     int seg_vr0[MAXSEG], seg_rows[MAXSEG];
-    // SCAN_FINAL only: the winner-takes-all stage fused into the last path (modes SGBM / HH)
+    // SCAN_FINAL only: the winner-takes-all stage fused into the last path (modes SGBM / HH / HH4: one segment)
     int16_t* raw; unsigned* disp2key;
     int W, minD, minX1, uniq;
-    // SGBM_3WAY in SCAN_FINAL: that mode's WTA rules (see sgbm_wta_lean3_kernel) and its stripes (volume row -> image row,
-    // overlap rows not emitted)
-    int tway;
-    int seg_y0[MAXSEG], seg_emit[MAXSEG];
 };
 enum { SCAN_STORE = 0, SCAN_ACCUM = 1, SCAN_FINAL = 2 };  // S = L | S = sat(S + L) | sat(S + L) -> WTA, S not written
 
@@ -310,20 +310,11 @@ __device__ __forceinline__ void scan_run(const ScanArgs& a, const ScanLine& ln, 
         __syncwarp();
         const int minS = (int)(wkey >> 8), d = (int)(wkey & 255u);
         const int j = first_step + lane;
-        int y = ln.vr + ln.dvr * j;
+        const int y = ln.vr + ln.dvr * j;
         const int x = ln.x + ln.dx * j;
-        bool emit = lane < count && !wrej;
-        if (a.tway) {  // stripe volume row -> image row; the overlap rows of a stripe only feed the recurrence
-            int seg = 0;
-            for (int q = 1; q < a.nseg; q++) if (y >= a.seg_vr0[q]) seg = q;
-            y = a.seg_y0[seg] + (y - a.seg_vr0[seg]);
-            emit = emit && y >= a.seg_emit[seg];
-        } else {
-            emit = emit && minS < 32767;  // minS == 32767: nothing beat MAX_COST, pixel stays invalid
-        }
-        if (emit) {
+        if (lane < count && !wrej && minS < 32767) {  // minS == 32767: nothing beat MAX_COST, pixel stays invalid
             const int x2 = x + a.minX1 - d - a.minD;
-            if (x2 >= 0 && x2 < (a.tway ? a.W : a.W + 2) && minS < 32767)
+            if (x2 >= 0 && x2 < a.W + 2)
                 atomicMax(a.disp2key + (size_t)y * (a.W + 2) + x2, ((unsigned)(0x7fff - minS) << 16) | (unsigned)x);
             int dd = d * 16;
             if (0 < d && d < a.D - 1) {
@@ -363,49 +354,13 @@ __device__ __forceinline__ void scan_run(const ScanArgs& a, const ScanLine& ln, 
             bool rej = false;
             const int slot = nsteps & 31;
             if (active) *(vec*)(stash + (size_t)slot * B + (size_t)lane * sizeof(vec)) = vec_pack<NP>(out);
-            if (a.tway) {  // SGBM_3WAY: SIMD-lane arg-min and SIMD-form uniqueness test (sgbm_wta_lean3_kernel)
-                int sv[DPL];
 #pragma unroll
-                for (int q = 0; q < NP; q++) { sv[2 * q] = (int)(out[q] & 0xffffu); sv[2 * q + 1] = (int)(out[q] >> 16); }
-                int m = 32767;
-#pragma unroll
-                for (int jj = 0; jj < DPL; jj++) m = min(m, sv[jj]);
-                const int minS = __reduce_min_sync(FULL_MASK, m);
-                int best = 0x7fffffff;
-#pragma unroll
-                for (int jj = 0; jj < DPL; jj++) {
-                    const unsigned bb = __ballot_sync(FULL_MASK, active && sv[jj] == minS);
-                    constexpr int LPC = 8 / DPL > 0 ? 8 / DPL : 1;
-#pragma unroll
-                    for (int r = 0; r < LPC; r++) {
-                        unsigned pat = 0;
-#pragma unroll
-                        for (int l = r; l < 32; l += LPC) pat |= 1u << l;
-                        const unsigned mm = bb & pat;
-                        if (mm) best = min(best, (31 - __clz(mm)) * DPL + jj);
-                    }
-                }
-                if (a.uniq > 0) {
-                    const int thresh = (100 * minS) / (100 - a.uniq);
-                    const int tr = (int)(short)(thresh + 1);
-                    bool v = false;
-#pragma unroll
-                    for (int jj = 0; jj < DPL; jj++) {
-                        const int d = lane * DPL + jj;
-                        if (active && sv[jj] < tr && (d < best - 1 || d > best + 1)) v = true;
-                    }
-                    rej = __any_sync(FULL_MASK, v);
-                }
-                key = ((unsigned)minS << 8) | (unsigned)(best & 255);
-            } else {
-#pragma unroll
-                for (int q = 0; q < NP; q++) {
-                    key = min(key, ((out[q] << 8) & 0xffff00u) | (dkey + 2 * q));
-                    key = min(key, ((out[q] >> 8) & 0xffff00u) | (dkey + 2 * q + 1));
-                }
-                key = __reduce_min_sync(FULL_MASK, key);
-                if (a.uniq > 0) rej = wta_not_unique<NP>(out, key, a.uniq, dkey, active);
+            for (int q = 0; q < NP; q++) {
+                key = min(key, ((out[q] << 8) & 0xffff00u) | (dkey + 2 * q));
+                key = min(key, ((out[q] >> 8) & 0xffff00u) | (dkey + 2 * q + 1));
             }
+            key = __reduce_min_sync(FULL_MASK, key);
+            if (a.uniq > 0) rej = wta_not_unique<NP>(out, key, a.uniq, dkey, active);
             if (lane == slot) { wkey = key; wrej = rej; }
             nsteps++;
         }
@@ -431,7 +386,7 @@ __device__ __forceinline__ void scan_run(const ScanArgs& a, const ScanLine& ln, 
 }
 
 template <int NP, int SMODE, bool FULL>
-__global__ void __launch_bounds__(32) sgbm_scan_kernel(const ScanArgs a) {
+__global__ void __launch_bounds__(32) sgbm_scan_kernel(const __grid_constant__ ScanArgs a) {
     extern __shared__ __align__(128) unsigned char scan_smem[];
     const int lane = threadIdx.x;
     ScanLine ln;
@@ -444,11 +399,12 @@ __global__ void __launch_bounds__(32) sgbm_scan_kernel(const ScanArgs a) {
 }
 
 // Both horizontal paths of one row in one CTA of two warps: warp 0 runs left-to-right, warp 1
-// right-to-left.  Each first covers its own half storing S = L, the CTA synchronises, and each
-// continues through the other half accumulating S = sat(S + L) -- every S vector is written once
-// and read-modified once, and the two serial recurrences of a row run concurrently.
+// right-to-left.  Each first covers its own half storing S = L; at the middle the two exchange
+// their path states and each walks back over its own half with the other direction's path,
+// accumulating S = sat(S + L) -- every S vector is written once and read-modified once, and the
+// two serial recurrences of a row run concurrently.
 template <int NP, bool FULL>
-__global__ void __launch_bounds__(64) sgbm_scan_hpair_kernel(const ScanArgs a) {
+__global__ void __launch_bounds__(64) sgbm_scan_hpair_kernel(const __grid_constant__ ScanArgs a) {
     extern __shared__ __align__(128) unsigned char scan_smem[];
     __shared__ uint32_t xch[2][32][NP + 1];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -456,29 +412,23 @@ __global__ void __launch_bounds__(64) sgbm_scan_hpair_kernel(const ScanArgs a) {
     const int vr = a.hp_row0 + blockIdx.x, width1 = a.width1, mid = width1 / 2;
     ScanLine s1, s2;
     s1.vr = s2.vr = vr; s1.dvr = s2.dvr = 0;
-    if (warp == 0) { s1.x = 0; s1.n = mid; s1.dx = 1; s2.x = mid; s2.n = width1 - mid; s2.dx = 1; }
-    else { s1.x = width1 - 1; s1.n = width1 - mid; s1.dx = -1; s2.x = mid - 1; s2.n = mid; s2.dx = -1; }
+    if (warp == 0) { s1.x = 0; s1.n = mid; s1.dx = 1; s2.x = mid - 1; s2.n = mid; s2.dx = -1; }
+    else { s1.x = width1 - 1; s1.n = width1 - mid; s1.dx = -1; s2.x = mid; s2.n = width1 - mid; s2.dx = 1; }
     uint32_t L[NP];
 #pragma unroll
     for (int k = 0; k < NP; k++) L[k] = (FULL || lane < a.nact) ? 0u : INF2;
     uint32_t minL = 0;
     scan_run<NP, SCAN_STORE, FULL, HPAIR_NST>(a, s1, my_smem, L, minL, lane);
-    if (a.hp_mode == 1) {
-        // turn round: the two warps exchange their path states at the middle and each walks back over ITS OWN half with
-        // the other direction's path -- the vectors it needs first are the ones it touched last (L2 reuse distance grows
-        // from zero instead of being half a row for every vector)
+    // turn round: the two warps exchange their path states at the middle and each walks back over ITS OWN half with
+    // the other direction's path -- the vectors it needs first are the ones it touched last (L2 reuse distance grows
+    // from zero instead of being half a row for every vector)
 #pragma unroll
-        for (int k = 0; k < NP; k++) xch[warp][lane][k] = L[k];
-        xch[warp][lane][NP] = minL;
-        __syncthreads();
+    for (int k = 0; k < NP; k++) xch[warp][lane][k] = L[k];
+    xch[warp][lane][NP] = minL;
+    __syncthreads();
 #pragma unroll
-        for (int k = 0; k < NP; k++) L[k] = xch[warp ^ 1][lane][k];
-        minL = xch[warp ^ 1][lane][NP];
-        if (warp == 0) { s2.x = mid - 1; s2.n = mid; s2.dx = -1; }
-        else { s2.x = mid; s2.n = width1 - mid; s2.dx = 1; }
-    } else {
-        __syncthreads();  // the other warp's S stores of its first half are visible before we accumulate onto them
-    }
+    for (int k = 0; k < NP; k++) L[k] = xch[warp ^ 1][lane][k];
+    minL = xch[warp ^ 1][lane][NP];
     scan_run<NP, SCAN_ACCUM, FULL, HPAIR_NST>(a, s2, my_smem, L, minL, lane);
 }
 
@@ -487,101 +437,11 @@ __global__ void __launch_bounds__(64) sgbm_scan_hpair_kernel(const ScanArgs a) {
 // ------------------------------------------------------------------------------------------
 struct WtaArgs {
     const int16_t* S; int16_t* raw; unsigned* disp2key;
-    int W, width1, D, nact, DPL, minD, minX1, uniq, mode;
+    int W, width1, D, nact, DPL, minD, minX1, uniq;
     int HV, nseg;
     int seg_vr0[MAXSEG], seg_y0[MAXSEG], seg_rows[MAXSEG], seg_emit[MAXSEG];
 };
 constexpr int WTA_WARPS = 8;
-
-template <int NP>
-__global__ void __launch_bounds__(WTA_WARPS * 32) sgbm_wta_kernel(const WtaArgs a) {
-    typedef typename VecOf<NP>::T vec;
-    constexpr int DPL = NP * 2;
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const long pix = (long)blockIdx.x * WTA_WARPS + warp;
-    const int width1 = a.width1;
-    if (pix >= (long)a.HV * width1) return;
-    const int vr = (int)(pix / width1), x = (int)(pix - (long)vr * width1);
-    int seg = 0;
-    for (int s = 1; s < a.nseg; s++) if (vr >= a.seg_vr0[s]) seg = s;
-    const int y = a.seg_y0[seg] + (vr - a.seg_vr0[seg]);
-    if (y < a.seg_emit[seg]) return;
-    const int16_t* Sp = a.S + ((size_t)vr * width1 + x) * a.D;
-    uint32_t w[NP];
-    if (lane < a.nact) vec_unpack<NP>(*(const vec*)(Sp + lane * DPL), w);
-    else {
-#pragma unroll
-        for (int k = 0; k < NP; k++) w[k] = INF2;
-    }
-    int s[DPL];
-#pragma unroll
-    for (int k = 0; k < NP; k++) { s[2 * k] = (int)(w[k] & 0xffffu); s[2 * k + 1] = (int)(w[k] >> 16); }
-    const int d0 = lane * DPL;
-    int minS, best;
-    if (a.mode != 2) {
-        unsigned key = 0xffffffffu;
-#pragma unroll
-        for (int j = 0; j < DPL; j++) key = min(key, ((unsigned)s[j] << 8) | (unsigned)((d0 + j) & 255));
-        key = __reduce_min_sync(FULL_MASK, key);
-        minS = (int)(key >> 8); best = (int)(key & 255);
-        if (minS >= 32767) return;  // nothing beats MAX_COST: pixel stays invalid, disp2 untouched
-        bool rej = false;
-#pragma unroll
-        for (int j = 0; j < DPL; j++) {
-            int d = d0 + j;
-            if (lane < a.nact && s[j] * (100 - a.uniq) < minS * 100 && abs(best - d) > 1) rej = true;
-        }
-        if (__any_sync(FULL_MASK, rej)) return;
-    } else {
-        int m = 32767;
-#pragma unroll
-        for (int j = 0; j < DPL; j++) m = min(m, s[j]);
-        minS = __reduce_min_sync(FULL_MASK, m);
-        // OpenCV's 8-lane SIMD arg-min: per residue class d mod 8 the LAST disparity that attains the minimum, then the
-        // smallest of those.  One ballot per register slot j gives the lanes holding the minimum at d = lane * DPL + j;
-        // the classes of a slot are lane patterns (d mod 8 = (lane * DPL + j) mod 8), so "last in class" is the highest
-        // set bit of the ballot under the class's lane mask.
-        best = 0x7fffffff;
-#pragma unroll
-        for (int j = 0; j < DPL; j++) {
-            const unsigned b = __ballot_sync(FULL_MASK, lane < a.nact && s[j] == minS);
-            constexpr int LPC = 8 / DPL > 0 ? 8 / DPL : 1;   // lanes per period of d mod 8 (DPL 2: 4, DPL 4: 2, DPL 8: 1)
-#pragma unroll
-            for (int r = 0; r < LPC; r++) {
-                unsigned pat = 0;                            // lanes with lane % LPC == r
-#pragma unroll
-                for (int l = r; l < 32; l += LPC) pat |= 1u << l;
-                const unsigned m = b & pat;
-                if (m) best = min(best, (31 - __clz(m)) * DPL + j);
-            }
-        }
-        if (a.uniq > 0) {
-            int thresh = (100 * minS) / (100 - a.uniq);
-            int tr = (int)(short)(thresh + 1);
-            bool rej = false;
-#pragma unroll
-            for (int j = 0; j < DPL; j++) {
-                int d = d0 + j;
-                if (lane < a.nact && s[j] < tr && (d < best - 1 || d > best + 1)) rej = true;
-            }
-            if (__any_sync(FULL_MASK, rej)) return;
-        }
-    }
-    if (lane == 0) {
-        int d = best;
-        int x2 = x + a.minX1 - d - a.minD;
-        bool ok2 = (a.mode == 2) ? (x2 >= 0 && x2 < a.W) : (x2 >= 0 && x2 < a.W + 2);
-        if (ok2 && minS < 32767)
-            atomicMax(a.disp2key + (size_t)y * (a.W + 2) + x2, ((unsigned)(0x7fff - minS) << 16) | (unsigned)x);
-        int dd;
-        if (0 < d && d < a.D - 1) {
-            int sm = Sp[d - 1], sp = Sp[d + 1], sc = Sp[d];
-            int denom2 = max(sm + sp - 2 * sc, 1);
-            dd = d * 16 + ((sm - sp) * 16 + denom2) / (denom2 * 2);
-        } else dd = d * 16;
-        a.raw[(size_t)y * a.W + x + a.minX1] = (int16_t)(dd + a.minD * 16);
-    }
-}
 
 // Lean WTA for modes SGBM / HH (single segment): a warp walks 32 consecutive pixels; for each it
 // loads the pixel's S vector (one coalesced 64..512 B access), reduces a packed (cost << 8 | d) key
@@ -589,7 +449,7 @@ __global__ void __launch_bounds__(WTA_WARPS * 32) sgbm_wta_kernel(const WtaArgs 
 // The per-pixel tail (disp2 vote, sub-pixel interpolation with its integer division, store) then
 // runs once for 32 pixels in parallel instead of once per pixel on one lane.
 template <int NP, bool FULL>
-__global__ void __launch_bounds__(WTA_WARPS * 32) sgbm_wta_lean_kernel(const WtaArgs a) {
+__global__ void __launch_bounds__(WTA_WARPS * 32) sgbm_wta_lean_kernel(const __grid_constant__ WtaArgs a) {
     typedef typename VecOf<NP>::T vec;
     constexpr int DPL = NP * 2;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -653,9 +513,9 @@ __global__ void __launch_bounds__(WTA_WARPS * 32) sgbm_wta_lean_kernel(const Wta
 
 // Lean WTA for mode SGBM_3WAY: the same 32-pixels-per-warp walk over the stripe volumes, with that mode's rules (the
 // 8-lane SIMD arg-min, the SIMD form of the uniqueness test, disp2 votes only inside [0, W), overlap rows of a stripe
-// not emitted) -- see sgbm_wta_kernel for the per-pixel restatement this kernel batches.
+// not emitted).
 template <int NP>
-__global__ void __launch_bounds__(WTA_WARPS * 32) sgbm_wta_lean3_kernel(const WtaArgs a) {
+__global__ void __launch_bounds__(WTA_WARPS * 32) sgbm_wta_lean3_kernel(const __grid_constant__ WtaArgs a) {
     typedef typename VecOf<NP>::T vec;
     constexpr int DPL = NP * 2;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -694,14 +554,18 @@ __global__ void __launch_bounds__(WTA_WARPS * 32) sgbm_wta_lean3_kernel(const Wt
 #pragma unroll
         for (int j = 0; j < DPL; j++) m = min(m, sv[j]);
         const int minS = __reduce_min_sync(FULL_MASK, m);
+        // OpenCV's 8-lane SIMD arg-min: per residue class d mod 8 the LAST disparity that attains the minimum, then the
+        // smallest of those.  One ballot per register slot j gives the lanes holding the minimum at d = lane * DPL + j;
+        // the classes of a slot are lane patterns (d mod 8 = (lane * DPL + j) mod 8), so "last in class" is the highest
+        // set bit of the ballot under the class's lane mask.
         int best = 0x7fffffff;
 #pragma unroll
         for (int j = 0; j < DPL; j++) {
             const unsigned b = __ballot_sync(FULL_MASK, active && sv[j] == minS);
-            constexpr int LPC = 8 / DPL > 0 ? 8 / DPL : 1;
+            constexpr int LPC = 8 / DPL > 0 ? 8 / DPL : 1;   // lanes per period of d mod 8 (DPL 2: 4, DPL 4: 2, DPL 8: 1)
 #pragma unroll
             for (int r = 0; r < LPC; r++) {
-                unsigned pat = 0;
+                unsigned pat = 0;                            // lanes with lane % LPC == r
 #pragma unroll
                 for (int l = r; l < 32; l += LPC) pat |= 1u << l;
                 const unsigned mm = b & pat;
@@ -786,15 +650,12 @@ static int launch_scan_t(Lane& L, const ScanArgs& sa, int lines) {
 template <int NP>
 static int launch_hpair(Lane& L, const ScanArgs& sa0) {
     const size_t smem = 2 * scan_smem_bytes_dev(sa0.D);
-    static const int hp_mode = getenv("L3D_HPAIR_MODE") ? atoi(getenv("L3D_HPAIR_MODE")) : 1;
     // Row slices.  Alone, ONE launch over all rows is fastest (the two serial recurrences per row need every row in flight
     // to cover their latency: 0.168 ms against 0.213 ms in three slices at config 3) -- that is what single calls and the
     // kernel-timing leg use.  Inside the frame pipeline three slices let the other streams' kernels (above all the
-    // aggregation clusters, which need whole free SMs) start sooner: +2 % frames/s (tools/skip_probe.py, L3D_HPAIR_WAVES).
-    static const int hp_waves_env = getenv("L3D_HPAIR_WAVES") ? std::max(1, atoi(getenv("L3D_HPAIR_WAVES"))) : 0;
-    const int hp_waves = hp_waves_env ? hp_waves_env : ((L.back_stream && !L.timing && sa0.HV >= 360) ? 3 : 1);
+    // aggregation clusters, which need whole free SMs) start sooner: +2 % frames/s (tools/skip_probe.py).
+    const int hp_waves = (L.back_stream && !L.timing && sa0.HV >= 360) ? 3 : 1;
     ScanArgs sa = sa0;
-    sa.hp_mode = hp_mode;
     const int per = cdiv(sa.HV, hp_waves);
     for (int r0 = 0; r0 < sa.HV; r0 += per) {
         const int rows = std::min(per, sa.HV - r0);
@@ -835,10 +696,7 @@ static void scan_args_of(const SgbmRun& r, ScanArgs& sa) {
     sa.HV = g.HV; sa.nseg = g.nseg;
     for (int s = 0; s < MAXSEG; s++) { sa.seg_vr0[s] = g.seg_vr0[s]; sa.seg_rows[s] = g.seg_rows[s]; }
     sa.raw = r.raw; sa.disp2key = r.d2; sa.W = r.W; sa.minD = g.minD; sa.minX1 = g.minX1; sa.uniq = g.uniq;
-    sa.kind = 0; sa.store = 1; sa.lines_per_seg = 0; sa.zero = 0; sa.hp_mode = 0; sa.hp_row0 = 0;
-    sa.tway = g.mode == 2;
-    // (the winner-takes-all stage maps volume rows to OUTPUT rows: the stripe's first image row minus its shift, make_geom)
-    for (int s = 0; s < MAXSEG; s++) { sa.seg_y0[s] = g.seg_y0[s] - g.seg_shift[s]; sa.seg_emit[s] = g.seg_emit[s]; }
+    sa.kind = 0; sa.store = 1; sa.lines_per_seg = 0; sa.zero = 0; sa.hp_row0 = 0;
 }
 
 // front, first part: geometry, invalid-filled raw image, scratch volumes, disp2 vote buffer
@@ -916,8 +774,7 @@ int sgbm_front_pair(Lane& L, const l3d_sgbm_params& pl, const l3d_sgbm_params& p
     if (rl.g.width1 <= 0 && rr.g.width1 <= 0) return L3D_OK;
     if ((rc = sgbm_prefilter(L, left, W, H, rl.g.ftzero, dL)) != L3D_OK) return rc;
     if ((rc = sgbm_prefilter(L, right, W, H, rl.g.ftzero, dR)) != L3D_OK) return rc;
-    static const bool no_dual = getenv("L3D_COST_NO_DUAL") != nullptr;
-    if (!no_dual && rl.g.width1 > 0 && rr.g.width1 > 0 && sgbm_cost_dual_ok(rl.g, rr.g)) {
+    if (rl.g.width1 > 0 && rr.g.width1 > 0 && sgbm_cost_dual_ok(rl.g, rr.g)) {
         L.t_begin("sgbm_cost");
         rc = sgbm_cost_dual(L, rl.g, rr.g, dL, dR, rl.C, rr.C);
         L.t_end("sgbm_cost");
@@ -956,10 +813,9 @@ int sgbm_middle_split(Lane& L, SgbmRun& r, bool keep_S) {
     if (g.mode <= 1) { kinds[nk++] = 3; kinds[nk++] = 4; }
     if (g.mode == 1) { kinds[nk++] = 5; kinds[nk++] = 6; kinds[nk++] = 7; }
     if (g.mode == 3) kinds[nk++] = 5;  // HH4: horizontal pair (front) + down + up
-    // SGBM_3WAY: the stand-alone lean WTA is faster than the fused form (measured 834 vs 696 frames/s at 1280x720: the
-    // arg-min ballots sit on the scan's serial chain), so fusing is opt-in there
-    static const bool fuse3 = getenv("L3D_3WAY_FUSE_WTA") != nullptr;
-    const bool fuse_wta = !keep_S && (g.mode != 2 || fuse3);
+    // SGBM_3WAY keeps the stand-alone lean WTA: fused into the last scan it was slower (834 -> 696 frames/s at 1280x720:
+    // the arg-min ballots sit on the scan's serial chain)
+    const bool fuse_wta = !keep_S && g.mode != 2;
     for (int i = 0; i < nk; i++) {
         const int k = kinds[i];
         sa.kind = k; sa.store = 0;
@@ -986,38 +842,30 @@ int sgbm_back(Lane& L, SgbmRun& r, int16_t* disp, SgbmDebug* dbg) {
     if (g.width1 > 0) {
         WtaArgs wa;
         wa.S = r.S; wa.raw = r.raw; wa.disp2key = r.d2; wa.W = W; wa.width1 = g.width1; wa.D = g.D; wa.nact = g.nact;
-        wa.DPL = g.DPL; wa.minD = g.minD; wa.minX1 = g.minX1; wa.uniq = g.uniq; wa.mode = g.mode;
+        wa.DPL = g.DPL; wa.minD = g.minD; wa.minX1 = g.minX1; wa.uniq = g.uniq;
         wa.HV = g.HV; wa.nseg = g.nseg;
         for (int s = 0; s < MAXSEG; s++) {
             wa.seg_vr0[s] = g.seg_vr0[s]; wa.seg_y0[s] = g.seg_y0[s] - g.seg_shift[s]; wa.seg_rows[s] = g.seg_rows[s]; wa.seg_emit[s] = g.seg_emit[s];
         }
-        if (!r.wta_done) L.t_begin("sgbm_wta");   // (fused into the last aggregation pass otherwise: nothing to time here)
-        if (r.wta_done) {
-        } else if (g.mode != 2) {
+        if (!r.wta_done) {  // (fused into the last aggregation pass otherwise: nothing to time here)
+            L.t_begin("sgbm_wta");
             const int wgrid = cdiv(cdiv((long)g.HV * g.width1, 32), WTA_WARPS);
-            const bool full = g.nact == 32;
+            if (g.mode != 2) {
+                const bool full = g.nact == 32;
 #define L3D_WTA(NPV)                                                                                         \
     do {                                                                                                     \
         if (full) L3D_LAUNCH(L, (sgbm_wta_lean_kernel<NPV, true>), wgrid, WTA_WARPS * 32, 0, wa);            \
         else L3D_LAUNCH(L, (sgbm_wta_lean_kernel<NPV, false>), wgrid, WTA_WARPS * 32, 0, wa);                \
     } while (0)
-            if (g.NP == 1) L3D_WTA(1); else if (g.NP == 2) L3D_WTA(2); else L3D_WTA(4);
+                if (g.NP == 1) L3D_WTA(1); else if (g.NP == 2) L3D_WTA(2); else L3D_WTA(4);
 #undef L3D_WTA
-        } else {
-            static const bool per_pixel = getenv("L3D_WTA_PER_PIXEL") != nullptr;  // the warp-per-pixel restatement
-            if (per_pixel) {
-                const int wgrid = cdiv((long)g.HV * g.width1, WTA_WARPS);
-                if (g.NP == 1) L3D_LAUNCH(L, sgbm_wta_kernel<1>, wgrid, WTA_WARPS * 32, 0, wa);
-                else if (g.NP == 2) L3D_LAUNCH(L, sgbm_wta_kernel<2>, wgrid, WTA_WARPS * 32, 0, wa);
-                else L3D_LAUNCH(L, sgbm_wta_kernel<4>, wgrid, WTA_WARPS * 32, 0, wa);
             } else {
-                const int wgrid = cdiv(cdiv((long)g.HV * g.width1, 32), WTA_WARPS);
                 if (g.NP == 1) L3D_LAUNCH(L, sgbm_wta_lean3_kernel<1>, wgrid, WTA_WARPS * 32, 0, wa);
                 else if (g.NP == 2) L3D_LAUNCH(L, sgbm_wta_lean3_kernel<2>, wgrid, WTA_WARPS * 32, 0, wa);
                 else L3D_LAUNCH(L, sgbm_wta_lean3_kernel<4>, wgrid, WTA_WARPS * 32, 0, wa);
             }
+            L.t_end("sgbm_wta");
         }
-        if (!r.wta_done) L.t_end("sgbm_wta");
         L3D_LAUNCH(L, sgbm_lrcheck_kernel, dim3(cdiv(g.width1, 128), H), 128, 0, r.raw, r.d2, W, H, g.minX1, g.maxX1, g.minD, g.d12);
         if (dbg) {
             const size_t nvol = (size_t)g.HV * g.width1 * g.D;
@@ -1067,10 +915,9 @@ int sgbm_middle_vgroup(Lane& L, SgbmRun* const* runs, int nruns, bool keep_S) {
 // L3D_VWAVE (read at every call, so that a test can switch it): 0 = never, 1 = wherever the kernel covers the geometry,
 // unset = where it is the faster choice (vwave_pays)
 bool sgbm_vwave_ok(int width1, int H, int D, int mode) {
-    static const bool off = getenv("L3D_NO_VWAVE") && atoi(getenv("L3D_NO_VWAVE")) > 0;
     const char* e = getenv("L3D_VWAVE");
     const int policy = e ? atoi(e) : -1;
-    if (off || policy == 0 || mode != 1 || width1 <= 0) return false;
+    if (policy == 0 || mode != 1 || width1 <= 0) return false;
     return policy == 1 ? vwave_supported(width1, H, D) : vwave_pays(width1, H, D);
 }
 

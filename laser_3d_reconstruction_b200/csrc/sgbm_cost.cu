@@ -5,9 +5,12 @@
 //
 // Kernels:
 //   sgbm_prefilter_kernel     x-Sobel clip + half-pixel min/max, as pixel-pair operand entries (2 planes x 16 B / pixel)
-//   sgbm_cost_warp_kernel     Birchfield-Tomasi pixel cost -> blockSize^2 box sum -> C (+P2); disparity pairs split over
-//                             the warps, warp-private cost strips and row-sum rings, TMA operand ring, no block barrier
-//   sgbm_cost_kernel          the block-synchronous form (D = 256 and every other geometry)
+//   sgbm_cost_dual_kernel     Birchfield-Tomasi pixel cost -> blockSize^2 box sum -> C (+P2) of one or both matchers of a
+//                             frame: single-segment volumes at block 5 / D 64, block 9 / D 128, block 11 / D 256
+//   sgbm_cost_warp_kernel     the same sums for one volume, disparity pairs split over the warps, warp-private cost strips
+//                             and row-sum rings, TMA operand ring, no block barrier: SGBM_3WAY's striped volumes at
+//                             block 5 / D 64 and block 9 / D 128 (the dual kernel takes no segments)
+//   sgbm_cost_kernel          the block-synchronous form: every other geometry, SGBM_3WAY's at block 11 / D 256 among them
 #include "sgbm.cuh"
 
 namespace l3d {
@@ -92,7 +95,6 @@ struct CostArgs {
     int W, H, minD, D, minX1, width1, SW2, bs, P2, TX, TXH;
     int nxg, cpg;  // phase B: column groups per CTA, columns per group
     unsigned* flags;  // bit 0 is set when a cost value reaches 32768 (OpenCV's int16 would wrap there; see make_geom)
-    int dbg;       // L3D_COST_DBG experiment bits: 1 no C stores, 2 no phase B, 4 no phase A (results are garbage)
     int nbands;
     int band_vr0[MAXBAND], band_y0[MAXBAND], band_rows[MAXBAND], band_clo[MAXBAND], band_chi[MAXBAND];
 };
@@ -414,7 +416,6 @@ __global__ void __launch_bounds__(COST_THREADS, 1) sgbm_cost_warp_kernel(const C
         cost_mbar_wait(bars + 8 * s, (uint32_t)((k / CW_NS) & 1));
         const uint4* T0 = tabs + s * STAGE_U4;
         // ---- phase A
-        if (!(a.dbg & 4))
 #pragma unroll
         for (int hh = 0; hh < 2; hh++) {
             const uint4 l0 = T0[2 * NEMAX + lcol[hh]], l1 = T0[2 * NEMAX + TXH + lcol[hh]];
@@ -438,7 +439,7 @@ __global__ void __launch_bounds__(COST_THREADS, 1) sgbm_cost_warp_kernel(const C
         __syncwarp();  // strip complete; every lane's table reads have returned
         if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bars + 8 * (CW_NS + s)) : "memory");
         // ---- phase B
-        if (ncb > 0 && !(a.dbg & 2)) {
+        if (ncb > 0) {
             uint32_t* rp = rpb + (size_t)slot * DPW * TX;
             const bool sub = k >= BS, emit = k >= BS - 1;
             constexpr int NV = CPG + BS - 1;
@@ -461,7 +462,7 @@ __global__ void __launch_bounds__(COST_THREADS, 1) sgbm_cost_warp_kernel(const C
                 if (j < ncb) {
                     rp[j] = hs[j];
                     ovf |= crun[j];
-                    if (emit && !((a.dbg & 1) && crun[j] != 0x12345u)) Cdst[(size_t)j * D2] = crun[j];
+                    if (emit) Cdst[(size_t)j * D2] = crun[j];
                 }
             }
         }
@@ -506,8 +507,6 @@ struct DualArgs {
     int x1[CD_MAXT1];
     int emit, RA, RB;           // role-0 tiles also write columns RA <= x' < RB of C[1]
     unsigned* flags;            // bit 0 is set when a cost value reaches 32768 (OpenCV's int16 would wrap there)
-    int cta0;                   // first CTA of this launch (a launch may be split so that other streams' kernels get in between)
-    int dbg;
 };
 
 template <int BS, int DD>
@@ -550,7 +549,7 @@ __global__ void __launch_bounds__(COST_THREADS, 1) sgbm_cost_dual_kernel(const D
     const int lane = threadIdx.x & 31;
     const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);
     // ---- CTA -> (role, tile, band)
-    int cta = a.cta0 + blockIdx.x;
+    int cta = blockIdx.x;
     const int n0 = a.ntiles[0] * a.nbands[0];
     const int role = cta >= n0 ? 1 : 0;
     if (role) cta -= n0;
@@ -638,22 +637,20 @@ __global__ void __launch_bounds__(COST_THREADS, 1) sgbm_cost_dual_kernel(const D
     auto write_out = [&](int er) {  // emitted row er of the band (image row y0 + er), staged in Ls[er & 1]
         const uint32_t* ls = Ls + (er & 1) * TX * CS;
         const size_t rowbase = (size_t)(y0 + er) * width1;
-        if (!(a.dbg & 1)) {
-            if (CS % 4 == 0) {
-                constexpr int CPC = D2 / 4;                    // 16-byte chunks per column
-                for (int q = threadIdx.x; q < ncopy * CPC; q += COST_THREADS) {
-                    const int col = q / CPC, part = q - col * CPC;
-                    const uint4 v = *(const uint4*)(ls + col * CS + part * 4);
-                    *(uint4*)(Cown32 + (rowbase + x0 + col) * D2 + part * 4) = v;
-                }
-            } else {
-                for (int q = threadIdx.x; q < ncopy * D2; q += COST_THREADS) {
-                    const int col = q / D2, part = q - col * D2;
-                    Cown32[(rowbase + x0 + col) * D2 + part] = ls[col * CS + part];
-                }
+        if (CS % 4 == 0) {
+            constexpr int CPC = D2 / 4;                    // 16-byte chunks per column
+            for (int q = threadIdx.x; q < ncopy * CPC; q += COST_THREADS) {
+                const int col = q / CPC, part = q - col * CPC;
+                const uint4 v = *(const uint4*)(ls + col * CS + part * 4);
+                *(uint4*)(Cown32 + (rowbase + x0 + col) * D2 + part * 4) = v;
+            }
+        } else {
+            for (int q = threadIdx.x; q < ncopy * D2; q += COST_THREADS) {
+                const int col = q / D2, part = q - col * D2;
+                Cown32[(rowbase + x0 + col) * D2 + part] = ls[col * CS + part];
             }
         }
-        if (emitR && !(a.dbg & 8)) {
+        if (emitR) {
             // units (wrapped line s, 32-word piece h) are dealt to the warps round robin: unit = warp + NW i, so a warp
             // keeps its piece h = warp % NH and its line advances by NW / NH per unit -- column, staged-row address and
             // global address all move by constants (with one conditional wrap)
@@ -689,7 +686,6 @@ __global__ void __launch_bounds__(COST_THREADS, 1) sgbm_cost_dual_kernel(const D
             cost_mbar_wait(bars + 8 * s, (uint32_t)((k / CD_NS) & 1));
             const uint4* T0 = tabs + s * STAGE_U4;
             // ---- phase A
-            if (!(a.dbg & 4))
 #pragma unroll
             for (int hh = 0; hh < NHH; hh++) {
                 const uint4 l0 = T0[2 * NEMAX + lcol[hh]], l1 = T0[2 * NEMAX + TXH + lcol[hh]];
@@ -719,7 +715,7 @@ __global__ void __launch_bounds__(COST_THREADS, 1) sgbm_cost_dual_kernel(const D
             // ---- phase B
             const bool emit = e >= 0;
             if (e >= 2) cost_mbar_wait(bar_lse + 8 * (e & 1), (uint32_t)(((e >> 1) - 1) & 1));  // row e - 2 written out
-            if (ncb > 0 && !(a.dbg & 2)) {
+            if (ncb > 0) {
                 uint32_t* rp = rpb + (size_t)slot * DPW * TX;
                 uint32_t* lp = lsb + (e & 1) * TX * CS;
                 const bool sub = k >= BS;
@@ -798,8 +794,6 @@ int sgbm_cost_single(Lane& L, const Geom& g, const uint4* dL, const uint4* dR, i
     ca.Ldesc = dL; ca.Rdesc = dR; ca.C = C;
     ca.W = W; ca.H = H; ca.minD = g.minD; ca.D = g.D; ca.minX1 = g.minX1; ca.width1 = g.width1;
     ca.SW2 = g.SW2; ca.bs = g.bs; ca.P2 = g.P2; ca.flags = L.flags;
-    static const int cost_dbg = getenv("L3D_COST_DBG") ? atoi(getenv("L3D_COST_DBG")) : 0;
-    ca.dbg = cost_dbg;
     const int D2 = g.D / 2;
     auto cost_smem = [&](int txh) {
         int tx = txh - 2 * g.SW2;
@@ -815,10 +809,9 @@ int sgbm_cost_single(Lane& L, const Geom& g, const uint4* dL, const uint4* dR, i
     ca.TXH = TXH; ca.TX = TXH - 2 * g.SW2;
     ca.cpg = cdiv(ca.TX, ca.nxg);
     size_t smem = cost_smem(TXH);
-    static const bool no_warp_cost = getenv("L3D_COST_CLASSIC") != nullptr;
-    static const bool no_staged = getenv("L3D_COST_NO_STAGED") != nullptr;
-    const bool warp_form = !no_warp_cost && ((g.D == 128 && g.bs == 9) || (g.D == 64 && g.bs == 5));
-    if (!no_warp_cost && !no_staged && g.nseg == 1 && cost_dual_cfg(g.bs, g.D)) return cost_single_staged(L, g, dL, dR, C);
+    if (g.nseg == 1 && cost_dual_cfg(g.bs, g.D)) return cost_single_staged(L, g, dL, dR, C);
+    // from here on: SGBM_3WAY's striped volumes (nseg > 1) and the geometries the staged kernel is not instantiated for
+    const bool warp_form = (g.D == 128 && g.bs == 9) || (g.D == 64 && g.bs == 5);
     if (warp_form) {
         // warp-decoupled form: 64-column tiles
         ca.TXH = CW_TXH; ca.TX = CW_TXH - 2 * g.SW2;
@@ -826,8 +819,7 @@ int sgbm_cost_single(Lane& L, const Geom& g, const uint4* dL, const uint4* dR, i
     }
     // the grid is close to one wave of CTAs (one CTA per SM: the row-sum ring takes most of the shared memory)
     const int xtiles = cdiv(g.width1, ca.TX);
-    static const int waves = getenv("L3D_COST_WAVES") ? atoi(getenv("L3D_COST_WAVES")) : 1;
-    cost_bands(g, H, std::max(1, (waves * NUM_SMS) / xtiles), ca);
+    cost_bands(g, H, std::max(1, NUM_SMS / xtiles), ca);
     const int dpa_step = COST_THREADS / TXH;
     const int nit = (D2 % dpa_step == 0) ? D2 / dpa_step : 0;
 #define COST_CASE(KERN)                                                                                          \
@@ -835,11 +827,9 @@ int sgbm_cost_single(Lane& L, const Geom& g, const uint4* dL, const uint4* dR, i
         L3D_CHECK(L, cudaFuncSetAttribute(KERN, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));       \
         L3D_LAUNCH(L, KERN, dim3(xtiles, ca.nbands), COST_THREADS, smem, ca);                                    \
     }
-    // specialised for the configurations of BASELINE.json (c3: D 128 / block 9, c1-c2: D 64 / block 5, c4: D 256 / block 11)
+    // specialised for the configurations of BASELINE.json (c1-c2: D 64 / block 5, c3: D 128 / block 9, c4: D 256 / block 11)
     if (warp_form && g.D == 128) COST_CASE((sgbm_cost_warp_kernel<9, 128>))
     else if (warp_form) COST_CASE((sgbm_cost_warp_kernel<5, 64>))
-    else if (nit == 8 && g.bs == 9 && g.D == 128 && TXH == 64) COST_CASE((sgbm_cost_kernel<8, 9, 128, 64>))
-    else if (nit == 4 && g.bs == 5 && g.D == 64 && TXH == 64) COST_CASE((sgbm_cost_kernel<4, 5, 64, 64>))
     else if (nit == 8 && g.bs == 11 && g.D == 256 && TXH == 32) COST_CASE((sgbm_cost_kernel<8, 11, 256, 32>))
     else COST_CASE((sgbm_cost_kernel<0, 0, 0, 0>))
 #undef COST_CASE
@@ -855,13 +845,7 @@ static int launch_cost_dual(Lane& L, const DualArgs& da) {
     const int ncta = da.ntiles[0] * da.nbands[0] + da.ntiles[1] * da.nbands[1];
     L3D_CHECK(L, cudaFuncSetAttribute((sgbm_cost_dual_kernel<BS, DD>), cudaFuncAttributeMaxDynamicSharedMemorySize,
                                       (int)K::smem_bytes()));
-    static const int split = getenv("L3D_COST_SPLIT") ? std::max(1, atoi(getenv("L3D_COST_SPLIT"))) : 1;
-    const int per = cdiv(ncta, split);
-    DualArgs d = da;
-    for (int c0 = 0; c0 < ncta; c0 += per) {
-        d.cta0 = c0;
-        L3D_LAUNCH(L, (sgbm_cost_dual_kernel<BS, DD>), std::min(per, ncta - c0), COST_THREADS, K::smem_bytes(), d);
-    }
+    L3D_LAUNCH(L, (sgbm_cost_dual_kernel<BS, DD>), ncta, COST_THREADS, K::smem_bytes(), da);
     return L3D_OK;
 }
 static int launch_cost_dual_any(Lane& L, int bs, int D, const DualArgs& da) {
@@ -921,8 +905,6 @@ static int cost_single_staged(Lane& L, const Geom& g, const uint4* dL, const uin
     }
     da.nbands[0] = it->second;
     da.emit = 0; da.RA = da.RB = 0; da.flags = L.flags;
-    static const int cost_dbg = getenv("L3D_COST_DBG") ? atoi(getenv("L3D_COST_DBG")) : 0;
-    da.dbg = cost_dbg;
     return launch_cost_dual_any(L, g.bs, g.D, da);
 }
 
@@ -967,8 +949,6 @@ int sgbm_cost_dual(Lane& L, const Geom& gl, const Geom& gr, const uint4* dLv, co
         it = cache.emplace(key, std::make_pair(b0, b1)).first;
     }
     da.nbands[0] = it->second.first; da.nbands[1] = it->second.second;
-    static const int cost_dbg = getenv("L3D_COST_DBG") ? atoi(getenv("L3D_COST_DBG")) : 0;
-    da.dbg = cost_dbg;
     if (getenv("L3D_DEBUG_CLUSTERS"))
         fprintf(stderr, "[l3d] cost dual: %d x %d + %d x %d CTAs, RA %d RB %d\n", da.ntiles[0], da.nbands[0], nt1, da.nbands[1], da.RA, da.RB);
     return launch_cost_dual_any(L, gl.bs, D, da);

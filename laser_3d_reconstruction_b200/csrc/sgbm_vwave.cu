@@ -61,17 +61,11 @@ static bool vwave_shape(int width1, int D, int& cluster, int& cpw) {
         return true;
     }
     if (!(D == 64 || D == 128)) return false;
-    // L3D_VWAVE_CLUSTER=n tries an n-CTA cluster first (any size up to 16; experiments and the 8-vs-9 comparison)
-    static const int forced = getenv("L3D_VWAVE_CLUSTER") ? atoi(getenv("L3D_VWAVE_CLUSTER")) : 0;
-    if (forced >= 1 && forced <= 16) {
-        const int c = cdiv(width1, forced * vwave_warps(D));
-        if (c <= VW_MAXCPW && c >= 2 && vwave_smem_bytes(D, c, true) <= 227 * 1024) { cluster = forced; cpw = c; return true; }
-    }
     // Nine CTAs where they cover the volume exactly with fewer columns per warp than eight would need (config 3: 1152 =
     // 9 x 16 x 8 instead of 8 x 16 x 9).  Two 9-CTA clusters fit a 20-SM GPC like two 8-CTA ones, so the 14 volumes of a
     // lane set are still one wave, on 126 SMs instead of 112: 0.141 + 0.181 -> 0.126 + 0.161 ms per run alone; the frame
     // pipeline, whose other streams were using the 36 free SMs, is unchanged (1124 vs 1119 frames/s).
-    if (forced == 0 && width1 % (9 * vwave_warps(D)) == 0) {
+    if (width1 % (9 * vwave_warps(D)) == 0) {
         const int c = width1 / (9 * vwave_warps(D));
         // ... provided this GPU keeps a lane set's 14 volumes resident as 9-CTA clusters too (one wave per launch)
         if (c >= 2 && c < cdiv(width1, 8 * vwave_warps(D)) && c <= VW_MAXCPW && vwave_smem_bytes(D, c, true) <= 227 * 1024 &&

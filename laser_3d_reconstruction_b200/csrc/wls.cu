@@ -603,13 +603,11 @@ static int wls_lut(Lane& L, double sigma, float** out) {
 // The FGS passes of the WLS filter (dev_wls; l3d_fgs_solve runs them alone): `iters` iterations of (row solves with
 // weights ch, column solves with weights cv) on num/den in place; Dscr (w x h) is scratch of the serial kernels.
 // solver: 0 = partitioned parallel solves (default), 1 = serial solves in the oracle's operation order (bit-identical
-// to oracle/csrc/orc_wls.c); L3D_FGS_SERIAL=1 forces the serial form everywhere, and so do lines longer than
-// FGSP_W_MAX / FGSP_H_MAX or shorter than 2.
+// to oracle/csrc/orc_wls.c); lines longer than FGSP_W_MAX / FGSP_H_MAX or shorter than 2 take the serial form too.
 int dev_fgs(Lane& L, int solver, int variant, double lambda, int iters, const float* ch, const float* cv, int w, int h,
             float* num, float* den, float* Dscr, bool* parallel_used) {
     float lam = (float)lambda;
-    static const bool force_serial = getenv("L3D_FGS_SERIAL") && atoi(getenv("L3D_FGS_SERIAL")) > 0;
-    const bool parallel = !force_serial && solver != 1 && w <= FGSP_W_MAX && h <= FGSP_H_MAX && w >= 2 && h >= 2;
+    const bool parallel = solver != 1 && w <= FGSP_W_MAX && h <= FGSP_H_MAX && w >= 2 && h >= 2;
     *parallel_used = parallel;
     const size_t smr = fgsp_rows_smem(w);
     int nc = 8;  // columns per CTA: 16 where a 16-column CTA fits an SM, else 8

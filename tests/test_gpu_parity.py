@@ -316,7 +316,7 @@ def test_sgbm_properties_full_size(ctx):
 @pytest.mark.parametrize("bs,H", [(11, 8), (11, 20), (11, 24), (11, 28), (9, 20), (5, 12), (3, 8), (9, 5)])
 def test_sgbm_3way_tiny_images(ctx, bs, H):
     """SGBM_3WAY on images of a few rows: OpenCV's shifted stripe rows (tests/test_oracle_cv2.py has the story) on the GPU,
-    through the stand-alone and the fused winner-takes-all."""
+    through that mode's stand-alone winner-takes-all, with and without the raw disparity read back."""
     for D, W, seed in ((48, 194, 5), (16, 90, 9)):
         lg, rg = gray_pair(W, H, D, seed)
         for (uq, d12, sw) in ((0, 5, 200), (10, 1, 0)):
@@ -326,7 +326,7 @@ def test_sgbm_3way_tiny_images(ctx, bs, H):
             p = N.SgbmParams(**kw)
             eq(ctx.sgbm_compute(p, lg, rg), want, "3way tiny %s" % ((bs, H, D, uq),))
             disp, raw = ctx.sgbm_compute(p, lg, rg, want_raw=True)
-            eq(disp, want, "3way tiny (S kept) %s" % ((bs, H, D, uq),))
+            eq(disp, want, "3way tiny (raw read back) %s" % ((bs, H, D, uq),))
 
 
 @pytest.mark.parametrize("H", [1, 2, 3, 5, 8])
@@ -868,38 +868,3 @@ def test_grouped_pipeline_without_wls_uniqueness(ctx, W, H, D, bs):
         cv2.cvtColor(lrect, cv2.COLOR_BGR2GRAY), cv2.cvtColor(rrect, cv2.COLOR_BGR2GRAY))
     eq(results[15][8]["disp16"], want, "no-WLS grouped disparity vs cv2")
 
-
-@pytest.mark.parametrize("switch,cases", [
-    ("L3D_COST_CLASSIC", ((320, 360, 64, 5, 0), (1280, 720, 128, 9, 1))),      # block-synchronous cost kernel
-    ("L3D_3WAY_FUSE_WTA", ((320, 360, 64, 5, 2), (1280, 200, 128, 9, 2))),     # SGBM_3WAY WTA fused into the last scan
-    ("L3D_WTA_PER_PIXEL", ((320, 360, 64, 5, 2), (640, 120, 128, 9, 2))),      # warp-per-pixel SGBM_3WAY WTA
-])
-def test_alternative_kernel_forms(switch, cases):
-    """Kernel forms that are not the default (selected by an environment switch that is read once per process, hence the
-    subprocess) still give cv2's bits."""
-    import os
-    import subprocess
-    import sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    code = r"""
-import sys, numpy as np, cv2
-sys.path.insert(0, %r)
-from laser_3d_reconstruction_b200 import _native as N, synth
-ctx = N.Context(0)
-for (W, H, D, bs, mode) in %r:
-    l, r = synth.stereo_pair(W, H, D, seed=5)
-    lg, rg = cv2.cvtColor(l, cv2.COLOR_BGR2GRAY), cv2.cvtColor(r, cv2.COLOR_BGR2GRAY)
-    for minD, a, b in ((0, lg, rg), (-(D - 1), rg, lg)):
-        for uq, d12, sw in ((10, 1, 100), (0, 1000000, 0)):
-            p = N.SgbmParams(minD, D, bs, 24 * bs * bs, 96 * bs * bs, d12, 63, uq, sw, 32, mode)
-            want = cv2.StereoSGBM_create(minDisparity=minD, numDisparities=D, blockSize=bs, P1=24 * bs * bs, P2=96 * bs * bs,
-                                         disp12MaxDiff=d12, preFilterCap=63, uniquenessRatio=uq, speckleWindowSize=sw,
-                                         speckleRange=32, mode=mode).compute(a, b)
-            got = ctx.sgbm_compute(p, a, b)
-            assert np.array_equal(got, want), (W, H, D, bs, mode, minD, uq, int((got != want).sum()))
-print("alternative form ok")
-""" % (root, tuple(cases))
-    env = dict(os.environ)
-    env[switch] = "1"
-    res = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, timeout=600)
-    assert res.returncode == 0 and "alternative form ok" in res.stdout, res.stdout + res.stderr
