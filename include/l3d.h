@@ -84,7 +84,9 @@ int l3d_bm_compute(l3d_ctx* ctx, const l3d_bm_params* p, const uint8_t* left, co
 typedef struct {
     int minDisparity, numDisparities, blockSize, P1, P2, disp12MaxDiff, preFilterCap,
         uniquenessRatio, speckleWindowSize, speckleRange, mode;
-} l3d_sgbm_params; /* cv2.StereoSGBM_create arguments, camera/single_usb_stereo_camera.py:252-274 */
+} l3d_sgbm_params; /* cv2.StereoSGBM_create arguments, camera/single_usb_stereo_camera.py:252-274;
+                    * numDisparities: a multiple of 16 in [16, 512] in every mode; blockSize: odd in [1, 21], and at most 15
+                    * when numDisparities > 272 (L3D_ERR_UNSUPPORTED otherwise) */
 
 /* cv2.StereoSGBM.compute(left, right) -> int16 disparity x16
  * (camera/single_usb_stereo_camera.py:324-325, test_improved_laser.py:151, test_depth.py:68) */

@@ -5,8 +5,8 @@
 //
 // HBM layout: cost volume C and aggregated volume S are int16 [vrow][x][d] (d fastest), x in
 // width1 = maxX1-minX1 coordinates.  A warp owns one pixel's disparity range: lane l holds DPL
-// consecutive disparities packed as u16x2 words (DPL = 2/4/8 for D <= 64/128/256), so one warp
-// access is one contiguous 64..512 B segment.
+// consecutive disparities packed as u16x2 words (DPL = 2/4/8/16 for D <= 64/128/256/512), so one warp
+// access is one contiguous 64..1024 B segment.
 //
 // Kernels:
 //   sgbm_prefilter_kernel     x-Sobel clip + half-pixel min/max, as pixel-pair operand entries (2 planes x 16 B / pixel)
@@ -41,12 +41,19 @@ int make_geom(const l3d_sgbm_params& p, int W, int H, Geom& g, std::string* err)
     g.W = W; g.H = H; g.minD = p.minDisparity; g.D = p.numDisparities; g.maxD = g.minD + g.D;
     g.mode = p.mode;
     if (W < 2 || H < 1) { set_err(err, "sgbm: image too small"); return L3D_ERR_ARG; }
-    if (g.D < 16 || g.D > 256 || (g.D % 16)) {
-        set_err(err, "sgbm: numDisparities must be a multiple of 16 in [16,256], got %d", g.D);
+    if (g.D < 16 || g.D > 512 || (g.D % 16)) {
+        set_err(err, "sgbm: numDisparities must be a multiple of 16 in [16,512], got %d", g.D);
         return L3D_ERR_UNSUPPORTED;
     }
     if (p.blockSize < 1 || !(p.blockSize & 1) || p.blockSize > 21) {
         set_err(err, "sgbm: blockSize must be odd in [1,21], got %d", p.blockSize);
+        return L3D_ERR_UNSUPPORTED;
+    }
+    // Above 272 disparities the block-synchronous cost kernel's row-sum ring leaves room for tiles of 16 computed
+    // columns only (sgbm_cost_single), and a tile must be wider than the window's 2 * (blockSize / 2) halo columns.
+    if (g.D > 272 && p.blockSize > 15) {
+        set_err(err, "sgbm: blockSize %d with numDisparities %d unsupported (blockSize <= 15 above 272 disparities)",
+                p.blockSize, g.D);
         return L3D_ERR_UNSUPPORTED;
     }
     if (p.mode < 0 || p.mode > 3) { set_err(err, "sgbm: mode %d unsupported (0 SGBM, 1 HH, 2 SGBM_3WAY, 3 HH4)", p.mode); return L3D_ERR_UNSUPPORTED; }
@@ -64,7 +71,7 @@ int make_geom(const l3d_sgbm_params& p, int W, int H, Geom& g, std::string* err)
         return L3D_ERR_UNSUPPORTED;
     }
     g.minX1 = std::max(g.maxD, 0); g.maxX1 = W + std::min(g.minD, 0); g.width1 = g.maxX1 - g.minX1;
-    g.DPL = g.D <= 64 ? 2 : (g.D <= 128 ? 4 : 8);
+    g.DPL = g.D <= 64 ? 2 : (g.D <= 128 ? 4 : (g.D <= 256 ? 8 : 16));
     g.NP = g.DPL / 2;
     g.nact = g.D / g.DPL;
     if (g.mode == 2) {
@@ -128,15 +135,30 @@ template <int NP> struct VecOf;
 template <> struct VecOf<1> { typedef uint32_t T; };
 template <> struct VecOf<2> { typedef uint2 T; };
 template <> struct VecOf<4> { typedef uint4 T; };
+struct __align__(32) u32x8 { uint4 lo, hi; };   // D in (256, 512]: 16 disparities per lane
+template <> struct VecOf<8> { typedef u32x8 T; };
 
 template <int NP> __device__ __forceinline__ void vec_unpack(const typename VecOf<NP>::T& v, uint32_t (&o)[NP]);
 template <> __device__ __forceinline__ void vec_unpack<1>(const uint32_t& v, uint32_t (&o)[1]) { o[0] = v; }
 template <> __device__ __forceinline__ void vec_unpack<2>(const uint2& v, uint32_t (&o)[2]) { o[0] = v.x; o[1] = v.y; }
 template <> __device__ __forceinline__ void vec_unpack<4>(const uint4& v, uint32_t (&o)[4]) { o[0] = v.x; o[1] = v.y; o[2] = v.z; o[3] = v.w; }
+template <> __device__ __forceinline__ void vec_unpack<8>(const u32x8& v, uint32_t (&o)[8]) {
+    o[0] = v.lo.x; o[1] = v.lo.y; o[2] = v.lo.z; o[3] = v.lo.w; o[4] = v.hi.x; o[5] = v.hi.y; o[6] = v.hi.z; o[7] = v.hi.w;
+}
 template <int NP> __device__ __forceinline__ typename VecOf<NP>::T vec_pack(const uint32_t (&o)[NP]);
 template <> __device__ __forceinline__ uint32_t vec_pack<1>(const uint32_t (&o)[1]) { return o[0]; }
 template <> __device__ __forceinline__ uint2 vec_pack<2>(const uint32_t (&o)[2]) { return make_uint2(o[0], o[1]); }
 template <> __device__ __forceinline__ uint4 vec_pack<4>(const uint32_t (&o)[4]) { return make_uint4(o[0], o[1], o[2], o[3]); }
+template <> __device__ __forceinline__ u32x8 vec_pack<8>(const uint32_t (&o)[8]) {
+    return u32x8{make_uint4(o[0], o[1], o[2], o[3]), make_uint4(o[4], o[5], o[6], o[7])};
+}
+// read-only global load of one lane's words (the lean WTA kernels).  NP = 8 takes two 16-byte loads: one 32-byte
+// access (ld.global.nc.v8.b32) was measured too and was no faster (MODE_HH pipeline at 1920x1080 / D 384: 57.1 against
+// 58.0 frames/s, with 32-byte S stores in the scans as well)
+template <int NP> __device__ __forceinline__ typename VecOf<NP>::T vec_ldg(const typename VecOf<NP>::T* p) { return __ldg(p); }
+template <> __device__ __forceinline__ u32x8 vec_ldg<8>(const u32x8* p) {
+    return u32x8{__ldg(&p->lo), __ldg(&p->hi)};
+}
 
 constexpr int SCAN_WARPS = 4;
 
@@ -191,12 +213,26 @@ __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commi
 template <int N>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 
+// Winner-takes-all key: (cost << KS) | d, so that one unsigned minimum finds the lowest cost and, among equal costs, the
+// first disparity.  d needs 8 bits up to D = 256 and 9 bits above; the cost (<= 32767) takes 15.
+template <int NP> __host__ __device__ constexpr int wta_kshift() { return NP == 8 ? 9 : 8; }
+template <int NP> __host__ __device__ constexpr unsigned wta_dmask() { return (1u << wta_kshift<NP>()) - 1u; }
+// the keys of both halves of a packed u16x2 word whose low half holds disparity d0
+template <int NP> __device__ __forceinline__ unsigned wta_key_lo(uint32_t w, unsigned d0) {
+    constexpr int KS = wta_kshift<NP>();
+    return ((w << KS) & (0xffffu << KS)) | d0;
+}
+template <int NP> __device__ __forceinline__ unsigned wta_key_hi(uint32_t w, unsigned d0) {
+    constexpr int KS = wta_kshift<NP>();
+    return ((w >> (16 - KS)) & (0xffffu << KS)) | (d0 + 1);
+}
+
 // OpenCV's uniqueness test (modes SGBM / HH): reject when another disparity further than 1 from
 // the winner costs less than minS * 100 / (100 - uniq).  Kept out of line: only the as-constructed
 // parameter set (uniquenessRatio > 0) pays for it.
 template <int NP>
 __device__ __noinline__ bool wta_not_unique(const uint32_t (&w)[NP], unsigned key, int uniq, unsigned dkey, bool active) {
-    const int minS = (int)(key >> 8), best = (int)(key & 255u);
+    const int minS = (int)(key >> wta_kshift<NP>()), best = (int)(key & wta_dmask<NP>());
     bool rej = false;
 #pragma unroll
     for (int q = 0; q < NP; q++) {
@@ -208,40 +244,56 @@ __device__ __noinline__ bool wta_not_unique(const uint32_t (&w)[NP], unsigned ke
     return __any_sync(FULL_MASK, rej) && minS < 32767;
 }
 
-constexpr int SCAN_CH = 16;   // steps per chunk
-constexpr int SCAN_NST = 3;   // chunks in flight per warp (two chunks = 32 steps of look-ahead)
-
-constexpr int HPAIR_NST = 2;  // 1440 warps must be resident at once: a shallower ring keeps the launch to one wave
-__device__ __host__ __forceinline__ size_t scan_smem_bytes_dev(int D) { return (size_t)HPAIR_NST * SCAN_CH * (D * 2) * 2; }
-static size_t scan_smem_bytes(int D, int smode) {
-    return (size_t)SCAN_NST * SCAN_CH * (D * 2) * (smode == 0 ? 1 : 2) + (smode == 2 ? (size_t)32 * D * 2 : 0);
+// cp.async ring of the scan kernels, per words per lane
+template <int NP> struct ScanRing {
+    static constexpr int CH = 16;     // steps per chunk (divides 32: SCAN_FINAL flushes its WTA every 32 steps)
+    static constexpr int NST = 3;     // chunks in flight per warp (two chunks = 32 steps of look-ahead)
+    static constexpr int HP_NST = 2;  // horizontal pair: 1440 warps must be resident at once, a shallower ring keeps the launch to one wave
+};
+// D in (256, 512]: a step moves 512..1024 bytes per array and has twice the arithmetic of D = 256; a ring of two 8-step
+// chunks half the size lets twice the one-warp CTAs share an SM (SCAN_FINAL at D = 384: 49 KB instead of 98 KB), which
+// is worth more than the deeper look-ahead.  1920x1080 / D 384 / block 11 on a B200, kernels alone: SCAN_FINAL 1.737 -> 0.760 ms, accumulating scans
+// 0.64-0.72 -> 0.63-0.70 ms, horizontal pair 0.95 -> 1.00 ms; MODE_HH pipeline 58.0 -> 68.8 frames/s (4 lanes).
+// Also measured: 8 x 3 (66.5 frames/s), 4 x 4 (67.5), 4 x 3 (68.2).
+template <> struct ScanRing<8> {
+    static constexpr int CH = 8;
+    static constexpr int NST = 2;
+    static constexpr int HP_NST = 2;
+};
+template <int NP> __device__ __host__ __forceinline__ size_t scan_smem_bytes_dev(int D) {
+    return (size_t)ScanRing<NP>::HP_NST * ScanRing<NP>::CH * (D * 2) * 2;
+}
+template <int NP> static size_t scan_smem_bytes(int D, int smode) {
+    return (size_t)ScanRing<NP>::NST * ScanRing<NP>::CH * (D * 2) * (smode == 0 ? 1 : 2) + (smode == 2 ? (size_t)32 * D * 2 : 0);
 }
 
 // One warp (= one CTA) per scan line.  The line's C (and, when accumulating, S) vectors are staged
 // through a shared-memory ring with 16-byte cp.async copies (LDGSTS.128: one instruction moves 512
-// contiguous ring bytes = two 128-disparity steps), 32 steps ahead of the consumer, so that the
-// HBM latency is off the recurrence's critical path; the recurrence itself lives in registers.
+// contiguous ring bytes = two 128-disparity steps), NST - 1 chunks of ScanRing<NP>::CH steps ahead of the
+// consumer (32 steps for NP <= 4, 8 for NP = 8), so that the HBM latency is off the recurrence's critical
+// path; the recurrence itself lives in registers.
 template <int NP, int SMODE, bool FULL, int NST>
 __device__ __forceinline__ void scan_run(const ScanArgs& a, const ScanLine& ln, unsigned char* scan_smem,
                                          uint32_t (&L)[NP], uint32_t& minL, const int lane) {
     typedef typename VecOf<NP>::T vec;
+    constexpr int CH = ScanRing<NP>::CH;
     constexpr bool STORE = SMODE == SCAN_STORE;
     constexpr bool FINAL = SMODE == SCAN_FINAL;
     constexpr int DPL = NP * 2;
     const int nact = a.nact, n = ln.n;
     const bool active = FULL || lane < nact;
     const uint32_t B = (uint32_t)a.D * 2u;                      // bytes per pixel vector
-    const uint32_t stage_bytes = SCAN_CH * B * (STORE ? 1 : 2);
+    const uint32_t stage_bytes = CH * B * (STORE ? 1 : 2);
     const uint32_t ring = smem_u32(scan_smem);
     const long pstride = (long)ln.dvr * a.width1 + ln.dx;      // pixel-index step along the line
     const long pix0 = (long)ln.vr * a.width1 + ln.x;
     const char* __restrict__ Cb = (const char*)a.C;
     const char* __restrict__ Sb = (const char*)a.S;
     vec* __restrict__ Sv = (vec*)a.S;
-    const int nchunks = (n + SCAN_CH - 1) / SCAN_CH;
-    // 16-byte pieces: ppv per pixel vector, SCAN_CH * ppv per chunk and array; piece p = it * 32 + lane
+    const int nchunks = (n + CH - 1) / CH;
+    // 16-byte pieces: ppv per pixel vector, CH * ppv per chunk and array; piece p = it * 32 + lane
     const int ppv = a.D >> 3;
-    const int pieces = SCAN_CH * ppv;
+    const int pieces = CH * ppv;
     const int li0 = lane / ppv, lr0 = lane - li0 * ppv, di = 32 / ppv, dr = 32 - di * ppv;
     const long step_bytes = pstride * (long)B;                      // between consecutive steps of the line
     const long it_bytes = (long)di * step_bytes + (long)dr * 16;    // piece p -> p + 32
@@ -249,20 +301,31 @@ __device__ __forceinline__ void scan_run(const ScanArgs& a, const ScanLine& ln, 
     const long lane_off = pix0 * (long)B + (long)li0 * step_bytes + (long)lr0 * 16;
     auto issue = [&](int chunk) {
         if (chunk < nchunks) {
-            const int first = chunk * SCAN_CH;
-            const int cnt = min(SCAN_CH, n - first);
+            const int first = chunk * CH;
+            const int cnt = min(CH, n - first);
             uint32_t dst = ring + (chunk % NST) * stage_bytes + lane * 16;
             long off = lane_off + (long)first * step_bytes;
-            if (FULL) {
+            if constexpr (FULL && 8 * NP > 32) {
+                // D = 512: a pixel vector is 64 pieces, two warp-wide iterations of 32 pieces per step
+                constexpr int SPI = 8 * NP / 32, ITERS = CH * SPI;
+#pragma unroll
+                for (int it = 0; it < ITERS; it++) {
+                    if (cnt == CH || it / SPI < cnt) {
+                        const long o = off + (long)(it / SPI) * step_bytes + (it % SPI) * 512;
+                        cp_async16(dst + it * 512, Cb + o);
+                        if (!STORE) cp_async16(dst + it * 512 + CH * B, Sb + o);
+                    }
+                }
+            } else if (FULL) {
                 // D = 64 * NP: a pixel vector is 8 * NP pieces, which divides 32 -- no piece straddles two
                 // steps' boundaries differently per iteration, every constant folds
-                constexpr int PPV = 8 * NP, DI = 32 / PPV, ITERS = SCAN_CH * PPV / 32;
+                constexpr int PPV = 8 * NP, DI = 32 / PPV, ITERS = CH * PPV / 32;
                 const long it_b = (long)DI * step_bytes;
-                if (cnt == SCAN_CH) {
+                if (cnt == CH) {
 #pragma unroll
                     for (int it = 0; it < ITERS; it++) {
                         cp_async16(dst + it * 512, Cb + off);
-                        if (!STORE) cp_async16(dst + it * 512 + SCAN_CH * B, Sb + off);
+                        if (!STORE) cp_async16(dst + it * 512 + CH * B, Sb + off);
                         off += it_b;
                     }
                 } else {
@@ -270,7 +333,7 @@ __device__ __forceinline__ void scan_run(const ScanArgs& a, const ScanLine& ln, 
                     for (int it = 0; it < ITERS; it++) {
                         if (li0 + it * DI < cnt) {
                             cp_async16(dst + it * 512, Cb + off);
-                            if (!STORE) cp_async16(dst + it * 512 + SCAN_CH * B, Sb + off);
+                            if (!STORE) cp_async16(dst + it * 512 + CH * B, Sb + off);
                         }
                         off += it_b;
                     }
@@ -280,7 +343,7 @@ __device__ __forceinline__ void scan_run(const ScanArgs& a, const ScanLine& ln, 
                 for (int p = lane; p < pieces; p += 32) {
                     if (i < cnt) {
                         cp_async16(dst, Cb + off);
-                        if (!STORE) cp_async16(dst + SCAN_CH * B, Sb + off);
+                        if (!STORE) cp_async16(dst + CH * B, Sb + off);
                     }
                     dst += 512; i += di; r += dr; off += it_bytes;
                     if (r >= ppv) { r -= ppv; i++; off += wrap_bytes; }
@@ -308,7 +371,7 @@ __device__ __forceinline__ void scan_run(const ScanArgs& a, const ScanLine& ln, 
     unsigned char* stash = scan_smem + NST * stage_bytes;  // [32][B]
     auto wta_flush = [&](int first_step, int count) {
         __syncwarp();
-        const int minS = (int)(wkey >> 8), d = (int)(wkey & 255u);
+        const int minS = (int)(wkey >> wta_kshift<NP>()), d = (int)(wkey & wta_dmask<NP>());
         const int j = first_step + lane;
         const int y = ln.vr + ln.dvr * j;
         const int x = ln.x + ln.dx * j;
@@ -356,8 +419,8 @@ __device__ __forceinline__ void scan_run(const ScanArgs& a, const ScanLine& ln, 
             if (active) *(vec*)(stash + (size_t)slot * B + (size_t)lane * sizeof(vec)) = vec_pack<NP>(out);
 #pragma unroll
             for (int q = 0; q < NP; q++) {
-                key = min(key, ((out[q] << 8) & 0xffff00u) | (dkey + 2 * q));
-                key = min(key, ((out[q] >> 8) & 0xffff00u) | (dkey + 2 * q + 1));
+                key = min(key, wta_key_lo<NP>(out[q], dkey + 2 * q));
+                key = min(key, wta_key_hi<NP>(out[q], dkey + 2 * q));
             }
             key = __reduce_min_sync(FULL_MASK, key);
             if (a.uniq > 0) rej = wta_not_unique<NP>(out, key, a.uniq, dkey, active);
@@ -370,17 +433,17 @@ __device__ __forceinline__ void scan_run(const ScanArgs& a, const ScanLine& ln, 
         cp_async_wait<NST - 1>();
         __syncwarp();
         const vec* cs = (const vec*)(scan_smem + s * stage_bytes);
-        const vec* ss = (const vec*)(scan_smem + s * stage_bytes + SCAN_CH * B);
-        const int cnt = min(SCAN_CH, n - c * SCAN_CH);
-        if (cnt == SCAN_CH) {
+        const vec* ss = (const vec*)(scan_smem + s * stage_bytes + CH * B);
+        const int cnt = min(CH, n - c * CH);
+        if (cnt == CH) {
 #pragma unroll
-            for (int i = 0; i < SCAN_CH; i++) step(cs, ss, i);
+            for (int i = 0; i < CH; i++) step(cs, ss, i);
         } else {
             for (int i = 0; i < cnt; i++) step(cs, ss, i);
         }
         __syncwarp();  // every lane is done reading the slot before it is refilled
         issue(c + NST);
-        if (FINAL && (nsteps & 31) == 0) wta_flush(nsteps - 32, 32);  // SCAN_CH divides 32
+        if (FINAL && (nsteps & 31) == 0) wta_flush(nsteps - 32, 32);  // CH divides 32
     }
     if (FINAL && (nsteps & 31)) wta_flush(nsteps & ~31, nsteps & 31);
 }
@@ -395,7 +458,7 @@ __global__ void __launch_bounds__(32) sgbm_scan_kernel(const __grid_constant__ S
 #pragma unroll
     for (int k = 0; k < NP; k++) L[k] = (FULL || lane < a.nact) ? 0u : INF2;
     uint32_t minL = 0;  // packed: warp-wide min of L in both halves
-    scan_run<NP, SMODE, FULL, SCAN_NST>(a, ln, scan_smem, L, minL, lane);
+    scan_run<NP, SMODE, FULL, ScanRing<NP>::NST>(a, ln, scan_smem, L, minL, lane);
 }
 
 // Both horizontal paths of one row in one CTA of two warps: warp 0 runs left-to-right, warp 1
@@ -408,7 +471,7 @@ __global__ void __launch_bounds__(64) sgbm_scan_hpair_kernel(const __grid_consta
     extern __shared__ __align__(128) unsigned char scan_smem[];
     __shared__ uint32_t xch[2][32][NP + 1];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    unsigned char* my_smem = scan_smem + (size_t)warp * scan_smem_bytes_dev(a.D);
+    unsigned char* my_smem = scan_smem + (size_t)warp * scan_smem_bytes_dev<NP>(a.D);
     const int vr = a.hp_row0 + blockIdx.x, width1 = a.width1, mid = width1 / 2;
     ScanLine s1, s2;
     s1.vr = s2.vr = vr; s1.dvr = s2.dvr = 0;
@@ -418,7 +481,7 @@ __global__ void __launch_bounds__(64) sgbm_scan_hpair_kernel(const __grid_consta
 #pragma unroll
     for (int k = 0; k < NP; k++) L[k] = (FULL || lane < a.nact) ? 0u : INF2;
     uint32_t minL = 0;
-    scan_run<NP, SCAN_STORE, FULL, HPAIR_NST>(a, s1, my_smem, L, minL, lane);
+    scan_run<NP, SCAN_STORE, FULL, ScanRing<NP>::HP_NST>(a, s1, my_smem, L, minL, lane);
     // turn round: the two warps exchange their path states at the middle and each walks back over ITS OWN half with
     // the other direction's path -- the vectors it needs first are the ones it touched last (L2 reuse distance grows
     // from zero instead of being half a row for every vector)
@@ -429,7 +492,7 @@ __global__ void __launch_bounds__(64) sgbm_scan_hpair_kernel(const __grid_consta
 #pragma unroll
     for (int k = 0; k < NP; k++) L[k] = xch[warp ^ 1][lane][k];
     minL = xch[warp ^ 1][lane][NP];
-    scan_run<NP, SCAN_ACCUM, FULL, HPAIR_NST>(a, s2, my_smem, L, minL, lane);
+    scan_run<NP, SCAN_ACCUM, FULL, ScanRing<NP>::HP_NST>(a, s2, my_smem, L, minL, lane);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -466,7 +529,7 @@ __global__ void __launch_bounds__(WTA_WARPS * 32) sgbm_wta_lean_kernel(const __g
     bool myok = false;
     for (int k = 0; k < cnt; k++) {
         uint32_t w[NP];
-        if (active) vec_unpack<NP>(__ldg(Sv + (size_t)k * nact), w);
+        if (active) vec_unpack<NP>(vec_ldg<NP>(Sv + (size_t)k * nact), w);
         else {
 #pragma unroll
             for (int q = 0; q < NP; q++) w[q] = INF2;
@@ -474,11 +537,11 @@ __global__ void __launch_bounds__(WTA_WARPS * 32) sgbm_wta_lean_kernel(const __g
         unsigned key = 0xffffffffu;
 #pragma unroll
         for (int q = 0; q < NP; q++) {
-            key = min(key, ((w[q] << 8) & 0xffff00u) | (dkey + 2 * q));
-            key = min(key, ((w[q] >> 8) & 0xffff00u) | (dkey + 2 * q + 1));
+            key = min(key, wta_key_lo<NP>(w[q], dkey + 2 * q));
+            key = min(key, wta_key_hi<NP>(w[q], dkey + 2 * q));
         }
         key = __reduce_min_sync(FULL_MASK, key);
-        const int minS = (int)(key >> 8), best = (int)(key & 255u);
+        const int minS = (int)(key >> wta_kshift<NP>()), best = (int)(key & wta_dmask<NP>());
         bool ok = minS < 32767;  // nothing beats MAX_COST: pixel stays invalid, disp2 untouched
         if (uniq > 0 && ok) {
             bool rej = false;
@@ -496,7 +559,7 @@ __global__ void __launch_bounds__(WTA_WARPS * 32) sgbm_wta_lean_kernel(const __g
     if (lane < cnt && myok) {
         const long pix = base + lane;
         const int y = (int)(pix / a.width1), x = (int)(pix - (long)y * a.width1);
-        const int minS = (int)(mykey >> 8), d = (int)(mykey & 255u);
+        const int minS = (int)(mykey >> wta_kshift<NP>()), d = (int)(mykey & wta_dmask<NP>());
         const int x2 = x + a.minX1 - d - a.minD;
         if (x2 >= 0 && x2 < a.W + 2)
             atomicMax(a.disp2key + (size_t)y * (a.W + 2) + x2, ((unsigned)(0x7fff - minS) << 16) | (unsigned)x);
@@ -542,7 +605,7 @@ __global__ void __launch_bounds__(WTA_WARPS * 32) sgbm_wta_lean3_kernel(const __
     for (int k = 0; k < cnt; k++) {
         if (!((emit_mask >> k) & 1u)) continue;  // warp-uniform
         uint32_t w[NP];
-        if (active) vec_unpack<NP>(__ldg(Sv + (size_t)k * nact), w);
+        if (active) vec_unpack<NP>(vec_ldg<NP>(Sv + (size_t)k * nact), w);
         else {
 #pragma unroll
             for (int q = 0; q < NP; q++) w[q] = INF2;
@@ -557,19 +620,33 @@ __global__ void __launch_bounds__(WTA_WARPS * 32) sgbm_wta_lean3_kernel(const __
         // OpenCV's 8-lane SIMD arg-min: per residue class d mod 8 the LAST disparity that attains the minimum, then the
         // smallest of those.  One ballot per register slot j gives the lanes holding the minimum at d = lane * DPL + j;
         // the classes of a slot are lane patterns (d mod 8 = (lane * DPL + j) mod 8), so "last in class" is the highest
-        // set bit of the ballot under the class's lane mask.
+        // set bit of the ballot under the class's lane mask.  DPL 16: every lane holds two disparities of each class, at
+        // slots c and c + 8; the last of class c is the larger of the two slots' highest candidates.
         int best = 0x7fffffff;
+        if constexpr (DPL > 8) {
 #pragma unroll
-        for (int j = 0; j < DPL; j++) {
-            const unsigned b = __ballot_sync(FULL_MASK, active && sv[j] == minS);
-            constexpr int LPC = 8 / DPL > 0 ? 8 / DPL : 1;   // lanes per period of d mod 8 (DPL 2: 4, DPL 4: 2, DPL 8: 1)
+            for (int c = 0; c < 8; c++) {
+                int last = -1;
 #pragma unroll
-            for (int r = 0; r < LPC; r++) {
-                unsigned pat = 0;                            // lanes with lane % LPC == r
+                for (int j = c; j < DPL; j += 8) {
+                    const unsigned b = __ballot_sync(FULL_MASK, active && sv[j] == minS);
+                    if (b) last = max(last, (31 - __clz(b)) * DPL + j);
+                }
+                if (last >= 0) best = min(best, last);
+            }
+        } else {
 #pragma unroll
-                for (int l = r; l < 32; l += LPC) pat |= 1u << l;
-                const unsigned mm = b & pat;
-                if (mm) best = min(best, (31 - __clz(mm)) * DPL + j);
+            for (int j = 0; j < DPL; j++) {
+                const unsigned b = __ballot_sync(FULL_MASK, active && sv[j] == minS);
+                constexpr int LPC = 8 / DPL;                     // lanes per period of d mod 8 (DPL 2: 4, DPL 4: 2, DPL 8: 1)
+#pragma unroll
+                for (int r = 0; r < LPC; r++) {
+                    unsigned pat = 0;                            // lanes with lane % LPC == r
+#pragma unroll
+                    for (int l = r; l < 32; l += LPC) pat |= 1u << l;
+                    const unsigned mm = b & pat;
+                    if (mm) best = min(best, (31 - __clz(mm)) * DPL + j);
+                }
             }
         }
         bool ok = true;
@@ -584,10 +661,10 @@ __global__ void __launch_bounds__(WTA_WARPS * 32) sgbm_wta_lean3_kernel(const __
             }
             ok = !__any_sync(FULL_MASK, rej);
         }
-        if (lane == k) { mykey = ((unsigned)minS << 8) | (unsigned)best; myok = ok; }
+        if (lane == k) { mykey = ((unsigned)minS << wta_kshift<NP>()) | (unsigned)best; myok = ok; }
     }
     if (emit && myok) {
-        const int minS = (int)(mykey >> 8), d = (int)(mykey & 255u);
+        const int minS = (int)(mykey >> wta_kshift<NP>()), d = (int)(mykey & wta_dmask<NP>());
         const int x2 = x + a.minX1 - d - a.minD;
         if (x2 >= 0 && x2 < a.W && minS < 32767)
             atomicMax(a.disp2key + (size_t)y * (a.W + 2) + x2, ((unsigned)(0x7fff - minS) << 16) | (unsigned)x);
@@ -637,7 +714,7 @@ __global__ void fill_s16_kernel(int16_t* p, size_t n, int16_t v) {
 // ------------------------------------------------------------------------------------------
 template <int NP, int SMODE>
 static int launch_scan_t(Lane& L, const ScanArgs& sa, int lines) {
-    const size_t smem = scan_smem_bytes(sa.D, SMODE);
+    const size_t smem = scan_smem_bytes<NP>(sa.D, SMODE);
     if (sa.nact == 32) {
         L3D_CHECK(L, cudaFuncSetAttribute(sgbm_scan_kernel<NP, SMODE, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         L3D_LAUNCH(L, (sgbm_scan_kernel<NP, SMODE, true>), lines, 32, smem, sa);
@@ -649,7 +726,7 @@ static int launch_scan_t(Lane& L, const ScanArgs& sa, int lines) {
 }
 template <int NP>
 static int launch_hpair(Lane& L, const ScanArgs& sa0) {
-    const size_t smem = 2 * scan_smem_bytes_dev(sa0.D);
+    const size_t smem = 2 * scan_smem_bytes_dev<NP>(sa0.D);
     // Row slices.  Alone, ONE launch over all rows is fastest (the two serial recurrences per row need every row in flight
     // to cover their latency: 0.168 ms against 0.213 ms in three slices at config 3) -- that is what single calls and the
     // kernel-timing leg use.  Inside the frame pipeline three slices let the other streams' kernels (above all the
@@ -679,7 +756,8 @@ static int launch_scan_m(Lane& L, int smode, const ScanArgs& sa, int lines) {
 static int launch_scan_np(Lane& L, int NP, int smode, const ScanArgs& sa, int lines) {
     if (NP == 1) return launch_scan_m<1>(L, smode, sa, lines);
     if (NP == 2) return launch_scan_m<2>(L, smode, sa, lines);
-    return launch_scan_m<4>(L, smode, sa, lines);
+    if (NP == 4) return launch_scan_m<4>(L, smode, sa, lines);
+    return launch_scan_m<8>(L, smode, sa, lines);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -739,7 +817,10 @@ static int sgbm_front_end(Lane& L, SgbmRun& r) {
     ScanArgs sa;
     scan_args_of(r, sa);
     L.t_begin("sgbm_scan_k0");
-    int rc = g.NP == 1 ? launch_hpair<1>(L, sa) : (g.NP == 2 ? launch_hpair<2>(L, sa) : launch_hpair<4>(L, sa));
+    int rc = g.NP == 1 ? launch_hpair<1>(L, sa)
+           : g.NP == 2 ? launch_hpair<2>(L, sa)
+           : g.NP == 4 ? launch_hpair<4>(L, sa)
+                       : launch_hpair<8>(L, sa);
     L.t_end("sgbm_scan_k0");
     return rc;
 }
@@ -857,12 +938,13 @@ int sgbm_back(Lane& L, SgbmRun& r, int16_t* disp, SgbmDebug* dbg) {
         if (full) L3D_LAUNCH(L, (sgbm_wta_lean_kernel<NPV, true>), wgrid, WTA_WARPS * 32, 0, wa);            \
         else L3D_LAUNCH(L, (sgbm_wta_lean_kernel<NPV, false>), wgrid, WTA_WARPS * 32, 0, wa);                \
     } while (0)
-                if (g.NP == 1) L3D_WTA(1); else if (g.NP == 2) L3D_WTA(2); else L3D_WTA(4);
+                if (g.NP == 1) L3D_WTA(1); else if (g.NP == 2) L3D_WTA(2); else if (g.NP == 4) L3D_WTA(4); else L3D_WTA(8);
 #undef L3D_WTA
             } else {
                 if (g.NP == 1) L3D_LAUNCH(L, sgbm_wta_lean3_kernel<1>, wgrid, WTA_WARPS * 32, 0, wa);
                 else if (g.NP == 2) L3D_LAUNCH(L, sgbm_wta_lean3_kernel<2>, wgrid, WTA_WARPS * 32, 0, wa);
-                else L3D_LAUNCH(L, sgbm_wta_lean3_kernel<4>, wgrid, WTA_WARPS * 32, 0, wa);
+                else if (g.NP == 4) L3D_LAUNCH(L, sgbm_wta_lean3_kernel<4>, wgrid, WTA_WARPS * 32, 0, wa);
+                else L3D_LAUNCH(L, sgbm_wta_lean3_kernel<8>, wgrid, WTA_WARPS * 32, 0, wa);
             }
             L.t_end("sgbm_wta");
         }

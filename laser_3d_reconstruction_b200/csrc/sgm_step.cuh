@@ -73,7 +73,8 @@ template <int NP, bool FMAFUNNEL = false, bool FULL = true>
 __device__ __forceinline__ uint32_t sgm_step(uint32_t (&O)[NP], const uint32_t (&I)[NP], uint32_t minI2,
                                              const uint32_t (&Cv)[NP], uint32_t p1x2, uint32_t k2, const SgmLane& s,
                                              bool active = true) {
-    uint32_t Ip[NP];                                     // I + P1, both halves (no carry: I + P1 < 2^16)
+    static_assert(NP == 1 || NP == 2 || NP == 4 || NP == 8, "sgm_step: the warp minimum covers NP = 1, 2, 4 and 8 words");
+    uint32_t Ip[NP];                                    // I + P1, both halves (no carry: I + P1 < 2^16)
 #pragma unroll
     for (int k = 0; k < NP; k++) Ip[k] = sgm_madlo(I[k], s.one, p1x2);
     const uint32_t up = __shfl_up_sync(0xffffffffu, Ip[NP - 1], 1);
@@ -95,6 +96,8 @@ __device__ __forceinline__ uint32_t sgm_step(uint32_t (&O)[NP], const uint32_t (
     uint32_t mn = Ln[0];
     if (NP == 2) mn = __vminu2(Ln[0], Ln[1]);
     if (NP == 4) mn = __vimin3_u16x2(__vminu2(Ln[0], Ln[1]), Ln[2], Ln[3]);
+    if constexpr (NP == 8)
+        mn = __vimin3_u16x2(__vimin3_u16x2(Ln[0], Ln[1], Ln[2]), __vimin3_u16x2(Ln[3], Ln[4], Ln[5]), __vminu2(Ln[6], Ln[7]));
 #pragma unroll
     for (int k = 0; k < NP; k++) O[k] = Ln[k];
     mn = __vminu2(mn, __byte_perm(mn, mn, 0x1032));  // both halves = min of the two
