@@ -203,7 +203,7 @@ enum {
     L3D_RECON_PLANE = 0,        /* Reconstructor.reconstruct_laser_line  core/reconstruction.py:30-143 */
     L3D_RECON_DEPTH = 1,        /* Reconstructor.reconstruct_from_depth  core/reconstruction.py:145-182 */
     L3D_RECON_DISPARITY = 2,    /* ImprovedLaserReconstructor.reconstruct_from_disparity  improved_reconstruction.py:37-86 */
-    L3D_RECON_DISPARITY_MEDIAN = 3 /* .reconstruct_with_interpolation (window 3)  improved_reconstruction.py:88-152 */
+    L3D_RECON_DISPARITY_MEDIAN = 3 /* .reconstruct_with_interpolation (window odd, <= 9)  improved_reconstruction.py:88-152 */
 };
 typedef struct {
     int kind;
@@ -213,7 +213,7 @@ typedef struct {
     double n_water;     /* 1.33 */
     double fx, baseline, cx, cy; /* DISPARITY kinds (from Q) */
     double min_disparity;
-    int window;         /* DISPARITY_MEDIAN: 3 */
+    int window;         /* DISPARITY_MEDIAN: odd, 1..9 (the reference defaults to 3) */
 } l3d_recon_params;
 /* xy: n points (f64 pairs).  img: depth or disparity map (f32, W x H) for the kinds that need it.
  * xyz: up to n rows of 3 f64; *n_out rows written (invalid points dropped, order kept). */
@@ -234,7 +234,10 @@ typedef struct {
     int extractor;            /* -1 none, 0..3 = L3D_STEGER_*, 4 = Simple */
     l3d_steger_params steger;
     int simple_hsv_lo[3], simple_hsv_hi[3], simple_bright_thr; double simple_min_area;
-    l3d_recon_params recon;   /* kind DEPTH normally (main.py:176) */
+    l3d_recon_params recon;   /* per-frame 3D: PLANE reads no image, DEPTH the frame's depth plane (main.py:176),
+                               * DISPARITY / DISPARITY_MEDIAN its int16 x16 disparity (the disp16 of l3d_pipeline_fetch:
+                               * WLS output with depth.use_wls, else the left matcher's) as disp16 / 16.0.  Create fails
+                               * with L3D_ERR_ARG for a DISPARITY_MEDIAN window that is not odd in [1, 9]. */
     int max_points;           /* per-frame point capacity */
     int lanes;                /* frames in flight (streams), >= 1 */
 } l3d_pipeline_config;

@@ -893,9 +893,15 @@ static int pipe_extract(l3d_pipeline* p, Lane& L, FrameOut& o) {
         xy32 = o.xy;
     }
     L.t_end("extract");
-    const float* img = (c.recon.kind == L3D_RECON_PLANE) ? nullptr : o.depth;
+    // PLANE reads no image, DEPTH the depth plane (metres), the DISPARITY kinds the int16 x16 disparity the frame
+    // returns (WLS-filtered when depth.use_wls): written by the same stream, ahead of this launch, in every mode
+    const float* depth = (c.recon.kind == L3D_RECON_PLANE) ? nullptr : o.depth;
+    const int16_t* disp = o.disp;
     L.t_begin("recon");
-    RC(dev_recon(L, c.recon, xy64, xy32, o.n_xy, c.max_points, img, W, H, o.xyz, o.n_xyz));
+    if (c.recon.kind == L3D_RECON_DISPARITY || c.recon.kind == L3D_RECON_DISPARITY_MEDIAN)
+        RC(dev_recon(L, c.recon, xy64, xy32, o.n_xy, c.max_points, disp, W, H, o.xyz, o.n_xyz));
+    else
+        RC(dev_recon(L, c.recon, xy64, xy32, o.n_xy, c.max_points, depth, W, H, o.xyz, o.n_xyz));
     L.t_end("recon");
     return L3D_OK;
 }
@@ -960,6 +966,7 @@ int l3d_pipeline_create(l3d_ctx* ctx, const l3d_pipeline_config* cfg, l3d_pipeli
     NEED(ctx, cfg->W > 1 && cfg->H > 0 && cfg->lanes >= 1 && cfg->lanes <= 64 && cfg->max_points > 0, "pipeline config");
     NEED(ctx, cfg->extractor >= -1 && cfg->extractor <= 4, "pipeline extractor");
     if (cfg->extractor == 4) NEED(ctx, cfg->max_points >= cfg->H, "max_points must be >= H for the Simple extractor");
+    if (cfg->recon.kind == L3D_RECON_DISPARITY_MEDIAN) NEED(ctx, recon_window_ok(cfg->recon.window), "median window must be odd, <= 9");
     CK(ctx, cudaSetDevice(ctx->device));
     l3d_pipeline* p = new l3d_pipeline();
     p->ctx = ctx; p->cfg = *cfg;

@@ -9,6 +9,7 @@
 #include <cstring>
 #include <map>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/l3d.h"
@@ -173,8 +174,12 @@ int dev_steger(Lane& L, const l3d_steger_params& p, const uint8_t* img, int chan
 int dev_colour_mask(Lane& L, const uint8_t* bgr, int W, int H, const int* lo, const int* hi, int thr, uint8_t* mask255);
 int dev_laser_depth_map(Lane& L, const double* xy, int n, const float* disp, int W, int H, double fx, double baseline,
                         float* out);
+// img: f32 depth / disparity map, or (DISPARITY kinds only) the matcher's int16 x16 disparity
+template <typename T>
 int dev_recon(Lane& L, const l3d_recon_params& p, const double* xy, const float* xy_f32,
-              const int* n_dev, int n_max, const float* img, int W, int H, double* xyz, int* n_out_dev);
+              const int* n_dev, int n_max, const T* img, int W, int H, double* xyz, int* n_out_dev);
+// DISPARITY_MEDIAN window: odd, 1..9 (the kernel's 81-entry sort buffer)
+inline bool recon_window_ok(int window) { return window >= 1 && window <= 9 && (window & 1); }
 
 }  // namespace l3d
 

@@ -67,32 +67,40 @@ __device__ bool recon_depth(const ReconArgs& a, double u, double v, const float*
     return true;
 }
 
-__device__ bool recon_disp(const ReconArgs& a, double x, double y, const float* img, int W, int H, double* o) {
+// A disparity element as the reference sees it: the f32 map as is, or the matcher's int16 x16 disparity as
+// `disp.astype(np.float32) / 16.0` (int16 -> f32 is exact and so is the power-of-two scale, |v| <= 32767).
+__device__ __forceinline__ float disp_px(float v) { return v; }
+__device__ __forceinline__ float disp_px(int16_t v) { return (float)v * 0.0625f; }
+
+template <typename T>
+__device__ bool recon_disp(const ReconArgs& a, double x, double y, const T* img, int W, int H, double* o) {
     if (!(fabs(x) < 2147483647.0 && fabs(y) < 2147483647.0)) return false;
     int px = (int)rint(x), py = (int)rint(y);  // python round(): half to even
     float disp;
     const float mind = (float)a.p.min_disparity;
     if (a.p.kind == L3D_RECON_DISPARITY) {
         if (px < 0 || px >= W || py < 0 || py >= H) return false;
-        disp = img[(size_t)py * W + px];
+        disp = disp_px(img[(size_t)py * W + px]);
         if (disp < mind || isnan(disp) || isinf(disp)) return false;
     } else {
         const int hw = a.p.window / 2;
         if (px < hw || px >= W - hw || py < hw || py >= H - hw) return false;
-        float vals[81];
+        // sorted by the raw element: the conversion is monotonic, so only the middle one(s) need converting
+        T vals[81];
         int n = 0;
         for (int dy = -hw; dy <= hw; dy++)
             for (int dx = -hw; dx <= hw; dx++) {
-                float d = img[(size_t)(py + dy) * W + px + dx];
+                T k = img[(size_t)(py + dy) * W + px + dx];
+                float d = disp_px(k);
                 if (d >= mind && !isnan(d) && !isinf(d)) {
                     int j = n++;
-                    while (j > 0 && vals[j - 1] > d) { vals[j] = vals[j - 1]; j--; }
-                    vals[j] = d;
+                    while (j > 0 && vals[j - 1] > k) { vals[j] = vals[j - 1]; j--; }
+                    vals[j] = k;
                 }
             }
         if (n == 0) return false;
         // np.median on float32: odd -> middle, even -> f32 mean of the two middle values
-        disp = (n & 1) ? vals[n / 2] : __fmul_rn(__fadd_rn(vals[n / 2 - 1], vals[n / 2]), 0.5f);
+        disp = (n & 1) ? disp_px(vals[n / 2]) : __fmul_rn(__fadd_rn(disp_px(vals[n / 2 - 1]), disp_px(vals[n / 2])), 0.5f);
     }
     double Z = __ddiv_rn(__dmul_rn(a.p.fx, a.p.baseline), (double)disp);
     double X = __ddiv_rn(__dmul_rn((double)px - a.p.cx, Z), a.p.fx);
@@ -102,8 +110,10 @@ __device__ bool recon_disp(const ReconArgs& a, double x, double y, const float* 
     return true;
 }
 
+// T = float: l3d_reconstruct's host maps (every kind); T = int16_t: the frame pipeline's x16 disparity (DISPARITY kinds)
+template <typename T>
 __global__ void recon_points_kernel(ReconArgs a, const double* __restrict__ xy, const float* __restrict__ xyf,
-                                    const int* __restrict__ n_dev, int n_max, const float* __restrict__ img, int W,
+                                    const int* __restrict__ n_dev, int n_max, const T* __restrict__ img, int W,
                                     int H, double* __restrict__ tmp, int* __restrict__ flag) {
     int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n_max) return;
@@ -112,7 +122,8 @@ __global__ void recon_points_kernel(ReconArgs a, const double* __restrict__ xy, 
     double o[3] = {0, 0, 0};
     if (i < n) {
         double u = xy ? xy[2 * i] : (double)xyf[2 * i], v = xy ? xy[2 * i + 1] : (double)xyf[2 * i + 1];
-        if (a.p.kind == L3D_RECON_PLANE) ok = recon_plane(a, u, v, o);
+        if constexpr (std::is_same<T, int16_t>::value) ok = recon_disp(a, u, v, img, W, H, o);
+        else if (a.p.kind == L3D_RECON_PLANE) ok = recon_plane(a, u, v, o);
         else if (a.p.kind == L3D_RECON_DEPTH) ok = recon_depth(a, u, v, img, W, H, o);
         else ok = recon_disp(a, u, v, img, W, H, o);
     }
@@ -164,23 +175,31 @@ static bool inv3(const double* m, double* o) {
     return true;
 }
 
+template <typename T>
 int dev_recon(Lane& L, const l3d_recon_params& p, const double* xy, const float* xy_f32, const int* n_dev,
-              int n_max, const float* img, int W, int H, double* xyz, int* n_out_dev) {
+              int n_max, const T* img, int W, int H, double* xyz, int* n_out_dev) {
     L3D_ARG(L, p.kind >= 0 && p.kind <= 3, "recon kind");
+    if (std::is_same<T, int16_t>::value) {
+        L3D_ARG(L, p.kind == L3D_RECON_DISPARITY || p.kind == L3D_RECON_DISPARITY_MEDIAN, "an int16 disparity map serves the DISPARITY kinds only");
+    }
     if (n_max <= 0) { L3D_CHECK(L, cudaMemsetAsync(n_out_dev, 0, sizeof(int), L.stream)); return L3D_OK; }
     ReconArgs a;
     a.p = p;
     memset(a.Kinv, 0, sizeof(a.Kinv));
     if (p.kind == L3D_RECON_PLANE) L3D_ARG(L, inv3(p.K, a.Kinv), "camera matrix is singular");
-    if (p.kind == L3D_RECON_DISPARITY_MEDIAN) L3D_ARG(L, p.window >= 1 && p.window <= 9 && (p.window & 1), "median window must be odd, <= 9");
+    if (p.kind == L3D_RECON_DISPARITY_MEDIAN) L3D_ARG(L, recon_window_ok(p.window), "median window must be odd, <= 9");
     if (p.kind != L3D_RECON_PLANE) L3D_ARG(L, img != nullptr, "recon needs a depth/disparity map");
     double* tmp = L.get<double>(S_RC_XYZ, (size_t)n_max * 3);
     int* flag = L.get<int>(S_RC_N, (size_t)n_max * 2);
     int* off = flag + n_max;
-    L3D_LAUNCH(L, recon_points_kernel, cdiv(n_max, 128), 128, 0, a, xy, xy_f32, n_dev, n_max, img, W, H, tmp, flag);
+    L3D_LAUNCH(L, recon_points_kernel<T>, cdiv(n_max, 128), 128, 0, a, xy, xy_f32, n_dev, n_max, img, W, H, tmp, flag);
     L3D_LAUNCH(L, row_scan_kernel, 1, 1024, 0, flag, n_max, off, n_out_dev);
     L3D_LAUNCH(L, recon_emit_kernel, cdiv(n_max, 128), 128, 0, tmp, flag, off, n_max, xyz);
     return L3D_OK;
 }
+template int dev_recon<float>(Lane&, const l3d_recon_params&, const double*, const float*, const int*, int, const float*, int,
+                              int, double*, int*);
+template int dev_recon<int16_t>(Lane&, const l3d_recon_params&, const double*, const float*, const int*, int, const int16_t*,
+                                int, int, double*, int*);
 
 }  // namespace l3d

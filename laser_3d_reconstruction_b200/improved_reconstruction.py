@@ -20,7 +20,9 @@ class ImprovedLaserReconstructor:
             print(f"ImprovedLaserReconstructor 初始化: fx {self.fx:.2f}, 基线 {self.baseline:.4f}m, "
                   f"主点 ({self.cx:.2f}, {self.cy:.2f})")
 
-    def _params(self, kind, min_disparity, window=3):
+    def recon_params(self, kind, min_disparity=1.0, window=3):
+        """The N.ReconParams of a DISPARITY kind with this camera's fx, baseline, cx, cy: what l3d_reconstruct and the
+        frame pipeline (make_pipeline_config(recon=...)) take."""
         p = N.ReconParams()
         p.kind = kind
         p.fx, p.baseline, p.cx, p.cy = float(self.fx), float(self.baseline), float(self.cx), float(self.cy)
@@ -36,7 +38,7 @@ class ImprovedLaserReconstructor:
         if disp.ndim != 2:
             raise ValueError("disparity_map must be HxW")
         xy = N.points_to_array(laser_points)
-        out = N.default_context(self.device).reconstruct(self._params(kind, min_disparity, window), xy,
+        out = N.default_context(self.device).reconstruct(self.recon_params(kind, min_disparity, window), xy,
                                                          disp.astype(np.float32, copy=False))
         return out.astype(np.float32) if len(out) else np.array([])
 

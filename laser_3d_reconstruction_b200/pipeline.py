@@ -36,11 +36,16 @@ def right_matcher_params(p):
                         1000000, p.preFilterCap, 0, 0, 0, p.mode)
 
 
-def depth_config(num_disparities, block_size, mode, Q, use_wls=True, use_maps=True, lam=8000.0, sigma_color=1.5):
+def depth_config(num_disparities, block_size, mode, Q, use_wls=True, use_maps=True, lam=8000.0, sigma_color=1.5,
+                 mutated_left=False):
+    """use_wls=False runs the left matcher alone, with its parameters as constructed; mutated_left=True runs it
+    as createDisparityWLSFilter leaves it instead (the Improved/Hybrid order of test_improved_laser.py:112-207).
+    With use_wls=True the left matcher is always the mutated one."""
     cfg = N.DepthConfig()
     left = sgbm_params(num_disparities, block_size, mode)
     if use_wls:
         cfg.right = right_matcher_params(left)  # created before the mutation, but identical either way
+    if use_wls or mutated_left:
         left = wls_mutate(left)
     cfg.left = left
     cfg.wls = N.WlsParams(lam, sigma_color, left.minDisparity, left.numDisparities, int(math.ceil(0.5 * block_size)), 24)
@@ -54,10 +59,13 @@ def depth_config(num_disparities, block_size, mode, Q, use_wls=True, use_maps=Tr
 
 def make_pipeline_config(W, H, num_disparities, block_size, mode, Q, K, extractor=N.STEGER_IMPROVED, lanes=2,
                          max_points=20000, use_wls=True, use_maps=True, sigma=3.0, bright_thr=200, resp_thr=0.5,
-                         hsv_lo=(50, 100, 180), hsv_hi=(70, 255, 255), min_area=50.0):
+                         hsv_lo=(50, 100, 180), hsv_hi=(70, 255, 255), min_area=50.0, recon=None, mutated_left=False):
+    """recon: the per-frame reconstruction as an N.ReconParams.  None (default) is reconstruct_from_depth with
+    camera matrix K (main.py:176).  The DISPARITY kinds come from ImprovedLaserReconstructor(Q).recon_params and
+    read the frame's int16 disparity (disp16) as disp16 / 16.0."""
     cfg = N.PipelineConfig()
     cfg.W, cfg.H = W, H
-    cfg.depth = depth_config(num_disparities, block_size, mode, Q, use_wls, use_maps)
+    cfg.depth = depth_config(num_disparities, block_size, mode, Q, use_wls, use_maps, mutated_left=mutated_left)
     cfg.extractor = extractor
     cfg.steger = N.StegerParams(min(extractor, 3), sigma, bright_thr, resp_thr, (C.c_int * 4)(0, 0, 0, 0),
                                 (C.c_int * 3)(*hsv_lo), (C.c_int * 3)(*hsv_hi))
@@ -65,10 +73,12 @@ def make_pipeline_config(W, H, num_disparities, block_size, mode, Q, K, extracto
     cfg.simple_hsv_hi[:] = list(hsv_hi)
     cfg.simple_bright_thr = bright_thr
     cfg.simple_min_area = min_area
-    cfg.recon = N.ReconParams()
-    cfg.recon.kind = N.RECON_DEPTH  # main.py:176 calls reconstruct_from_depth
-    cfg.recon.K[:] = [float(v) for v in np.asarray(K, np.float64).reshape(9)]
-    cfg.recon.n_water = 1.33
+    if recon is None:
+        recon = N.ReconParams()
+        recon.kind = N.RECON_DEPTH  # main.py:176 calls reconstruct_from_depth
+        recon.K[:] = [float(v) for v in np.asarray(K, np.float64).reshape(9)]
+        recon.n_water = 1.33
+    cfg.recon = recon
     cfg.max_points = max_points
     cfg.lanes = lanes
     return cfg
@@ -162,7 +172,8 @@ class FramePipeline:
 
     def fetch(self, frame):
         """Everything frame slot `frame` of the last run produced.  points_2d: float64 for the Simple extractor (its
-        exact centroids), float32 for the Steger variants -- the dtypes the reference's extractors return."""
+        exact centroids), float32 for the Steger variants -- the dtypes the reference's extractors return.  points_3d:
+        float32 for the DISPARITY kinds (what ImprovedLaserReconstructor returns), float64 otherwise."""
         W, H, cap = self.cfg.W, self.cfg.H, self.cfg.max_points
         rect = np.empty((H, W, 3), np.uint8)
         depth = np.empty((H, W), np.float32)
@@ -172,6 +183,8 @@ class FramePipeline:
         xy, xyz = self.fetch_points(frame, want_2d=True)
         if self.cfg.extractor != N.EXTRACT_SIMPLE:
             xy = xy.astype(np.float32)
+        if self.cfg.recon.kind in (N.RECON_DISPARITY, N.RECON_DISPARITY_MEDIAN):
+            xyz = xyz.astype(np.float32)
         return dict(left_rect=rect, depth=depth, disp16=disp, points_2d=xy, points_3d=xyz)
 
     def fetch_points(self, frame, want_2d=False):
