@@ -252,6 +252,16 @@ int l3d_pipeline_run_dev(l3d_pipeline* p, const uint8_t* left_dev, const uint8_t
  * (nframes*H*W f32, optional), xyz (nframes*max_points*3 f64) and counts. */
 int l3d_pipeline_run_host(l3d_pipeline* p, const uint8_t* left, const uint8_t* right, int nframes,
                           float* depth, double* xyz, int* counts);
+/* The same two steps on nframes stereo captures as cap.read() delivers them, split as _split_frame does
+ * (camera/single_usb_stereo_camera.py:143-150):
+ *   split = 0: each capture is H x 2W x 3 (left = columns [0, W), right = columns [W, 2W));
+ *   split = 1: each capture is 2H x W x 3 (left = rows [0, H), right = rows [H, 2H)).
+ * The views are read in place as strided rows: the host form uploads each capture with one copy, the device form reads
+ * the caller's buffer (nframes * 6*W*H bytes).  Results, counts and the optional depth / xyz outputs exactly as
+ * l3d_pipeline_run_host / _run_dev; L3D_ERR_ARG for a split other than 0 / 1, a null buffer or nframes <= 0. */
+int l3d_pipeline_run_captures_host(l3d_pipeline* p, const uint8_t* frames, int nframes, int split,
+                                   float* depth, double* xyz, int* counts);
+int l3d_pipeline_run_captures_dev(l3d_pipeline* p, const uint8_t* frames_dev, int nframes, int split, int* counts);
 /* fetch results of the last run for frame slot i (device -> host); any pointer may be NULL.  xy (f32 pairs) and xyz
  * (f64 triples) must hold max_points entries; l3d_pipeline_fetch_points is the form with explicit capacities. */
 int l3d_pipeline_fetch(l3d_pipeline* p, int frame, uint8_t* left_rect, float* depth, int16_t* disp,
@@ -271,8 +281,8 @@ int l3d_pipeline_points_needed(l3d_pipeline* p);
 int l3d_pipeline_pack_points_dev(l3d_pipeline* p, int nframes, const int* frame_ids, double* table_dev,
                                  long long* total_rows);
 long long l3d_pipeline_launch_count(l3d_pipeline* p);
-/* Number of steps the pipeline replayed as a captured CUDA graph so far.  A step (run_dev / run_host) that is
- * repeated with the same buffers and frame count and whose direct enqueue is launch-bound (host enqueue time
+/* Number of steps the pipeline replayed as a captured CUDA graph so far.  A step (run_dev / run_host /
+ * run_captures_*) that is repeated with the same buffers, input form and frame count and whose direct enqueue is launch-bound (host enqueue time
  * > 40 % of its GPU time, e.g. 320x360 frames) is captured on its third occurrence and replayed afterwards;
  * L3D_GRAPH=1 forces, L3D_NO_GRAPH=1 disables the replay. */
 long long l3d_pipeline_graph_replays(l3d_pipeline* p);

@@ -76,7 +76,8 @@ EXPORTS = (
     "l3d_set_rectify_maps l3d_init_undistort_rectify_map l3d_remap_gray l3d_bgr2gray l3d_sgbm_compute l3d_sgbm_compute_pair l3d_sgbm_debug l3d_sgbm_volume_rows "
     "l3d_sgbm_vgroup_time l3d_bm_compute l3d_median3_s16 l3d_filter_speckles l3d_wls_filter l3d_fgs_solve l3d_disp_to_depth l3d_compute_depth "
     "l3d_simple_extract l3d_colour_mask l3d_steger_extract l3d_reconstruct l3d_laser_depth_map l3d_voxel_downsample l3d_statistical_outlier_removal l3d_pipeline_create l3d_pipeline_destroy "
-    "l3d_pipeline_set_maps l3d_pipeline_run_dev l3d_pipeline_run_host l3d_pipeline_fetch l3d_pipeline_fetch_points l3d_pipeline_points_needed "
+    "l3d_pipeline_set_maps l3d_pipeline_run_dev l3d_pipeline_run_host l3d_pipeline_run_captures_dev "
+    "l3d_pipeline_run_captures_host l3d_pipeline_fetch l3d_pipeline_fetch_points l3d_pipeline_points_needed "
     "l3d_pipeline_pack_points_dev l3d_pipeline_launch_count l3d_pipeline_graph_replays l3d_pipeline_last_ms l3d_pipeline_set_timing l3d_pipeline_kernel_time "
     "l3d_host_alloc l3d_host_free l3d_dev_alloc l3d_dev_free l3d_memcpy_h2d l3d_memcpy_d2h"
 ).split()
@@ -439,6 +440,14 @@ def points_to_list_f32(pts):
     (core/laser_extractor.py:256 appends the float32 scalars as they are); zip of the two columns, ~9x faster than
     unpacking row by row."""
     a = np.asarray(pts, np.float32).reshape(-1, 2)
+    return list(zip(a[:, 0], a[:, 1]))
+
+
+def points_to_list_f64(pts):
+    """(n, 2) float64 array -> list of (np.float64, np.float64) tuples, the Simple extractor's points as the batched
+    LaserReconstructionSystem.process_frames returns them: the pairs row-wise unpacking gives, by the column zip of
+    points_to_list_f32."""
+    a = np.asarray(pts, np.float64).reshape(-1, 2)
     return list(zip(a[:, 0], a[:, 1]))
 
 

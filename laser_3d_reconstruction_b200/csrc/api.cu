@@ -799,9 +799,10 @@ struct l3d_pipeline {
     // (all lane / aggregation / back streams fork from and join `main`) and replayed as a CUDA graph -- the
     // 34 launches per frame otherwise make small configurations (320x360) host-launch-bound.
     struct GraphKey {
-        const void *left, *right, *depth_h, *xyz_h; int nframes; bool host_in;
+        const void *left, *right, *depth_h, *xyz_h; int nframes; bool host_in; int split;
         bool operator==(const GraphKey& o) const {
-            return left == o.left && right == o.right && depth_h == o.depth_h && xyz_h == o.xyz_h && nframes == o.nframes && host_in == o.host_in;
+            return left == o.left && right == o.right && depth_h == o.depth_h && xyz_h == o.xyz_h && nframes == o.nframes &&
+                   host_in == o.host_in && split == o.split;
         }
     };
     struct GraphEntry { GraphKey key; int seen = 0; bool launch_bound = false; cudaGraphExec_t exec = nullptr; long long launches = 0; };
@@ -866,11 +867,52 @@ static int pipe_prepare(l3d_pipeline* p, int nframes) {
     return L3D_OK;
 }
 
-// enqueue one frame on lane L (all device pointers)
+// Where a step reads its frames.  Separate eyes (split < 0): two packed arrays of W x H x 3 views.  Captures (split 0 / 1,
+// include/l3d.h): one array of stereo captures; both views of a frame are strided row sets of its capture, read in place
+// by the rectification kernels -- no de-interleaving pass.
+struct PipeSrc {
+    const uint8_t *left, *right;  // frame 0's views
+    size_t step;                  // bytes from a frame's view to the next frame's: W*H*3 for eyes, 2*W*H*3 for captures
+    long stride;                  // row stride of a view
+    int split;                    // -1 separate eyes, 0 side by side, 1 top / bottom
+    bool host;                    // host memory: staged per frame into the lane's scratch
+};
+static PipeSrc pipe_src_eyes(const l3d_pipeline* p, const uint8_t* left, const uint8_t* right, bool host) {
+    const size_t W = p->cfg.W, H = p->cfg.H;
+    return PipeSrc{left, right, W * H * 3, 3L * (long)W, -1, host};
+}
+static PipeSrc pipe_src_captures(const l3d_pipeline* p, const uint8_t* frames, int split, bool host) {
+    const size_t W = p->cfg.W, H = p->cfg.H;
+    return PipeSrc{frames, frames + (split == 0 ? W * 3 : W * H * 3), 2 * W * H * 3, (split == 0 ? 6L : 3L) * (long)W,
+                   split, host};
+}
+// frame f's two views as device pointers; host frames go up on the lane's stream first: separate eyes as two copies,
+// a capture as ONE copy of both views
+static int pipe_views(const PipeSrc& s, Lane& L, int f, const uint8_t*& l, const uint8_t*& r) {
+    l = s.left + s.step * f;
+    r = s.right + s.step * f;
+    if (!s.host) return L3D_OK;
+    if (s.split < 0) {
+        uint8_t* sl = L.get<uint8_t>(S_SRC_L, s.step);
+        uint8_t* sr = L.get<uint8_t>(S_SRC_R, s.step);
+        L3D_CHECK(L, cudaMemcpyAsync(sl, l, s.step, cudaMemcpyHostToDevice, L.stream));
+        L3D_CHECK(L, cudaMemcpyAsync(sr, r, s.step, cudaMemcpyHostToDevice, L.stream));
+        l = sl; r = sr;
+    } else {
+        // a slot of its own: growing S_SRC_L would free the buffer a graph captured for separate eyes reads
+        uint8_t* st = L.get<uint8_t>(S_SRC_CAP, s.step);
+        L3D_CHECK(L, cudaMemcpyAsync(st, l, s.step, cudaMemcpyHostToDevice, L.stream));
+        r = st + (r - l);
+        l = st;
+    }
+    return L3D_OK;
+}
+
+// enqueue one frame on lane L (device pointers, rows `stride` bytes apart)
 static int pipe_extract(l3d_pipeline* p, Lane& L, FrameOut& o);
-static int pipe_frame(l3d_pipeline* p, Lane& L, const uint8_t* l, const uint8_t* r, FrameOut& o) {
+static int pipe_frame(l3d_pipeline* p, Lane& L, const uint8_t* l, const uint8_t* r, long stride, FrameOut& o) {
     const l3d_pipeline_config& c = p->cfg;
-    RC(depth_path(L, c.depth, p->maps, l, r, c.W, c.H, 3L * c.W, o.rect, o.depth, o.disp));
+    RC(depth_path(L, c.depth, p->maps, l, r, c.W, c.H, stride, o.rect, o.depth, o.disp));
     return pipe_extract(p, L, o);
 }
 // laser centre line on the rectified left image + 3D points (main.py:172-178)
@@ -1054,12 +1096,11 @@ static bool pipe_grouped(const l3d_pipeline* p) {
     return width1 > 0 && vgroup_supported(width1, c.H, q.numDisparities);
 }
 
-static int pipe_run_grouped(l3d_pipeline* p, const uint8_t* left, const uint8_t* right, bool host_in, int nframes,
-                            float* depth_h, double* xyz_h) {
+static int pipe_run_grouped(l3d_pipeline* p, const PipeSrc& src, int nframes, float* depth_h, double* xyz_h) {
     l3d_ctx* ctx = p->ctx;
     const l3d_pipeline_config& c = p->cfg;
     const int W = c.W, H = c.H, cap = c.max_points;
-    const size_t nb = (size_t)W * H * 3, n = (size_t)W * H;
+    const size_t n = (size_t)W * H;
     const int nl = (int)p->lanes.size();
     const int gsz = pipe_group_size(p);
     const int nsets = p->timing ? 1 : std::max(1, std::min(l3d_pipeline::MAXSETS, nl / gsz));  // lane sets alternate
@@ -1080,20 +1121,14 @@ static int pipe_run_grouped(l3d_pipeline* p, const uint8_t* left, const uint8_t*
         for (int i = 0; i < ng; i++) {
             const int li = set * gsz + i, f = f0 + i;
             Lane& L = p->lanes[li];
-            const uint8_t *l = left + nb * f, *r = right + nb * f;
             if (p->timing && i > 0) CK(ctx, cudaStreamWaitEvent(L.stream, p->lane_front[li - 1], 0));  // kernels alone
-            if (host_in) {
-                uint8_t* sl = L.get<uint8_t>(S_SRC_L, nb);
-                uint8_t* sr = L.get<uint8_t>(S_SRC_R, nb);
-                L3D_CHECK(L, cudaMemcpyAsync(sl, l, nb, cudaMemcpyHostToDevice, L.stream));
-                L3D_CHECK(L, cudaMemcpyAsync(sr, r, nb, cudaMemcpyHostToDevice, L.stream));
-                l = sl; r = sr;
-            }
+            const uint8_t *l, *r;
+            RC(pipe_views(src, L, f, l, r));
             DepthRuns& dr = p->runs[li];
             dr.vwave = use_vwave;
             static const bool dbg_marks_on = getenv("L3D_DEBUG_PHASES") != nullptr;
             if (dbg_marks_on) p->mark("front0", f, L.stream);
-            RC(depth_front(L, c.depth, p->maps, l, r, W, H, 3L * W, p->outs[f].rect, dr));
+            RC(depth_front(L, c.depth, p->maps, l, r, W, H, src.stride, p->outs[f].rect, dr));
             if (dbg_marks_on) p->mark("front1", f, L.stream);
             CK(ctx, cudaEventRecord(p->lane_front[li], L.stream));
             CK(ctx, cudaStreamWaitEvent(M.stream, p->lane_front[li], 0));
@@ -1140,28 +1175,21 @@ static int pipe_run_grouped(l3d_pipeline* p, const uint8_t* left, const uint8_t*
 }
 
 // fork from `main`, enqueue one step on the lanes, join `main` again (capturable: no allocation in the steady state)
-static int pipe_enqueue(l3d_pipeline* p, const uint8_t* left, const uint8_t* right, bool host_in, int nframes,
-                        float* depth_h, double* xyz_h) {
+static int pipe_enqueue(l3d_pipeline* p, const PipeSrc& src, int nframes, float* depth_h, double* xyz_h) {
     l3d_ctx* ctx = p->ctx;
     const int W = p->cfg.W, H = p->cfg.H, cap = p->cfg.max_points;
-    const size_t nb = (size_t)W * H * 3, n = (size_t)W * H;
+    const size_t n = (size_t)W * H;
     const int nl = (int)p->lanes.size();
     CK(ctx, cudaEventRecord(p->ev_fork, p->main));
     for (auto& L : p->lanes) CK(ctx, cudaStreamWaitEvent(L.stream, p->ev_fork, 0));
     const bool grouped = pipe_grouped(p);
-    if (grouped) RC(pipe_run_grouped(p, left, right, host_in, nframes, depth_h, xyz_h));
+    if (grouped) RC(pipe_run_grouped(p, src, nframes, depth_h, xyz_h));
     for (int f = 0; f < nframes && !grouped; f++) {
         Lane& L = p->lanes[f % nl];
         FrameOut& o = p->outs[f];
-        const uint8_t *l = left + nb * f, *r = right + nb * f;
-        if (host_in) {
-            uint8_t* sl = L.get<uint8_t>(S_SRC_L, nb);
-            uint8_t* sr = L.get<uint8_t>(S_SRC_R, nb);
-            L3D_CHECK(L, cudaMemcpyAsync(sl, l, nb, cudaMemcpyHostToDevice, L.stream));
-            L3D_CHECK(L, cudaMemcpyAsync(sr, r, nb, cudaMemcpyHostToDevice, L.stream));
-            l = sl; r = sr;
-        }
-        RC(pipe_frame(p, L, l, r, o));
+        const uint8_t *l, *r;
+        RC(pipe_views(src, L, f, l, r));
+        RC(pipe_frame(p, L, l, r, src.stride, o));
         L3D_CHECK(L, cudaMemcpyAsync(p->counts_host + 2 * f, o.n_xy, sizeof(int), cudaMemcpyDeviceToHost, L.stream));
         L3D_CHECK(L, cudaMemcpyAsync(p->counts_host + 2 * f + 1, o.n_xyz, sizeof(int), cudaMemcpyDeviceToHost, L.stream));
         if (depth_h) L3D_CHECK(L, cudaMemcpyAsync(depth_h + n * f, o.depth, n * 4, cudaMemcpyDeviceToHost, L.stream));
@@ -1181,21 +1209,20 @@ static long long pipe_launches_now(const l3d_pipeline* p) {
     return s;
 }
 
-static int pipe_run(l3d_pipeline* p, const uint8_t* left, const uint8_t* right, bool host_in, int nframes,
-                    float* depth_h, double* xyz_h, int* counts) {
+static int pipe_run(l3d_pipeline* p, const PipeSrc& src, int nframes, float* depth_h, double* xyz_h, int* counts) {
     l3d_ctx* ctx = p->ctx;
     CK(ctx, cudaSetDevice(ctx->device));
     RC(pipe_prepare(p, nframes));
     for (auto& L : p->lanes) L.t_reset();
     auto t_enq0 = std::chrono::steady_clock::now();
-    // ---- CUDA-graph replay of a repeated step (same buffers, same frame count); the first occurrence runs with
-    // direct launches (it also grows the scratch buffers), the second decides whether the step is launch-bound,
-    // the third is captured, later ones are replayed
+    // ---- CUDA-graph replay of a repeated step (same buffers and input form, same frame count); the first occurrence
+    // runs with direct launches (it also grows the scratch buffers), the second decides whether the step is
+    // launch-bound, the third is captured, later ones are replayed
     static const bool graphs_off = (getenv("L3D_NO_GRAPH") && atoi(getenv("L3D_NO_GRAPH")) > 0) || getenv("L3D_DEBUG_PHASES") ||
                                    getenv("L3D_DEBUG_SKIP");
     l3d_pipeline::GraphEntry* ge = nullptr;
     if (!graphs_off && p->graphs_ok && !p->timing) {
-        const l3d_pipeline::GraphKey key{left, right, depth_h, xyz_h, nframes, host_in};
+        const l3d_pipeline::GraphKey key{src.left, src.right, depth_h, xyz_h, nframes, src.host, src.split};
         for (auto& g : p->graphs) if (g.key == key) ge = &g;
         if (!ge) {
             if (p->graphs.size() >= 8) {  // bounded cache: drop the oldest entry
@@ -1217,7 +1244,7 @@ static int pipe_run(l3d_pipeline* p, const uint8_t* left, const uint8_t* right, 
             cudaError_t e = cudaStreamBeginCapture(p->main, cudaStreamCaptureModeRelaxed);
             int rc = L3D_OK;
             if (e == cudaSuccess) {
-                rc = pipe_enqueue(p, left, right, host_in, nframes, depth_h, xyz_h);
+                rc = pipe_enqueue(p, src, nframes, depth_h, xyz_h);
                 e = cudaStreamEndCapture(p->main, &graph);
             }
             if (e == cudaSuccess && rc == L3D_OK && graph) e = cudaGraphInstantiate(&ge->exec, graph, 0);
@@ -1243,7 +1270,7 @@ static int pipe_run(l3d_pipeline* p, const uint8_t* left, const uint8_t* right, 
     }
     if (!replayed) {
         CK(ctx, cudaEventRecord(p->ev0, p->main));
-        RC(pipe_enqueue(p, left, right, host_in, nframes, depth_h, xyz_h));
+        RC(pipe_enqueue(p, src, nframes, depth_h, xyz_h));
     }
     CK(ctx, cudaEventRecord(p->ev1, p->main));
     const double enq_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_enq0).count();
@@ -1279,7 +1306,7 @@ int l3d_pipeline_run_dev(l3d_pipeline* p, const uint8_t* left_dev, const uint8_t
     l3d_ctx* ctx = p->ctx;
     API_BEGIN(ctx)
     NEED(ctx, left_dev && right_dev && nframes > 0, "pipeline_run_dev arguments");
-    return pipe_run(p, left_dev, right_dev, false, nframes, nullptr, nullptr, counts);
+    return pipe_run(p, pipe_src_eyes(p, left_dev, right_dev, false), nframes, nullptr, nullptr, counts);
     API_END(ctx)
 }
 
@@ -1289,7 +1316,26 @@ int l3d_pipeline_run_host(l3d_pipeline* p, const uint8_t* left, const uint8_t* r
     l3d_ctx* ctx = p->ctx;
     API_BEGIN(ctx)
     NEED(ctx, left && right && nframes > 0, "pipeline_run_host arguments");
-    return pipe_run(p, left, right, true, nframes, depth, xyz, counts);
+    return pipe_run(p, pipe_src_eyes(p, left, right, true), nframes, depth, xyz, counts);
+    API_END(ctx)
+}
+
+int l3d_pipeline_run_captures_dev(l3d_pipeline* p, const uint8_t* frames_dev, int nframes, int split, int* counts) {
+    if (!p) return L3D_ERR_ARG;
+    l3d_ctx* ctx = p->ctx;
+    API_BEGIN(ctx)
+    NEED(ctx, frames_dev && nframes > 0 && (split == 0 || split == 1), "pipeline_run_captures_dev arguments");
+    return pipe_run(p, pipe_src_captures(p, frames_dev, split, false), nframes, nullptr, nullptr, counts);
+    API_END(ctx)
+}
+
+int l3d_pipeline_run_captures_host(l3d_pipeline* p, const uint8_t* frames, int nframes, int split, float* depth,
+                                   double* xyz, int* counts) {
+    if (!p) return L3D_ERR_ARG;
+    l3d_ctx* ctx = p->ctx;
+    API_BEGIN(ctx)
+    NEED(ctx, frames && nframes > 0 && (split == 0 || split == 1), "pipeline_run_captures_host arguments");
+    return pipe_run(p, pipe_src_captures(p, frames, split, true), nframes, depth, xyz, counts);
     API_END(ctx)
 }
 

@@ -32,6 +32,7 @@ enum Slot {
     S_ST_GRAY, S_ST_TMP, S_ST_SM, S_ST_ROW, S_ST_CNT, S_ST_XY, S_ST_N,
     S_SM_MASK0, S_SM_MASK1, S_SM_LABEL, S_SM_LABEL2, S_SM_AREA, S_SM_ROW, S_SM_XY,
     S_RC_XY, S_RC_XYZ, S_RC_N, S_IO_A, S_IO_B, S_IO_C, S_IO_D, S_IO_E,
+    S_SRC_CAP,  // frame pipeline: one staged stereo capture (both views)
     S_NUM
 };
 

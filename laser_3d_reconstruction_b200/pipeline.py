@@ -131,18 +131,54 @@ class FramePipeline:
         for name, a in (("left", left), ("right", right)):
             if a.dtype != np.uint8 or a.shape != want or not a.flags.c_contiguous:
                 raise N.L3DError("run_host: %s must be a C-contiguous uint8 array of shape %s" % (name, want))
-        if depth_out is not None and (depth_out.dtype != np.float32 or not depth_out.flags.c_contiguous
-                                      or depth_out.size < n * self.cfg.H * self.cfg.W):
-            raise N.L3DError("run_host: depth_out must be C-contiguous float32 with room for %d frames" % n)
-        if xyz_out is not None and (xyz_out.dtype != np.float64 or not xyz_out.flags.c_contiguous
-                                    or xyz_out.size < n * self.cfg.max_points * 3):
-            raise N.L3DError("run_host: xyz_out must be C-contiguous float64 with room for %d x max_points x 3" % n)
+        self._check_outputs("run_host", n, depth_out, xyz_out)
         counts = (C.c_int * n)()
         self.ctx.check(self.lib.l3d_pipeline_run_host(self.h, C.c_void_p(left.ctypes.data), C.c_void_p(right.ctypes.data), n,
                                                       C.c_void_p(depth_out.ctypes.data) if depth_out is not None else None,
                                                       C.c_void_p(xyz_out.ctypes.data) if xyz_out is not None else None,
                                                       counts), "l3d_pipeline_run_host")
         return np.frombuffer(counts, np.int32).copy()
+
+    def capture_shape(self, n, split):
+        """Shape of n stereo captures as cap.read() delivers them: (n, H, 2W, 3) side by side (split 0, the camera's
+        'horizontal' split_mode) or (n, 2H, W, 3) one above the other (split 1)."""
+        if split not in (0, 1):
+            raise N.L3DError("split must be 0 (side by side) or 1 (top / bottom), not %r" % (split,))
+        W, H = self.cfg.W, self.cfg.H
+        return (n, H, 2 * W, 3) if split == 0 else (n, 2 * H, W, 3)
+
+    def run_captures_host(self, frames, split, depth_out=None, xyz_out=None):
+        """run_host on stereo captures: frames = (n, H, 2W, 3) (split 0) or (n, 2H, W, 3) (split 1) C-contiguous uint8
+        host array (pinned for full overlap), each capture uploaded with one copy and split on the device;
+        depth_out / xyz_out as for run_host."""
+        frames = np.asarray(frames)
+        n = frames.shape[0] if frames.ndim == 4 else 0
+        want = self.capture_shape(n, split)
+        if frames.dtype != np.uint8 or frames.shape != want or n == 0 or not frames.flags.c_contiguous:
+            raise N.L3DError("run_captures_host: frames must be a C-contiguous uint8 array of shape %s" % (want,))
+        self._check_outputs("run_captures_host", n, depth_out, xyz_out)
+        counts = (C.c_int * n)()
+        self.ctx.check(self.lib.l3d_pipeline_run_captures_host(
+            self.h, C.c_void_p(frames.ctypes.data), n, int(split),
+            C.c_void_p(depth_out.ctypes.data) if depth_out is not None else None,
+            C.c_void_p(xyz_out.ctypes.data) if xyz_out is not None else None, counts), "l3d_pipeline_run_captures_host")
+        return np.frombuffer(counts, np.int32).copy()
+
+    def run_captures_dev(self, frames_dev, nframes, split):
+        """run_dev on nframes stereo captures already in HBM (device pointer to capture_shape(nframes, split) uint8)."""
+        self.capture_shape(nframes, split)
+        counts = (C.c_int * max(int(nframes), 1))()
+        self.ctx.check(self.lib.l3d_pipeline_run_captures_dev(self.h, C.c_void_p(frames_dev), int(nframes), int(split), counts),
+                       "l3d_pipeline_run_captures_dev")
+        return np.frombuffer(counts, np.int32)[:nframes].copy()
+
+    def _check_outputs(self, what, n, depth_out, xyz_out):
+        if depth_out is not None and (depth_out.dtype != np.float32 or not depth_out.flags.c_contiguous
+                                      or depth_out.size < n * self.cfg.H * self.cfg.W):
+            raise N.L3DError("%s: depth_out must be C-contiguous float32 with room for %d frames" % (what, n))
+        if xyz_out is not None and (xyz_out.dtype != np.float64 or not xyz_out.flags.c_contiguous
+                                    or xyz_out.size < n * self.cfg.max_points * 3):
+            raise N.L3DError("%s: xyz_out must be C-contiguous float64 with room for %d x max_points x 3" % (what, n))
 
     @property
     def last_ms(self):
@@ -174,18 +210,24 @@ class FramePipeline:
         """Everything frame slot `frame` of the last run produced.  points_2d: float64 for the Simple extractor (its
         exact centroids), float32 for the Steger variants -- the dtypes the reference's extractors return.  points_3d:
         float32 for the DISPARITY kinds (what ImprovedLaserReconstructor returns), float64 otherwise."""
-        W, H, cap = self.cfg.W, self.cfg.H, self.cfg.max_points
-        rect = np.empty((H, W, 3), np.uint8)
-        depth = np.empty((H, W), np.float32)
-        disp = np.empty((H, W), np.int16)
-        self.ctx.check(self.lib.l3d_pipeline_fetch(self.h, int(frame), N._ptr(rect), N._ptr(depth), N._ptr(disp), None,
-                                                   None, None, None), "l3d_pipeline_fetch")
+        rect, depth, disp = self.fetch_images(frame, want_disp=True)
         xy, xyz = self.fetch_points(frame, want_2d=True)
         if self.cfg.extractor != N.EXTRACT_SIMPLE:
             xy = xy.astype(np.float32)
         if self.cfg.recon.kind in (N.RECON_DISPARITY, N.RECON_DISPARITY_MEDIAN):
             xyz = xyz.astype(np.float32)
         return dict(left_rect=rect, depth=depth, disp16=disp, points_2d=xy, points_3d=xyz)
+
+    def fetch_images(self, frame, want_disp=False):
+        """(left_rect (H,W,3) uint8, depth (H,W) float32) of frame slot `frame` of the last run, in new arrays, and its
+        int16 x16 disparity (disp16) as a third element with want_disp."""
+        W, H = self.cfg.W, self.cfg.H
+        rect = np.empty((H, W, 3), np.uint8)
+        depth = np.empty((H, W), np.float32)
+        disp = np.empty((H, W), np.int16) if want_disp else None
+        self.ctx.check(self.lib.l3d_pipeline_fetch(self.h, int(frame), N._ptr(rect), N._ptr(depth), N._ptr(disp), None,
+                                                   None, None, None), "l3d_pipeline_fetch")
+        return (rect, depth, disp) if want_disp else (rect, depth)
 
     def fetch_points(self, frame, want_2d=False):
         """The 3D points (and optionally the 2D centres) of frame slot `frame` of the last run (device -> host);

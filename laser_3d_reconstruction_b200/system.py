@@ -8,6 +8,8 @@ host round trip between the stages) and produce exactly what calling `process_fr
 produces.  `save_point_cloud` (main.py:190-232) runs the point-cloud sink (voxel down-sampling, outlier removal,
 PLY) through `utils.PointCloudProcessor`, the GPU form of the reference's Open3D-free code (SURVEY 8f N2).
 """
+import itertools
+
 import numpy as np
 
 from . import _native as N
@@ -17,6 +19,25 @@ from .config import Config
 from .core.laser_extractor import FastStegerExtractor, SimpleLaserExtractor
 from .core.reconstruction import Reconstructor
 from .utils.point_cloud import PointCloudProcessor
+
+# Frames per pipeline call of process_frames: about 1 GB of device results at 1280x720.  Measured on one B200 (1 000 W),
+# run_captures_host at 1280x720 in pieces of 28 / 56 / 112 / 224 frames gave 797 / 756 / 758 / 757 frames/s over 448
+# frames and 741 / 656 / 807 / 796 over 112 -- no size is faster beyond the noise, and 112 is bench.py's config-3 step.
+CHUNK_FRAMES = 112
+
+
+def _chunks(frames, k):
+    """Consecutive pieces of at most k frames: slices of an array, stacked lists of the items of any other iterable."""
+    if isinstance(frames, np.ndarray):
+        for c0 in range(0, frames.shape[0], k):
+            yield frames[c0:c0 + k]
+        return
+    it = iter(frames)
+    while True:
+        part = list(itertools.islice(it, k))
+        if not part:
+            return
+        yield np.stack(part)
 
 
 class LaserReconstructionSystem:
@@ -144,40 +165,54 @@ class LaserReconstructionSystem:
         return self._pipe
 
     def process_frames(self, frames=None, lefts=None, rights=None, lanes=8, want_images=True):
-        """Batched `process_frame`: `frames` = side-by-side captures (n, H, 2W, 3) as `cap.read()` delivers them, or
-        `lefts` / `rights` = already split views (n, H, W, 3).  Returns a list of (color_image, depth_image,
-        laser_points) per frame (images omitted when `want_images` is False) and accumulates the valid 3D points in
-        `self.point_cloud` in frame order, exactly as n calls of `process_frame` would."""
+        """Batched `process_frame`: `frames` = stereo captures as `cap.read()` delivers them -- an (n, H, 2W, 3) uint8
+        array, or (n, 2H, W, 3) when the camera's split_mode is not 'horizontal' (see `_split_frame`), or a list or other
+        iterable of single captures -- or `lefts` / `rights` = already split views (n, H, W, 3).  Returns a list of
+        (color_image, depth_image, laser_points) per frame (images omitted when `want_images` is False) and accumulates
+        the valid 3D points in `self.point_cloud` in frame order, exactly as n calls of `process_frame` would.
+
+        A C-contiguous uint8 capture array goes to the pipeline as it is: each capture is uploaded with one copy and
+        split on the device.  Frames run in chunks of CHUNK_FRAMES, so device memory (about 9 MB per frame at
+        1280x720) and the host copy a list is stacked into stay bounded whatever the recording's length."""
+        out = []
         if frames is not None:
-            pairs = [self.camera._split_frame(f) for f in frames]
-            lefts = np.stack([np.ascontiguousarray(p[0]) for p in pairs])
-            rights = np.stack([np.ascontiguousarray(p[1]) for p in pairs])
+            split = 0 if self.camera.split_mode == 'horizontal' else 1
+            for chunk in _chunks(frames, CHUNK_FRAMES):
+                chunk = np.ascontiguousarray(chunk, np.uint8)  # no copy for a slice of a C-contiguous uint8 array
+                self._process_chunk(lanes, want_images, out, lambda fp: fp.run_captures_host(chunk, split))
+            return out
         lefts = np.ascontiguousarray(lefts, np.uint8)
         rights = np.ascontiguousarray(rights, np.uint8)
-        n = lefts.shape[0]
+        for c0 in range(0, lefts.shape[0], CHUNK_FRAMES):
+            l, r = lefts[c0:c0 + CHUNK_FRAMES], rights[c0:c0 + CHUNK_FRAMES]
+            self._process_chunk(lanes, want_images, out, lambda fp: fp.run_host(l, r))
+        return out
+
+    def _process_chunk(self, lanes, want_images, out, run):
+        """One pipeline call (`run(fp)`) over a chunk of frames; its frames' results are appended to `out` and their
+        points to `self.point_cloud` only once the chunk has run with room for all of its points."""
         fp = self._pipeline(lanes, self._pipe_cap)
-        fp.run_host(lefts, rights)
+        n = len(run(fp))
         if fp.points_needed > fp.cfg.max_points:
             # a frame found more laser points than the pipeline's point lists hold (FastSteger emits one per bright
             # pixel: a saturated patch can exceed any fixed bound): nothing may be dropped silently -- the single-frame
-            # calls grow their buffers too -- so the pipeline is rebuilt with room for them and the batch runs again
-            self._pipe_cap = min(lefts.shape[1] * lefts.shape[2], 2 * fp.points_needed)
+            # calls grow their buffers too -- so the pipeline is rebuilt with room for them and the chunk runs again
+            self._pipe_cap = min(fp.cfg.W * fp.cfg.H, 2 * fp.points_needed)
             fp = self._pipeline(lanes, self._pipe_cap)
-            fp.run_host(lefts, rights)
+            run(fp)
             if fp.points_needed > fp.cfg.max_points:
                 raise N.L3DError("process_frames: %d laser points in one frame exceed the point list capacity %d"
                                  % (fp.points_needed, fp.cfg.max_points))
-        out = []
+        # np.float64 pairs (Simple) / np.float32 pairs (Steger), as the reference's extractors give them
+        to_list = N.points_to_list_f64 if fp.cfg.extractor == N.EXTRACT_SIMPLE else N.points_to_list_f32
         for i in range(n):
-            got = fp.fetch(i)
-            pts2 = [(x, y) for x, y in got["points_2d"]]  # np.float64 pairs (Simple) / np.float32 pairs (Steger), as the reference
-            p3 = got["points_3d"]
+            xy, p3 = fp.fetch_points(i, want_2d=True)
+            pts2 = to_list(xy)
             if len(p3) > 0:
                 p3 = p3[~np.isnan(p3).any(axis=1)]
                 self.point_cloud.extend(p3.tolist())
             self.frame_count += 1
-            out.append((got["left_rect"], got["depth"], pts2) if want_images else (None, None, pts2))
-        return out
+            out.append(fp.fetch_images(i) + (pts2,) if want_images else (None, None, pts2))
 
     # ---- reference :190-232 ---------------------------------------------------------------------
     def save_point_cloud(self, filename=None):
