@@ -107,10 +107,6 @@ int l3d_sgbm_compute_pair(l3d_ctx* ctx, const l3d_sgbm_params* left_params, cons
                           int16_t* disp_right, int16_t* Cl_out, int16_t* Cr_out);
 /* rows of the C/S volumes l3d_sgbm_debug writes (H, or the sum of 3WAY stripe heights) */
 int l3d_sgbm_volume_rows(const l3d_sgbm_params* p, int W, int H);
-/* Measurement hook for the cluster-fused aggregation kernel (sgbm_vgroup.cu): runs pass `dir` over njobs
- * synthetic width1 x H x D volumes `reps` times and returns the mean CUDA-event time of one launch. */
-int l3d_sgbm_vgroup_time(l3d_ctx* ctx, int width1, int H, int D, int P1, int P2, int njobs, int dir, int reps,
-                         float* ms_per_launch);
 /* cv2.medianBlur(disp, 3) and cv2.filterSpeckles as applied inside StereoSGBM.compute
  * (camera/single_usb_stereo_camera.py:324-325 with speckleWindowSize / speckleRange of :266-267) */
 int l3d_median3_s16(l3d_ctx* ctx, const int16_t* src, int W, int H, int16_t* dst);

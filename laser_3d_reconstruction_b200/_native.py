@@ -74,7 +74,7 @@ RECON_PLANE, RECON_DEPTH, RECON_DISPARITY, RECON_DISPARITY_MEDIAN = 0, 1, 2, 3
 EXPORTS = (
     "l3d_ctx_create l3d_ctx_destroy l3d_last_error l3d_sync l3d_device_count l3d_version l3d_launch_count "
     "l3d_set_rectify_maps l3d_init_undistort_rectify_map l3d_remap_gray l3d_bgr2gray l3d_sgbm_compute l3d_sgbm_compute_pair l3d_sgbm_debug l3d_sgbm_volume_rows "
-    "l3d_sgbm_vgroup_time l3d_bm_compute l3d_median3_s16 l3d_filter_speckles l3d_wls_filter l3d_fgs_solve l3d_disp_to_depth l3d_compute_depth "
+    "l3d_bm_compute l3d_median3_s16 l3d_filter_speckles l3d_wls_filter l3d_fgs_solve l3d_disp_to_depth l3d_compute_depth "
     "l3d_simple_extract l3d_colour_mask l3d_steger_extract l3d_reconstruct l3d_laser_depth_map l3d_voxel_downsample l3d_statistical_outlier_removal l3d_pipeline_create l3d_pipeline_destroy "
     "l3d_pipeline_set_maps l3d_pipeline_run_dev l3d_pipeline_run_host l3d_pipeline_run_captures_dev "
     "l3d_pipeline_run_captures_host l3d_pipeline_fetch l3d_pipeline_fetch_points l3d_pipeline_points_needed "

@@ -1,4 +1,5 @@
-// hostcopy.cuh -- staged host<->device copies for the single-frame calls of the C ABI (host code, api.cu only).
+// hostcopy.cuh -- staged host<->device copies for the single-frame calls of the C ABI (host code, api.cu; pipeline.cu
+// includes it through api.cuh only for API_BEGIN's per-call reset of the stager).
 //
 // The reference-facing calls take ordinary (pageable) numpy arrays.  cudaMemcpyAsync on pageable memory goes through the
 // driver's own staging buffers on ONE host thread and blocks the caller; at config 3 a frame moves 5.5 MB up and up to

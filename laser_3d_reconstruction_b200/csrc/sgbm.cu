@@ -70,7 +70,7 @@ int make_geom(const l3d_sgbm_params& p, int W, int H, Geom& g, std::string* err)
         set_err(err, "sgbm: P2=%d with blockSize=%d exceeds the 16-bit cost domain", g.P2, g.bs);
         return L3D_ERR_UNSUPPORTED;
     }
-    g.minX1 = std::max(g.maxD, 0); g.maxX1 = W + std::min(g.minD, 0); g.width1 = g.maxX1 - g.minX1;
+    g.minX1 = std::max(g.maxD, 0); g.maxX1 = W + std::min(g.minD, 0); g.width1 = sgbm_width1(p, W);
     g.DPL = g.D <= 64 ? 2 : (g.D <= 128 ? 4 : (g.D <= 256 ? 8 : 16));
     g.NP = g.DPL / 2;
     g.nact = g.D / g.DPL;
@@ -765,7 +765,7 @@ static int launch_scan_np(Lane& L, int NP, int smode, const ScanArgs& sa, int li
 //                               + middle (the previous-row paths: cluster-fused or direction-split)
 //                               + back (WTA if not fused, LR check, median, speckles).
 // The frame pipeline runs the fronts of a group of frames on their lanes, ONE cluster-fused middle
-// launch per pass over all the group's volumes, and the backs on the lanes again (api.cu).
+// launch per pass over all the group's volumes, and the backs on the lanes again (pipeline.cu).
 // ------------------------------------------------------------------------------------------
 
 static void scan_args_of(const SgbmRun& r, ScanArgs& sa) {
@@ -994,7 +994,8 @@ int sgbm_middle_vgroup(Lane& L, SgbmRun* const* runs, int nruns, bool keep_S) {
 }
 
 // can all eight paths of this geometry go through the wavefront kernel?  (MODE_HH only: its two passes carry four paths each)
-// L3D_VWAVE (read at every call, so that a test can switch it): 0 = never, 1 = wherever the kernel covers the geometry,
+// L3D_VWAVE (read at every call; the frame pipeline calls this once, when it is created, so that a test can switch it
+// per pipeline): 0 = never, 1 = wherever the kernel covers the geometry,
 // unset = where it is the faster choice (vwave_pays)
 bool sgbm_vwave_ok(int width1, int H, int D, int mode) {
     const char* e = getenv("L3D_VWAVE");

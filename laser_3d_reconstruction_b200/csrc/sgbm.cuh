@@ -1,4 +1,5 @@
-// sgbm.cuh -- types shared by the StereoSGBM translation units (sgbm_cost.cu, sgbm.cu, sgbm_hrow.cu, api.cu).
+// sgbm.cuh -- types shared by the StereoSGBM translation units (sgbm_cost.cu, sgbm.cu) and the C ABI's (api.cu,
+// pipeline.cu, through api.cuh).
 // Internal to libl3d.so.
 #pragma once
 #include "common.cuh"
@@ -16,6 +17,10 @@ struct Geom {
     int seg_shift[MAXSEG];  // SGBM_3WAY on images of a few rows: output row = computed row - shift (make_geom)
 };
 int make_geom(const l3d_sgbm_params& p, int W, int H, Geom& g, std::string* err);
+// columns of the cost volume: maxX1 - minX1 of make_geom (<= 0: no column has a full disparity range)
+inline int sgbm_width1(const l3d_sgbm_params& p, int W) {
+    return (W + std::min(p.minDisparity, 0)) - std::max(p.minDisparity + p.numDisparities, 0);
+}
 
 // One matcher run = front (BT operands, cost volume, both horizontal paths)
 //                 + middle (the previous-row paths: cluster-fused or direction-split)

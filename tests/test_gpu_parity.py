@@ -773,7 +773,7 @@ def test_grouped_pipeline_ragged_geometry(ctx, W, H, D, bs, policy):
     results = {}
     saved = os.environ.get("L3D_VWAVE")
     if policy is not None:
-        os.environ["L3D_VWAVE"] = policy  # read by the library at every pipeline run
+        os.environ["L3D_VWAVE"] = policy  # read by the library when a pipeline is created
     try:
         for lanes in (2, 14):
             cfg = pipeline.make_pipeline_config(W, H, D, bs, mode, Q, K, extractor=N.STEGER_IMPROVED, lanes=lanes, max_points=8000)
