@@ -193,6 +193,13 @@ __device__ __noinline__ bool vw_not_unique(typename VwVec<NP>::T wv, unsigned ke
 //   B, column 0   -> right edge out (the left neighbour needs it for its NEXT row, late in its row-time)
 //   A columns, B columns 1 .. CPW-2, right edge in (the right neighbour's B state after the previous row), B column CPW-1
 //   V + S sum (+ winner-takes-all keys) per column, epilogue, TMA store / loads
+// PAIRED (D = 128, an even CPW >= 4): the A, V and B paths of columns p and p + CPW/2 run as one sgm_step_pair, so "column j"
+// above reads "slot j" and the diagonal hand-off stays a register rename (A of slot p reads slot p-1, B reads slot p+1).  The
+// edge slots of the neighbours carry one column in sgm_step's layout as before; the first and the last slot assemble their
+// mixed input (A: the left neighbour's column and my column CPW/2 - 1; B: my column CPW/2, kept from before slot 0 moved
+// on, and the right neighbour's column) with PRMTs.  V runs beside A on the same interleaved costs; the S sum adds A + B +
+// V of both columns in the paired layout and splits it before the horizontal path's costs are added.  Odd CPW, and
+// D = 64 / 256, keep one column per slot (sgm_step).
 // NW = warps per CTA: 16 (128 registers per thread) up to D = 128, 8 (255 registers) at D = 256, where a column's state is
 // 15 registers.  At D = 256 the neighbour slots are single-buffered (SB) and the last pass adds the horizontal path's
 // costs into the S row in place (HIP): see vwave_warp_bytes.
@@ -214,6 +221,9 @@ __global__ void __launch_bounds__(NW * 32, 1) sgbm_vwave_kernel(const VWaveArgs 
     constexpr uint32_t WB = WBS + (LAST && !HIP ? rowb : 0);                         // + the horizontal path's row
     constexpr int DIR = LAST ? -1 : 1;
     constexpr bool UNROLL2 = !LAST && NP <= 2;
+    // the previous-row paths (A, V, B) of columns p and p + HP share words (sgm_step_pair); the horizontal chain cannot
+    constexpr bool PAIRED = NP == 2 && CPW % 2 == 0 && CPW >= 4;
+    constexpr int HP = CPW / 2, NS = PAIRED ? HP : CPW, NWD = PAIRED ? 4 : NP;
     extern __shared__ __align__(128) unsigned char vw_smem[];
     cg::cluster_group cluster = cg::this_cluster();
     const int rank = (int)cluster.block_rank();
@@ -284,13 +294,15 @@ __global__ void __launch_bounds__(NW * 32, 1) sgbm_vwave_kernel(const VWaveArgs 
         if (H > 1) load_row(1);
     }
 
-    // path state: A = diagonal fed from the left neighbour column, V = vertical, Bp = diagonal fed from the right
-    uint32_t LA[CPW][NP], LV[CPW][NP], LB[CPW][NP];
-    uint32_t mA[CPW], mV[CPW], mB[CPW];
+    // path state: A = diagonal fed from the left neighbour column, V = vertical, Bp = diagonal fed from the right.
+    // PAIRED: slot p holds columns p (low halves) and p + HP (high halves) in sgm_step_pair's layout, 4 words per lane;
+    // otherwise slot j is column j, NP words in sgm_step's layout.
+    uint32_t LA[NS][NWD], LV[NS][NWD], LB[NS][NWD];
+    uint32_t mA[NS], mV[NS], mB[NS];
 #pragma unroll
-    for (int j = 0; j < CPW; j++) {
+    for (int j = 0; j < NS; j++) {
 #pragma unroll
-        for (int k = 0; k < NP; k++) { LA[j][k] = 0; LV[j][k] = 0; LB[j][k] = 0; }
+        for (int k = 0; k < NWD; k++) { LA[j][k] = 0; LV[j][k] = 0; LB[j][k] = 0; }
         mA[j] = 0; mV[j] = 0; mB[j] = 0;
     }
     const uint32_t p1x2 = (uint32_t)a.P1 * 0x10001u;
@@ -374,53 +386,115 @@ __global__ void __launch_bounds__(NW * 32, 1) sgbm_vwave_kernel(const VWaveArgs 
 #pragma unroll
             for (int j = 0; j < CPW; j++) h_column(JB(j), valid(j));
         }
-        // ---- left edge out
+        // PAIRED: one column of a slot in sgm_step's layout (k = 0: the low halves, 1: the high halves).  The minimum words
+        // that go with an edge slot stay packed (min of column p | min of column p + HP << 16): the consumer picks its half.
+        auto half_of = [&](const uint32_t (&w)[NWD], int k, uint32_t (&o)[NP]) {
+            const uint32_t sel = k ? 0x7632u : 0x5410u;
+            o[0] = __byte_perm(w[0], w[1 % NWD], sel);
+            o[NP - 1] = __byte_perm(w[2 % NWD], w[3 % NWD], sel);
+        };
+        // PAIRED: the costs of every slot, interleaved once per row (below) and shared by its A, V and B steps
+        [[maybe_unused]] uint32_t Cs[PAIRED ? NS : 1][NWD];
+        auto c_slot = [&](int p, uint32_t (&Cp)[NWD]) {
+            if constexpr (PAIRED) {
+#pragma unroll
+                for (int k = 0; k < NWD; k++) Cp[k] = Cs[p][k];
+            } else {
+                vw_unpack<NP>(cs[JB(p) * 32], Cp);
+            }
+        };
+        auto step = [&](uint32_t (&O)[NWD], const uint32_t (&I)[NWD], uint32_t minI2, const uint32_t (&Cp)[NWD]) -> uint32_t {
+            if constexpr (PAIRED) return sgm_step_pair(O, I, minI2, Cp, p1x2, k2, sl);
+            else return sgm_step<NP>(O, I, minI2, Cp, p1x2, k2, sl);
+        };
+        // ---- left edge out: my last column's A state as it still is (after the previous row)
         if (has_right) {
+            uint32_t eA[NP], emA;
+            if constexpr (PAIRED) { half_of(LA[HP - 1], 1, eA); emA = mA[HP - 1]; }   // column CPW - 1: the high half
+            else {
+#pragma unroll
+                for (int k = 0; k < NP; k++) eA[k] = LA[CPW - 1][k % NWD];
+                emA = mA[CPW - 1];
+            }
             if (reuse) vw_mbar_wait(sblk_s + B_LE, fph);
             const uint32_t q = nbR + sso + O_LIN, rb = nbR + sso + B_LF;
             if (!right_remote) {
                 vw_st_local_vec<NP>(q + lane * (uint32_t)sizeof(vec), LH);
-                vw_st_local_vec<NP>(q + slot + lane * (uint32_t)sizeof(vec), LA[CPW - 1]);
+                vw_st_local_vec<NP>(q + slot + lane * (uint32_t)sizeof(vec), eA);
                 vw_st_shared_if(q + B, mH, lane0);
-                vw_st_shared_if(q + slot + B, mA[CPW - 1], lane0);
+                vw_st_shared_if(q + slot + B, emA, lane0);
                 __syncwarp();
                 vw_mbar_arrive_if(rb, lane0);
             } else {
                 vw_st_async_vec<NP>(q + lane * (uint32_t)sizeof(vec), LH, rb);
-                vw_st_async_vec<NP>(q + slot + lane * (uint32_t)sizeof(vec), LA[CPW - 1], rb);
+                vw_st_async_vec<NP>(q + slot + lane * (uint32_t)sizeof(vec), eA, rb);
                 vw_st_async_if(q + B, mH, rb, lane0);
-                vw_st_async_if(q + slot + B, mA[CPW - 1], rb, lane0);
+                vw_st_async_if(q + slot + B, emA, rb, lane0);
             }
         }
-        // ---- B path, first column, and right edge out
-        vw_unpack<NP>(cs[JB(0) * 32], Cw);
-        mB[0] = sgm_step<NP>(LB[0], LB[1], mB[1], Cw, p1x2, k2, sl);
+        // A of slot 0 reads (the left neighbour's last column, my column HP - 1): assembled before slot HP - 1 moves on
+        uint32_t inA0[NWD], inA0m;
+        if constexpr (PAIRED) {
+            inA0[0] = __byte_perm(inA[0], LA[HP - 1][0], 0x5410); inA0[1] = __byte_perm(inA[0], LA[HP - 1][1], 0x5432);
+            inA0[2] = __byte_perm(inA[1], LA[HP - 1][2], 0x5410); inA0[3] = __byte_perm(inA[1], LA[HP - 1][3], 0x5432);
+            inA0m = __byte_perm(inAm, mA[HP - 1], 0x5432);
+        } else {
+#pragma unroll
+            for (int k = 0; k < NWD; k++) inA0[k] = inA[k % NP];
+            inA0m = inAm;
+        }
+        // ---- B path, first column (slot 0), and right edge out.  PAIRED: B of the last slot reads (column HP, the right
+        // neighbour's first column); column HP is the high half of slot 0, kept here as it was after the previous row.
+        [[maybe_unused]] uint32_t svB[NP], svBm = 0;
+        if constexpr (PAIRED) { half_of(LB[0], 1, svB); svBm = mB[0]; }
+        if constexpr (PAIRED) {
+#pragma unroll
+            for (int p = 0; p < NS; p++) {
+                uint32_t ca[NP], cb[NP];
+                vw_unpack<NP>(cs[JB(p) * 32], ca);
+                vw_unpack<NP>(cs[JB(p + HP) * 32], cb);
+                Cs[p][0] = __byte_perm(ca[0], cb[0], 0x5410); Cs[p][1] = __byte_perm(ca[0], cb[0], 0x7632);
+                Cs[p][2] = __byte_perm(ca[1], cb[1], 0x5410); Cs[p][3] = __byte_perm(ca[1], cb[1], 0x7632);
+            }
+        }
+        uint32_t Cp[NWD];
+        c_slot(0, Cp);
+        mB[0] = step(LB[0], LB[1], mB[1], Cp);
         if (has_left && it + 1 < H) {
+            uint32_t eB[NP], emB;
+            if constexpr (PAIRED) { half_of(LB[0], 0, eB); emB = mB[0]; }   // column 0: the low half
+            else {
+#pragma unroll
+                for (int k = 0; k < NP; k++) eB[k] = LB[0][k % NWD];
+                emB = mB[0];
+            }
             if (reuse) vw_mbar_wait(sblk_s + B_RE, fph);                // the neighbour has read the slot's previous content
             const uint32_t q = nbL + sso + O_RIN, rb = nbL + sso + B_RF;
             if (!left_remote) {
-                vw_st_local_vec<NP>(q + lane * (uint32_t)sizeof(vec), LB[0]);
-                vw_st_shared_if(q + B, mB[0], lane0);
+                vw_st_local_vec<NP>(q + lane * (uint32_t)sizeof(vec), eB);
+                vw_st_shared_if(q + B, emB, lane0);
                 __syncwarp();
                 vw_mbar_arrive_if(rb, lane0);
             } else {
-                vw_st_async_vec<NP>(q + lane * (uint32_t)sizeof(vec), LB[0], rb);
-                vw_st_async_if(q + B, mB[0], rb, lane0);
+                vw_st_async_vec<NP>(q + lane * (uint32_t)sizeof(vec), eB, rb);
+                vw_st_async_if(q + B, emB, rb, lane0);
             }
         }
-        // ---- diagonal A (fed from the left): in place, right to left (column j reads column j-1's old state)
+        // ---- diagonal A (fed from the left): in place, right to left (slot j reads slot j-1's old state)
 #pragma unroll
-        for (int j = CPW - 1; j >= 1; j--) {
-            vw_unpack<NP>(cs[JB(j) * 32], Cw);
-            mA[j] = sgm_step<NP>(LA[j], LA[j - 1], mA[j - 1], Cw, p1x2, k2, sl);
+        for (int j = NS - 1; j >= 1; j--) {
+            c_slot(j, Cp);
+            mA[j] = step(LA[j], LA[j - 1], mA[j - 1], Cp);
+            if (PAIRED) mV[j] = step(LV[j], LV[j], mV[j], Cp);   // (PAIRED: V shares the interleaved costs with A)
         }
-        vw_unpack<NP>(cs[JB(0) * 32], Cw);
-        mA[0] = sgm_step<NP>(LA[0], inA, inAm, Cw, p1x2, k2, sl);
-        // ---- diagonal B (fed from the right): in place, left to right; the last column needs the right neighbour's state
+        c_slot(0, Cp);
+        mA[0] = step(LA[0], inA0, inA0m, Cp);
+        if (PAIRED) mV[0] = step(LV[0], LV[0], mV[0], Cp);
+        // ---- diagonal B (fed from the right): in place, left to right; the last slot needs the right neighbour's state
 #pragma unroll
-        for (int j = 1; j < CPW - 1; j++) {
-            vw_unpack<NP>(cs[JB(j) * 32], Cw);
-            mB[j] = sgm_step<NP>(LB[j], LB[j + 1], mB[j + 1], Cw, p1x2, k2, sl);
+        for (int j = 1; j < NS - 1; j++) {
+            c_slot(j, Cp);
+            mB[j] = step(LB[j], LB[j + 1], mB[j + 1], Cp);
         }
         {
             uint32_t inB[NP], inBm = 0;
@@ -441,16 +515,31 @@ __global__ void __launch_bounds__(NW * 32, 1) sgbm_vwave_kernel(const VWaveArgs 
                 const uint32_t dep = (inB[0] | inBm) & sl.zero;
                 if (right_remote) vw_mbar_arrive_remote_if(nbR + seo + B_RE + dep, lane0); else vw_mbar_arrive_if(nbR + seo + B_RE, lane0);
             }
-            vw_unpack<NP>(cs[JB(CPW - 1) * 32], Cw);
-            mB[CPW - 1] = sgm_step<NP>(LB[CPW - 1], inB, inBm, Cw, p1x2, k2, sl);
+            uint32_t inBL[NWD], inBLm;
+            if constexpr (PAIRED) {
+                inBL[0] = __byte_perm(svB[0], inB[0], 0x5410); inBL[1] = __byte_perm(svB[0], inB[0], 0x7632);
+                inBL[2] = __byte_perm(svB[1], inB[1], 0x5410); inBL[3] = __byte_perm(svB[1], inB[1], 0x7632);
+                inBLm = __byte_perm(svBm, inBm, 0x5432);
+            } else {
+#pragma unroll
+                for (int k = 0; k < NWD; k++) inBL[k] = inB[k % NP];
+                inBLm = inBm;
+            }
+            c_slot(NS - 1, Cp);
+            mB[NS - 1] = step(LB[NS - 1], inBL, inBLm, Cp);
         }
         if (!FULL && ncols < CPW) {
             // columns outside the volume: their state must read as "no predecessor" (0) for the last valid column
 #pragma unroll
-            for (int j = 0; j < CPW; j++) {
-                if (j >= ncols) {
+            for (int j = 0; j < NS; j++) {
+                if constexpr (PAIRED) {   // slot j holds columns j and j + HP
+                    const uint32_t keep = (j < ncols ? 0xffffu : 0u) | (j + HP < ncols ? 0xffff0000u : 0u);
 #pragma unroll
-                    for (int k = 0; k < NP; k++) LB[j][k] = 0;
+                    for (int k = 0; k < NWD; k++) LB[j][k] &= keep;
+                    mB[j] &= keep;
+                } else if (j >= ncols) {
+#pragma unroll
+                    for (int k = 0; k < NWD; k++) LB[j][k] = 0;
                     mB[j] = 0;
                 }
             }
@@ -471,25 +560,50 @@ __global__ void __launch_bounds__(NW * 32, 1) sgbm_vwave_kernel(const VWaveArgs 
             if (lane == j) { wkey = key; wrej = rej; }
         };
 #pragma unroll
-        for (int j = 0; j < CPW; j++) {
-            vw_unpack<NP>(cs[JB(j) * 32], Cw);
-            mV[j] = sgm_step<NP>(LV[j], LV[j], mV[j], Cw, p1x2, k2, sl);
-            uint32_t Sw[NP], Hw[NP];
-            if (!(LAST && HIP)) vw_unpack<NP>(hs[JB(j) * 32], Hw);
-            if (LAST) vw_unpack<NP>(ss[JB(j) * 32], Sw);
+        for (int j = 0; j < NS; j++) {
+            if constexpr (PAIRED) {
+                // A + B + V of both columns at once, then per column + H (+ S): all terms are non-negative and at most
+                // 32767, so the saturating adds give min(sum, 32767) in any order
+                uint32_t s3[NWD];
 #pragma unroll
-            for (int k = 0; k < NP; k++) {
-                uint32_t s3 = __viaddmin_u16x2(LA[j][k], LB[j][k], INF);
-                if (LAST && HIP) {
-                    s3 = __viaddmin_u16x2(s3, LV[j][k], INF);
-                } else {
-                    const uint32_t s4 = __viaddmin_u16x2(LV[j][k], Hw[k], INF);
-                    s3 = __viaddmin_u16x2(s3, s4, INF);
+                for (int k = 0; k < NWD; k++) s3[k] = __viaddmin_u16x2(__viaddmin_u16x2(LA[j][k], LB[j][k], INF), LV[j][k], INF);
+#pragma unroll
+                for (int h = 0; h < 2; h++) {
+                    const int jc = j + h * HP;
+                    uint32_t Sw[NP], Hw[NP];
+                    half_of(s3, h, Sw);
+                    vw_unpack<NP>(hs[JB(jc) * 32], Hw);
+#pragma unroll
+                    for (int k = 0; k < NP; k++) Sw[k] = __viaddmin_u16x2(Sw[k], Hw[k], INF);
+                    if (LAST) {
+                        uint32_t Sr[NP];
+                        vw_unpack<NP>(ss[JB(jc) * 32], Sr);
+#pragma unroll
+                        for (int k = 0; k < NP; k++) Sw[k] = __viaddmin_u16x2(Sr[k], Sw[k], INF);
+                    }
+                    if (valid(jc)) ss[JB(jc) * 32] = vw_pack<NP>(Sw);
+                    if (LAST) wta_column(Sw, jc);
                 }
-                Sw[k] = LAST ? __viaddmin_u16x2(Sw[k], s3, INF) : s3;
+            } else {
+                c_slot(j, Cp);
+                mV[j] = step(LV[j], LV[j], mV[j], Cp);
+                uint32_t Sw[NP], Hw[NP];
+                if (!(LAST && HIP)) vw_unpack<NP>(hs[JB(j) * 32], Hw);
+                if (LAST) vw_unpack<NP>(ss[JB(j) * 32], Sw);
+#pragma unroll
+                for (int k = 0; k < NP; k++) {
+                    uint32_t s3 = __viaddmin_u16x2(LA[j][k % NWD], LB[j][k % NWD], INF);
+                    if (LAST && HIP) {
+                        s3 = __viaddmin_u16x2(s3, LV[j][k % NWD], INF);
+                    } else {
+                        const uint32_t s4 = __viaddmin_u16x2(LV[j][k % NWD], Hw[k], INF);
+                        s3 = __viaddmin_u16x2(s3, s4, INF);
+                    }
+                    Sw[k] = LAST ? __viaddmin_u16x2(Sw[k], s3, INF) : s3;
+                }
+                if (valid(j)) ss[JB(j) * 32] = vw_pack<NP>(Sw);  // columns outside the volume alias block column 0: never stored
+                if (LAST && !ROLLH) wta_column(Sw, j);
             }
-            if (valid(j)) ss[JB(j) * 32] = vw_pack<NP>(Sw);  // columns outside the volume alias block column 0: never stored
-            if (LAST && !ROLLH) wta_column(Sw, j);
         }
         if (LAST && ROLLH) {
             // winner-takes-all keys from the finished S row in shared memory, as a real loop (instruction footprint, see

@@ -2,6 +2,8 @@
 // kernels of sgbm.cu, sgbm_hrow.cu and sgbm_vgroup.cu; cv2.StereoSGBM modes SGBM / HH / HH4 / 3WAY, SURVEY A4).
 //
 // A warp owns one pixel's disparity range, lane l holds 2*NP consecutive disparities as NP packed u16x2 words.
+// sgm_step_pair (below) runs two independent D = 128 recurrences in the two halves of the words instead: no funnel words,
+// no half-combine, 15 ALU-pipe instructions per step of the pair where two sgm_step<2> take 24.
 // With delta = min_d(I) + P2 the step is
 //     T[d] = min(I[d], I[d-1] + P1, I[d+1] + P1)          (I + P1 once per word on the FMA pipe, one VIMNMX3.U16x2)
 //     O[d] = min(T[d] + (C[d] - delta), C[d])             (one VIADD.16x2, one VIADDMNMX.U16x2)
@@ -43,6 +45,8 @@ struct SgmLane {
     uint32_t neg1;        // 0xffffffff, opaque
     uint32_t m64k;        // 65536, opaque
     uint32_t one;         // 1, opaque
+    uint32_t upm, upa;    // sgm_step_pair: the d-1 word from the lane below is x * upm + upa (lane 0: all ones, never wins)
+    uint32_t dnm, dna;    // sgm_step_pair: the d+1 word from the lane above is x * dnm + dna (lane 31: all ones)
 };
 // zero_param = 0: a value the compiler cannot see (kernel parameter)
 __device__ __forceinline__ SgmLane sgm_lane_init(int lane, uint32_t zero_param) {
@@ -50,6 +54,8 @@ __device__ __forceinline__ SgmLane sgm_lane_init(int lane, uint32_t zero_param) 
     s.selA = lane == 0 ? 0x5454u : 0x5432u;
     s.selB = lane == 31 ? 0x3232u : 0x5432u;
     s.zero = zero_param; s.neg1 = ~zero_param; s.m64k = zero_param + 65536u; s.one = zero_param + 1u;
+    s.upm = zero_param + (lane == 0 ? 0u : 1u); s.upa = lane == 0 ? ~zero_param : zero_param;
+    s.dnm = zero_param + (lane == 31 ? 0u : 1u); s.dna = lane == 31 ? ~zero_param : zero_param;
     return s;
 }
 
@@ -102,6 +108,36 @@ __device__ __forceinline__ uint32_t sgm_step(uint32_t (&O)[NP], const uint32_t (
     for (int k = 0; k < NP; k++) O[k] = Ln[k];
     mn = __vminu2(mn, __byte_perm(mn, mn, 0x1032));  // both halves = min of the two
     return __reduce_min_sync(0xffffffffu, mn);        // packed halves are equal, so the u32 min is the packed min
+}
+
+// Two independent D = 128 recurrences at once (the paired form): word k of lane l holds disparity 4l + k of recurrence
+// a in its low half and of recurrence b in its high half, so the d-1 / d+1 neighbours of word k are words k-1 / k+1 and
+// only words 0 and 3 take one from the next lane (SHFL up / down; lanes 0 and 31 put all ones there through a
+// multiply-add with per-lane constants, FMA pipe).  The per-half arithmetic is sgm_step's.  minI2 and the result are
+// (min a | min b << 16): the four-word min tree gives the two per-lane minima directly, the warp takes them with two
+// CREDUX.MIN -- one on m (high half: min of the high halves), one on m << 16 (IMAD, FMA pipe: high half = min of the low
+// halves) -- and one PRMT repacks them.  Per step of the pair: 15 ALU-pipe instructions (4 VIMNMX3, 4 VADD2, 4 VIADDMNMX,
+// 2 min tree, 1 PRMT), 8 on the FMA pipe, 2 SHFL, 2 CREDUX; two sgm_step<2> take 24, ~8, 4 and 2.
+__device__ __forceinline__ uint32_t sgm_step_pair(uint32_t (&O)[4], const uint32_t (&I)[4], uint32_t minI2,
+                                                  const uint32_t (&Cv)[4], uint32_t p1x2, uint32_t k2, const SgmLane& s) {
+    uint32_t Ip[4];
+#pragma unroll
+    for (int k = 0; k < 4; k++) Ip[k] = sgm_madlo(I[k], s.one, p1x2);
+    const uint32_t up = sgm_madlo(__shfl_up_sync(0xffffffffu, Ip[3], 1), s.upm, s.upa);
+    const uint32_t dn = sgm_madlo(__shfl_down_sync(0xffffffffu, Ip[0], 1), s.dnm, s.dna);
+    const uint32_t nd2 = sgm_madlo(minI2, s.neg1, k2);
+    uint32_t Ln[4];
+#pragma unroll
+    for (int k = 0; k < 4; k++) {
+        const uint32_t t = __vimin3_u16x2(I[k], k ? Ip[k - 1] : up, k < 3 ? Ip[k + 1] : dn);
+        Ln[k] = __viaddmin_u16x2(t, __vadd2(Cv[k], nd2), Cv[k]);
+    }
+    const uint32_t mn = __vimin3_u16x2(__vminu2(Ln[0], Ln[1]), Ln[2], Ln[3]);
+#pragma unroll
+    for (int k = 0; k < 4; k++) O[k] = Ln[k];
+    const uint32_t hi = __reduce_min_sync(0xffffffffu, mn);
+    const uint32_t lo = __reduce_min_sync(0xffffffffu, sgm_madlo(mn, s.m64k, s.zero));
+    return __byte_perm(lo, hi, 0x7632);
 }
 
 }  // namespace l3d

@@ -144,6 +144,78 @@ __global__ void __launch_bounds__(512) bench(const uint32_t* __restrict__ cost, 
     if (threadIdx.x == 0 && blockIdx.x == 0) *cyc = t1 - t0;
 }
 
+// The paired form (sgm_step_pair) against sgm_step<2> on the same work: NPAIR pairs of D = 128 recurrences per warp,
+// pair c = recurrences (2c, 2c + 1) over cost rows (r, r + 1), each pair starting from its own state (so that nothing is
+// common to two pairs).  PAIRED = false runs the 2 NPAIR recurrences one by one with sgm_step<2>; PAIRED = true
+// interleaves the two cost rows once per step (four PRMTs, shared by the pairs, as in the kernel where the A, V and B
+// paths of a column pair read the same costs) and runs sgm_step_pair.  Both hash the states in sgm_step's layout.
+constexpr int NPAIR = 3;
+template <bool PAIRED>
+__global__ void __launch_bounds__(512) bench_pair(const uint32_t* __restrict__ cost, uint32_t* out, int iters, int P1, int P2,
+                                                  uint32_t zero, long long* cyc) {
+    __shared__ uint32_t cs[ROWS][64];
+    for (int i = threadIdx.x; i < ROWS * 64; i += blockDim.x) (&cs[0][0])[i] = cost[i];
+    __syncthreads();
+    const int lane = threadIdx.x & 31;
+    const uint32_t p1x2 = (uint32_t)P1 * 0x10001u, k2 = (0x10000u - (uint32_t)P2) * 0x10001u;
+    const SgmLane sl = sgm_lane_init(lane, zero);
+    uint32_t L[2 * NPAIR][2], mn[2 * NPAIR];   // sgm_step's layout (PAIRED = false)
+    uint32_t P[NPAIR][4], pm[NPAIR];           // paired layout
+    for (int c = 0; c < NPAIR; c++) {
+        const uint32_t v = (uint32_t)(100 * c + 7) * 0x10001u;
+        for (int k = 0; k < 2; k++) L[2 * c][k] = L[2 * c + 1][k] = v;
+        for (int k = 0; k < 4; k++) P[c][k] = v;
+        mn[2 * c] = mn[2 * c + 1] = v; pm[c] = v;
+    }
+    long long t0 = clock64();
+    for (int it = 0; it < iters; it++) {
+        const int r = it & (ROWS - 1);
+        const uint2 ca = *(const uint2*)&cs[r][lane * 2], cb = *(const uint2*)&cs[(r + 1) & (ROWS - 1)][lane * 2];
+        if (PAIRED) {
+            const uint32_t Cw[4] = {__byte_perm(ca.x, cb.x, 0x5410), __byte_perm(ca.x, cb.x, 0x7632),
+                                    __byte_perm(ca.y, cb.y, 0x5410), __byte_perm(ca.y, cb.y, 0x7632)};
+#pragma unroll
+            for (int c = 0; c < NPAIR; c++) pm[c] = sgm_step_pair(P[c], P[c], pm[c], Cw, p1x2, k2, sl);
+        } else {
+            const uint32_t Ca[2] = {ca.x, ca.y}, Cb[2] = {cb.x, cb.y};
+#pragma unroll
+            for (int c = 0; c < NPAIR; c++) {
+                mn[2 * c] = sgm_step<2>(L[2 * c], L[2 * c], mn[2 * c], Ca, p1x2, k2, sl);
+                mn[2 * c + 1] = sgm_step<2>(L[2 * c + 1], L[2 * c + 1], mn[2 * c + 1], Cb, p1x2, k2, sl);
+            }
+        }
+    }
+    long long t1 = clock64();
+    if (PAIRED) {
+        for (int c = 0; c < NPAIR; c++) {
+            L[2 * c][0] = __byte_perm(P[c][0], P[c][1], 0x5410); L[2 * c][1] = __byte_perm(P[c][2], P[c][3], 0x5410);
+            L[2 * c + 1][0] = __byte_perm(P[c][0], P[c][1], 0x7632); L[2 * c + 1][1] = __byte_perm(P[c][2], P[c][3], 0x7632);
+            mn[2 * c] = (pm[c] & 0xffffu) * 0x10001u; mn[2 * c + 1] = (pm[c] >> 16) * 0x10001u;
+        }
+    }
+    uint32_t acc = 0;
+    for (int c = 0; c < 2 * NPAIR; c++) { for (int k = 0; k < 2; k++) acc = acc * 31u + L[c][k]; acc = acc * 31u + mn[c]; }
+    out[blockIdx.x * blockDim.x + threadIdx.x] = acc;
+    if (threadIdx.x == 0 && blockIdx.x == 0) *cyc = t1 - t0;
+}
+
+template <bool PAIRED>
+static void run_pair(const char* name, const uint32_t* cost, uint32_t* out, uint32_t* host, long long* cyc, int P1, int P2) {
+    const int iters = 20000, n = 148 * 512;
+    cudaEvent_t a, b; cudaEventCreate(&a); cudaEventCreate(&b);
+    bench_pair<PAIRED><<<148, 512>>>(cost, out, 100, P1, P2, 0u, cyc);
+    cudaEventRecord(a);
+    bench_pair<PAIRED><<<148, 512>>>(cost, out, iters, P1, P2, 0u, cyc);
+    cudaEventRecord(b); cudaEventSynchronize(b);
+    float ms; cudaEventElapsedTime(&ms, a, b);
+    long long c; cudaMemcpy(&c, cyc, 8, cudaMemcpyDeviceToHost);
+    cudaMemcpy(host, out, n * 4, cudaMemcpyDeviceToHost);
+    unsigned long long h = 0; for (int i = 0; i < n; i++) h = h * 1000003ull + host[i];
+    const double per = (double)c / (iters * 2 * NPAIR);
+    printf("D=128 %-34s %8.3f ms  %7.2f cycles per (warp, vector-step) at 16 warps/SM = %6.2f per SM-subpartition-step   hash %016llx  err=%s\n",
+           name, ms, per, per / 4.0, h, cudaGetErrorString(cudaGetLastError()));
+}
+
 template <int NP, int FORM>
 static void run(const char* name, const uint32_t* cost, uint32_t* out, uint32_t* host, long long* cyc, int P1, int P2) {
     const int iters = 20000, n = 148 * 512;
@@ -181,6 +253,10 @@ int main() {
     run<2, 4>("+ L = min(T,delta) + (C-delta)", cost, out, host, cyc, P1, P2);
     run<2, 5>("+ two CREDUX min tree", cost, out, host, cyc, P1, P2);
     run<2, 9>("form 3, min(T + (C-delta), C)", cost, out, host, cyc, P1, P2);
+    run_pair<false>("sgm_step<2>, 6 recurrences", cost, out, host, cyc, P1, P2);
+    run_pair<true>("sgm_step_pair, 3 pairs", cost, out, host, cyc, P1, P2);
+    run_pair<false>("sgm_step<2>, 6 recurrences", cost, out, host, cyc, P1, P2);
+    run_pair<true>("sgm_step_pair, 3 pairs", cost, out, host, cyc, P1, P2);
     run<4, 9>("form 3, min(T + (C-delta), C)", cost, out, host, cyc, P1, P2);
     run<1, 9>("form 3, min(T + (C-delta), C)", cost, out, host, cyc, P1, P2);
     run<2, 6>("form 4 without the reduction", cost, out, host, cyc, P1, P2);
