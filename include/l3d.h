@@ -60,6 +60,30 @@ int l3d_voxel_downsample(l3d_ctx* ctx, const double* points, int n, double voxel
 int l3d_statistical_outlier_removal(l3d_ctx* ctx, const double* points, int n, int nb_neighbors, double std_ratio,
                                     double* out, int* n_out);
 
+/* -------- laser-plane fit (no reference counterpart: the reference takes the plane as a constant, config.py) --------
+ * RANSAC + least-squares refinement of a plane a x + b y + c z + d = 0 through n points (xyz: n x 3 f64, host).
+ * Hypothesis h in [0, hypotheses) takes the points i_k = splitmix64(seed + (3h + k + 1) * 0x9E3779B97F4A7C15) mod n,
+ * k = 0..2; its plane is n = (p1 - p0) x (p2 - p0), n / |n|, d = -n.p0, and a point is its inlier iff
+ * |((n.x p.x + n.y p.y) + n.z p.z) + d| <= threshold, every operation f64 round-to-nearest without FMA contraction
+ * (DESIGN.md section 4f has the exact contract).  A hypothesis with a non-finite point or |n| not in (0, inf) is
+ * invalid.  The winner has the most inliers (ties: lowest h).  Refinement, at most 10 times: centroid and covariance
+ * (divided by the count) of the inlier set S, normal = eigenvector of the smallest eigenvalue, d = -n.c, reselect S';
+ * stop when S' == S.  Output: the last fit with d >= 0, its S' (inliers, inlier_mask: n bytes 0/1, may be NULL), the
+ * rms residual over S'.  L3D_ERR_ARG: n < 3, threshold not finite or <= 0, hypotheses outside [1, 2^20], no valid
+ * hypothesis, a fit left with fewer than 3 inliers.  Deterministic: the same input gives the same bits. */
+typedef struct { double threshold; int hypotheses; unsigned long long seed; } l3d_plane_fit_params;
+typedef struct {
+    double plane[4];        /* unit normal, d >= 0 */
+    int inliers;            /* points within threshold of `plane` */
+    double rms;             /* sqrt(mean residual^2) over those inliers */
+    double eig[3];          /* ascending eigenvalues of the last least-squares fit's inlier covariance */
+    int hypothesis;         /* index of the winning RANSAC hypothesis */
+    int hypothesis_inliers; /* its inlier count */
+    int refits;             /* least-squares fits done */
+} l3d_plane_fit_result;
+int l3d_fit_plane(l3d_ctx* ctx, const double* xyz, int n, const l3d_plane_fit_params* p, l3d_plane_fit_result* out,
+                  uint8_t* inlier_mask);
+
 /* -------- init-time rectification maps (SURVEY 8f N3) ------------------------------------------
  * cv2.initUndistortRectifyMap(K, dist, R, P, (W, H), CV_32FC1) -> mapx, mapy (f32 HxW), as called once per eye in
  * camera/single_usb_stereo_camera.py:190-206.  K = 3x3 row-major; dist = ndist <= 14 coefficients

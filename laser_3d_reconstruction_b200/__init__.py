@@ -6,7 +6,7 @@ loads libl3d.so and raises if it (or a GPU) is missing -- there is no CPU fallba
 from .camera.single_usb_stereo_camera import SingleUSBStereoCameraManager
 from .config import Config
 from .core.laser_extractor import FastStegerExtractor, SimpleLaserExtractor
-from .core.reconstruction import Reconstructor
+from .core.reconstruction import LaserPlaneFit, Reconstructor, fit_laser_plane
 from .improved_reconstruction import ImprovedLaserReconstructor, fix_roi_alignment, visualize_laser_depth
 from .improved_steger import HybridLaserExtractor, ImprovedStegerExtractor, StegerLaserExtractor
 from .system import LaserReconstructionSystem
@@ -14,4 +14,5 @@ from .system import LaserReconstructionSystem
 __version__ = "0.1.0"
 __all__ = ["SingleUSBStereoCameraManager", "SimpleLaserExtractor", "FastStegerExtractor", "ImprovedStegerExtractor",
            "StegerLaserExtractor", "HybridLaserExtractor", "Reconstructor", "ImprovedLaserReconstructor",
-           "fix_roi_alignment", "visualize_laser_depth", "Config", "LaserReconstructionSystem"]
+           "fix_roi_alignment", "visualize_laser_depth", "Config", "LaserReconstructionSystem", "LaserPlaneFit",
+           "fit_laser_plane"]

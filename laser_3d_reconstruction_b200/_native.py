@@ -67,6 +67,17 @@ class PipelineConfig(C.Structure):
                 ("max_points", C.c_int), ("lanes", C.c_int)]
 
 
+class PlaneFitParams(C.Structure):
+    """include/l3d.h: l3d_plane_fit_params"""
+    _fields_ = [("threshold", C.c_double), ("hypotheses", C.c_int), ("seed", C.c_ulonglong)]
+
+
+class PlaneFitResult(C.Structure):
+    """include/l3d.h: l3d_plane_fit_result"""
+    _fields_ = [("plane", C.c_double * 4), ("inliers", C.c_int), ("rms", C.c_double), ("eig", C.c_double * 3),
+                ("hypothesis", C.c_int), ("hypothesis_inliers", C.c_int), ("refits", C.c_int)]
+
+
 STEGER_FAST, STEGER_IMPROVED, STEGER_OPTIMIZED, STEGER_HYBRID = 0, 1, 2, 3
 EXTRACT_SIMPLE = 4
 RECON_PLANE, RECON_DEPTH, RECON_DISPARITY, RECON_DISPARITY_MEDIAN = 0, 1, 2, 3
@@ -75,7 +86,7 @@ EXPORTS = (
     "l3d_ctx_create l3d_ctx_destroy l3d_last_error l3d_sync l3d_device_count l3d_version l3d_launch_count "
     "l3d_set_rectify_maps l3d_init_undistort_rectify_map l3d_remap_gray l3d_bgr2gray l3d_sgbm_compute l3d_sgbm_compute_pair l3d_sgbm_debug l3d_sgbm_volume_rows "
     "l3d_bm_compute l3d_median3_s16 l3d_filter_speckles l3d_wls_filter l3d_fgs_solve l3d_disp_to_depth l3d_compute_depth "
-    "l3d_simple_extract l3d_colour_mask l3d_steger_extract l3d_reconstruct l3d_laser_depth_map l3d_voxel_downsample l3d_statistical_outlier_removal l3d_pipeline_create l3d_pipeline_destroy "
+    "l3d_simple_extract l3d_colour_mask l3d_steger_extract l3d_reconstruct l3d_laser_depth_map l3d_voxel_downsample l3d_statistical_outlier_removal l3d_fit_plane l3d_pipeline_create l3d_pipeline_destroy "
     "l3d_pipeline_set_maps l3d_pipeline_run_dev l3d_pipeline_run_host l3d_pipeline_run_captures_dev "
     "l3d_pipeline_run_captures_host l3d_pipeline_fetch l3d_pipeline_fetch_points l3d_pipeline_points_needed "
     "l3d_pipeline_pack_points_dev l3d_pipeline_launch_count l3d_pipeline_graph_replays l3d_pipeline_last_ms l3d_pipeline_set_timing l3d_pipeline_kernel_time "
@@ -242,6 +253,21 @@ class Context:
                    "l3d_statistical_outlier_removal")
         res = out[:m.value]
         return res.astype(np.float32) if f32 else res.copy()
+
+    def fit_plane(self, points, threshold, hypotheses, seed):
+        """RANSAC + least-squares plane through n x 3 points (include/l3d.h: l3d_fit_plane).  -> dict with plane (4,)
+        float64 (unit normal, d >= 0), inlier_mask (n,) bool, inliers, rms, eig (3,) ascending, hypothesis,
+        hypothesis_inliers, refits"""
+        pts = np.ascontiguousarray(points, np.float64).reshape(-1, 3)
+        n = int(pts.shape[0])
+        p = PlaneFitParams(float(threshold), int(hypotheses), int(seed) & 0xFFFFFFFFFFFFFFFF)
+        r = PlaneFitResult()
+        mask = np.zeros(n, np.uint8)
+        self.check(self.lib.l3d_fit_plane(self.h, _ptr(pts) if n else None, n, C.byref(p), C.byref(r),
+                                          _ptr(mask) if n else None), "l3d_fit_plane")
+        return dict(plane=np.array(r.plane[:], np.float64), inlier_mask=mask.astype(bool), inliers=int(r.inliers),
+                    rms=float(r.rms), eig=np.array(r.eig[:], np.float64), hypothesis=int(r.hypothesis),
+                    hypothesis_inliers=int(r.hypothesis_inliers), refits=int(r.refits))
 
     def bm_compute(self, params, left, right):
         """cv2.StereoBM.compute(left, right) -> int16 disparity x16 (include/l3d.h: l3d_bm_compute)."""

@@ -6,7 +6,7 @@ filter_outliers / transform_points / merge_point_clouds (:184-261) are point-clo
 outside the per-frame hot path (SURVEY section 2, row 4): kept as plain numpy with the reference's
 semantics so that callers keep working.
 """
-from typing import List, Tuple
+from typing import List, NamedTuple, Tuple
 
 import numpy as np
 
@@ -83,3 +83,38 @@ class Reconstructor:
         """:240-261."""
         valid = [c for c in (clouds or []) if len(c) > 0]
         return np.vstack(valid) if valid else np.array([])
+
+
+class LaserPlaneFit(NamedTuple):
+    """Result of fit_laser_plane."""
+    plane: np.ndarray        # (4,) float64 a, b, c, d: unit normal, d >= 0 (Reconstructor's laser_plane)
+    inlier_mask: np.ndarray  # (n,) bool: the points within `threshold` of `plane`
+    inliers: int
+    rms: float               # sqrt(mean squared residual) over the inliers, metres
+    spread: float            # sqrt(eig[1] / eig[2]) of the inliers' covariance: ~0 for points along one line
+    hypothesis: int          # the winning RANSAC hypothesis and its inlier count
+    hypothesis_inliers: int
+
+
+def fit_laser_plane(points, threshold: float = 0.005, hypotheses: int = 1024, seed: int = 0, device=0) -> LaserPlaneFit:
+    """The laser plane a x + b y + c z + d = 0 through 3D laser points (n x 3, metres, in the rectified left camera's
+    frame), robust to outliers: RANSAC with `hypotheses` planes through point triples drawn from `seed`, then
+    least-squares refits on the points within `threshold` metres (l3d_fit_plane, on the GPU).
+
+    Raises ValueError when the points do not determine a usable plane: when they lie close to one line (the laser line
+    recorded at one distance, on one flat surface) or when the plane passes through the camera's optical centre, where
+    no laser pixel can be triangulated."""
+    r = N.default_context(device).fit_plane(points, threshold, hypotheses, seed)
+    eig = r["eig"]
+    spread = float(np.sqrt(max(eig[1], 0.0) / eig[2])) if eig[2] > 0 else 0.0
+    if not spread >= 0.01:
+        raise ValueError("the laser points are nearly collinear (spread %.3g < 0.01): they do not determine a plane. Record "
+                         "the laser line on surfaces at several distances from the camera, e.g. a board moved through the "
+                         "working range, so that the line sweeps across the laser plane" % spread)
+    plane = r["plane"]
+    if abs(plane[3]) < 1e-6:
+        raise ValueError("the fitted laser plane passes through the camera's optical centre (|d| = %.3g m < 1e-6 m): no laser "
+                         "pixel can be triangulated against it. The laser must be mounted off the camera's centre"
+                         % abs(plane[3]))
+    return LaserPlaneFit(plane, r["inlier_mask"], r["inliers"], r["rms"], spread, r["hypothesis"],
+                         r["hypothesis_inliers"])

@@ -1,5 +1,6 @@
 // api.cu -- the C ABI of include/l3d.h: context, host<->device marshalling, single-frame calls (the frame pipeline's
 // entry points are in pipeline.cu).
+#include <cmath>
 #include <stdexcept>
 
 #include <nvtx3/nvToolsExt.h>
@@ -384,6 +385,26 @@ int l3d_voxel_downsample(l3d_ctx* ctx, const double* points, int n, double voxel
 int l3d_statistical_outlier_removal(l3d_ctx* ctx, const double* points, int n, int nb_neighbors, double std_ratio,
                                     double* out, int* n_out) {
     return cloud_op(ctx, points, n, out, n_out, 1, std_ratio, nb_neighbors, 0);
+}
+
+int l3d_fit_plane(l3d_ctx* ctx, const double* xyz, int n, const l3d_plane_fit_params* p, l3d_plane_fit_result* out,
+                  uint8_t* inlier_mask) {
+    API_BEGIN(ctx)
+    NEED(ctx, xyz && p && out, "plane fit: points, parameters and result are required");
+    NEED(ctx, n >= 3, "plane fit: n >= 3 points");
+    NEED(ctx, std::isfinite(p->threshold) && p->threshold > 0.0, "plane fit: threshold must be finite and > 0");
+    NEED(ctx, p->hypotheses >= 1 && p->hypotheses <= (1 << 20), "plane fit: hypotheses in [1, 2^20]");
+    memset(out, 0, sizeof(*out));
+    CK(ctx, cudaSetDevice(ctx->device));
+    Lane& L = ctx->lane;
+    double* dp = L.get<double>(S_RC_XY, (size_t)n * 3);
+    RC(h2d(ctx, dp, xyz, (size_t)n * 24));
+    const uint8_t* mask_dev = nullptr;
+    RC(dev_fit_plane(L, dp, n, *p, out, &mask_dev));
+    if (inlier_mask) RC(d2h(ctx, inlier_mask, mask_dev, (size_t)n));
+    RC(finish(ctx));
+    return L3D_OK;
+    API_END(ctx)
 }
 
 int l3d_init_undistort_rectify_map(l3d_ctx* ctx, const double* K, const double* dist, int ndist, const double* iR,

@@ -156,6 +156,9 @@ int dev_sgbm_vwave(Lane& L, const int16_t* const* C, int16_t* const* S, int njob
                    int P2, int dir, const VGroupWta* wta);
 int dev_voxel_downsample(Lane& L, const double* pts, int n, double voxel, int f32, double* out, int* nvox_host);
 int dev_outlier_removal(Lane& L, const double* pts, int n, int nb_neighbors, double std_ratio, double* out, int* nout_host);
+// RANSAC + least-squares laser-plane fit of n device points (planefit.cu); *mask_dev: the result's inlier mask (device)
+int dev_fit_plane(Lane& L, const double* pts, int n, const l3d_plane_fit_params& p, l3d_plane_fit_result* res,
+                  const uint8_t** mask_dev);
 int dev_bm(Lane& L, const l3d_bm_params& p, const uint8_t* left, const uint8_t* right, int W, int H, int16_t* disp);
 int dev_median3(Lane& L, const int16_t* src, int W, int H, int16_t* dst);
 int dev_speckles(Lane& L, int16_t* img, int W, int H, int newVal, int maxSize, int maxDiff);

@@ -41,6 +41,53 @@ def stereo_pair(W, H, D, seed=0, laser=True):
     return np.rint(left).astype(np.uint8), np.rint(right).astype(np.uint8)
 
 
+def plane_stripe_pair(W, H, D, plane, scale=1.0, seed=0, baseline=0.06):
+    """A pair whose laser stripe lies on `plane` (a x + b y + c z + d = 0 in the left camera frame of
+    camera_model(W, H, baseline)), on the scene of disparity scale * disparity_field(W, H, D).
+    Returns (left_bgr, right_bgr, centres): centres[y] is the true left-view stripe centre of row y (float64; NaN where
+    the plane does not cross the row), found by bisection on the analytic disparity field; the right view's stripe is
+    painted at x - d(x, y)."""
+    rng = np.random.default_rng(seed)
+    pad = int(D * 1.5) + 16
+    tex = rng.integers(0, 256, (H, W + 2 * pad, 3)).astype(np.float32)
+    tex = cv2.GaussianBlur(tex, (0, 0), 1.5)
+    tex = np.clip((tex - 128.0) * 2.2 + 110.0, 0, 200)
+    di = np.rint(scale * disparity_field(W, H, D)).astype(np.int64)
+    xs = np.arange(W)[None, :]
+    ys = np.arange(H)[:, None]
+    left = tex[ys, xs + pad].copy()
+    right = tex[ys, xs + pad + di].copy()
+    f = 0.8 * W
+    pl = np.asarray(plane, np.float64)
+    y = np.arange(H, dtype=np.float64)
+
+    def disp(x):
+        return scale * (0.35 * D + 0.20 * D * np.sin(6 * x / W) * np.cos(4 * y / H))
+
+    def g(x):  # the plane's residual at the scene point seen at (x, y), every row at once
+        Z = f * baseline / disp(x)
+        return pl[0] * (x - W / 2.0) * Z / f + pl[1] * (y - H / 2.0) * Z / f + pl[2] * Z + pl[3]
+
+    lo, hi = np.zeros(H), np.full(H, W - 1.0)
+    crosses = g(lo) * g(hi) <= 0
+    for _ in range(60):
+        m = 0.5 * (lo + hi)
+        left_half = g(lo) * g(m) <= 0
+        hi = np.where(left_half, m, hi)
+        lo = np.where(left_half, lo, m)
+    centres = np.where(crosses, 0.5 * (lo + hi), np.nan)
+    colour = np.array([140.0, 255.0, 140.0], np.float32)
+
+    def paint(img, centre):
+        c = np.where(np.isnan(centre), -1e9, centre)
+        a = np.clip(3.0 * np.exp(-(xs - c[:, None]) ** 2 / (2 * 2.5 ** 2)), 0, 1)[..., None]
+        return img * (1 - a) + colour * a
+
+    left = paint(left, centres)
+    right = paint(right, centres - disp(np.where(crosses, centres, 0.0)))
+    return np.rint(left).astype(np.uint8), np.rint(right).astype(np.uint8), centres
+
+
 def camera_model(W, H, baseline=0.06):
     """K (3x3) and Q (4x4) of the synthetic rig: f = 0.8 W, principal point at the centre."""
     f = 0.8 * W

@@ -17,7 +17,8 @@ from . import pipeline as _pl
 from .camera.single_usb_stereo_camera import SingleUSBStereoCameraManager
 from .config import Config
 from .core.laser_extractor import FastStegerExtractor, SimpleLaserExtractor
-from .core.reconstruction import Reconstructor
+from .core.reconstruction import Reconstructor, fit_laser_plane
+from .improved_reconstruction import ImprovedLaserReconstructor
 from .utils.point_cloud import PointCloudProcessor
 
 # Frames per pipeline call of process_frames: about 1 GB of device results at 1280x720.  Measured on one B200 (1 000 W),
@@ -135,14 +136,16 @@ class LaserReconstructionSystem:
                 self.point_cloud.extend(points_3d.tolist())
 
     # ---- batched, device-resident form ---------------------------------------------------------
-    def _pipeline(self, lanes, cap=None):
+    def _pipeline(self, lanes, cap=None, recon=None):
+        """The frame pipeline for this system's camera and extractor, kept while its configuration holds.  recon: the
+        per-frame reconstruction (N.ReconParams); None is the reference's reconstruct_from_depth."""
         cam = self.camera
         W, H = cam.single_width, cam.single_height
         dcfg = cam._depth_config()
         simple = isinstance(self.laser_extractor, SimpleLaserExtractor)
         ex = self.laser_extractor
         cap = max(H, 20000, int(cap or 0))
-        key = (W, H, lanes, simple, bytes(dcfg), cap)
+        key = (W, H, lanes, simple, bytes(dcfg), cap, None if recon is None else bytes(recon))
         if self._pipe is not None and self._pipe_key == key:
             return self._pipe
         if self._pipe is not None:
@@ -151,11 +154,12 @@ class LaserReconstructionSystem:
             pc = _pl.make_pipeline_config(W, H, dcfg.left.numDisparities, dcfg.left.blockSize, dcfg.left.mode, None,
                                           self.reconstructor.K, extractor=N.EXTRACT_SIMPLE, lanes=lanes, max_points=cap,
                                           bright_thr=int(ex.brightness_threshold), hsv_lo=tuple(int(v) for v in ex.hsv_lower),
-                                          hsv_hi=tuple(int(v) for v in ex.hsv_upper), min_area=float(ex.min_area))
+                                          hsv_hi=tuple(int(v) for v in ex.hsv_upper), min_area=float(ex.min_area),
+                                          recon=recon)
         else:
             pc = _pl.make_pipeline_config(W, H, dcfg.left.numDisparities, dcfg.left.blockSize, dcfg.left.mode, None,
                                           self.reconstructor.K, extractor=N.STEGER_FAST, lanes=lanes, max_points=cap,
-                                          sigma=float(ex.sigma), bright_thr=int(ex.brightness_threshold))
+                                          sigma=float(ex.sigma), bright_thr=int(ex.brightness_threshold), recon=recon)
         pc.depth = dcfg  # exactly the camera's matcher / WLS / Q configuration
         maps = None
         if dcfg.use_maps:
@@ -175,34 +179,44 @@ class LaserReconstructionSystem:
         split on the device.  Frames run in chunks of CHUNK_FRAMES, so device memory (about 9 MB per frame at
         1280x720) and the host copy a list is stacked into stay bounded whatever the recording's length."""
         out = []
+        for run in self._chunk_runs(frames, lefts, rights):
+            fp, n = self._run_chunk(run, lambda cap: self._pipeline(lanes, cap))
+            self._take_chunk(fp, n, want_images, out)
+        return out
+
+    def _chunk_runs(self, frames, lefts, rights):
+        """One pipeline call `run(fp)` per chunk of CHUNK_FRAMES frames of the recording: captures or split views."""
         if frames is not None:
             split = 0 if self.camera.split_mode == 'horizontal' else 1
             for chunk in _chunks(frames, CHUNK_FRAMES):
                 chunk = np.ascontiguousarray(chunk, np.uint8)  # no copy for a slice of a C-contiguous uint8 array
-                self._process_chunk(lanes, want_images, out, lambda fp: fp.run_captures_host(chunk, split))
-            return out
+                yield lambda fp, chunk=chunk: fp.run_captures_host(chunk, split)
+            return
         lefts = np.ascontiguousarray(lefts, np.uint8)
         rights = np.ascontiguousarray(rights, np.uint8)
         for c0 in range(0, lefts.shape[0], CHUNK_FRAMES):
             l, r = lefts[c0:c0 + CHUNK_FRAMES], rights[c0:c0 + CHUNK_FRAMES]
-            self._process_chunk(lanes, want_images, out, lambda fp: fp.run_host(l, r))
-        return out
+            yield lambda fp, l=l, r=r: fp.run_host(l, r)
 
-    def _process_chunk(self, lanes, want_images, out, run):
-        """One pipeline call (`run(fp)`) over a chunk of frames; its frames' results are appended to `out` and their
-        points to `self.point_cloud` only once the chunk has run with room for all of its points."""
-        fp = self._pipeline(lanes, self._pipe_cap)
+    def _run_chunk(self, run, pipeline):
+        """One pipeline call `run(fp)` over a chunk of frames on `pipeline(cap)`, the pipeline with point capacity cap,
+        run again on a larger one if a frame found more points than it holds.  -> (fp, frames run)"""
+        fp = pipeline(self._pipe_cap)
         n = len(run(fp))
         if fp.points_needed > fp.cfg.max_points:
             # a frame found more laser points than the pipeline's point lists hold (FastSteger emits one per bright
             # pixel: a saturated patch can exceed any fixed bound): nothing may be dropped silently -- the single-frame
             # calls grow their buffers too -- so the pipeline is rebuilt with room for them and the chunk runs again
             self._pipe_cap = min(fp.cfg.W * fp.cfg.H, 2 * fp.points_needed)
-            fp = self._pipeline(lanes, self._pipe_cap)
+            fp = pipeline(self._pipe_cap)
             run(fp)
             if fp.points_needed > fp.cfg.max_points:
-                raise N.L3DError("process_frames: %d laser points in one frame exceed the point list capacity %d"
+                raise N.L3DError("%d laser points in one frame exceed the frame pipeline's point list capacity %d"
                                  % (fp.points_needed, fp.cfg.max_points))
+        return fp, n
+
+    def _take_chunk(self, fp, n, want_images, out):
+        """The results of a chunk's n frames appended to `out`, their valid 3D points to `self.point_cloud`."""
         # np.float64 pairs (Simple) / np.float32 pairs (Steger), as the reference's extractors give them
         to_list = N.points_to_list_f64 if fp.cfg.extractor == N.EXTRACT_SIMPLE else N.points_to_list_f32
         for i in range(n):
@@ -213,6 +227,48 @@ class LaserReconstructionSystem:
                 self.point_cloud.extend(p3.tolist())
             self.frame_count += 1
             out.append(fp.fetch_images(i) + (pts2,) if want_images else (None, None, pts2))
+
+    def calibrate_laser_plane(self, frames=None, lefts=None, rights=None, threshold=None, hypotheses=1024, seed=0,
+                              window=3, min_disparity=1.0, lanes=8):
+        """Measure the laser plane with the stereo rig and make it this system's plane.
+
+        Takes a recording as `process_frames` does (`frames` = captures, or `lefts` / `rights` = split views) in which
+        the laser line falls on surfaces at several distances.  Every frame runs through the frame pipeline with the
+        camera's own depth configuration and this system's extractor, and its laser points become metric 3D points from
+        the disparity (ImprovedLaserReconstructor.reconstruct_with_interpolation: median of the valid disparities in a
+        `window` x `window` neighbourhood, at least `min_disparity`).  `fit_laser_plane(points, threshold, hypotheses,
+        seed)` fits the plane through all of them.  The plane becomes `self.reconstructor.laser_plane` and this system's
+        `config.LASER_PLANE_COEFFICIENTS`; the point cloud and the frame count are left alone.  -> LaserPlaneFit
+
+        `threshold` (metres) None: 5 mm, or 10 mm when the camera runs the WLS filter.  The filtered disparity is noisier
+        at the laser line (on synthetic recordings its 10th-90th percentile error spans about 1.0 px against 0.6 px
+        without the filter), which beyond about 1 m is more than 5 mm of depth noise.  A 5 mm threshold then keeps the
+        near frames and only those far points that err towards the current plane, and that selection tilts the normal
+        (0.49 deg against 0.2 deg with 10 mm on the recording of tests/test_gpu_laser_plane.py).
+
+        Raises ValueError without a calibrated camera (no Q), when fewer than 3 laser points were found and when the
+        points do not determine a plane."""
+        cam = self.camera
+        if cam is None or getattr(cam, "Q", None) is None:
+            raise ValueError("calibrate_laser_plane needs a stereo-calibrated camera (its Q matrix): load the camera's "
+                             "calibration file before measuring the laser plane")
+        recon = ImprovedLaserReconstructor(cam.Q, device=cam.device, verbose=False).recon_params(
+            N.RECON_DISPARITY_MEDIAN, min_disparity, window)
+        clouds = []
+        for run in self._chunk_runs(frames, lefts, rights):
+            fp, n = self._run_chunk(run, lambda cap: self._pipeline(lanes, cap, recon))
+            clouds += [fp.fetch_points(i) for i in range(n)]
+        points = np.concatenate(clouds) if clouds else np.empty((0, 3))
+        if len(points) < 3:
+            raise ValueError("calibrate_laser_plane found %d laser point(s) with a valid disparity in the recording, a "
+                             "plane needs 3 or more: the laser line was not detected. Check that it is visible in both "
+                             "views and that the extractor's colour and brightness settings match it" % len(points))
+        if threshold is None:
+            threshold = 0.01 if cam._depth_config().use_wls else 0.005
+        fit = fit_laser_plane(points, threshold, hypotheses, seed, device=cam.device)
+        self.reconstructor.laser_plane = fit.plane.copy()
+        self.config.LASER_PLANE_COEFFICIENTS = fit.plane.copy()  # this instance's setting; Config keeps the reference's
+        return fit
 
     # ---- reference :190-232 ---------------------------------------------------------------------
     def save_point_cloud(self, filename=None):
