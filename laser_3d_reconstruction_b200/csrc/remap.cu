@@ -9,12 +9,19 @@
 
 namespace l3d {
 
-// CV_32FC1 maps -> {ix | iy<<16 (int16 each), ax | ay<<8}; rint = round-half-even like cvRound
+// cvRound(v * 32): round-half-even; a non-finite product becomes INT_MIN as x86's cvtss2si makes it, so a NaN or
+// infinite map entry saturates to tap -32768 and samples the constant border (cvt.rni would turn NaN into 0, pixel 0)
+__device__ __forceinline__ int map_fixed(float v) {
+    const float s = __fmul_rn(v, 32.0f);
+    return isfinite(s) ? __float2int_rn(s) : INT_MIN;
+}
+
+// CV_32FC1 maps -> {ix | iy<<16 (int16 each), ax | ay<<8}
 __global__ void build_rectmap_kernel(const float* __restrict__ mx, const float* __restrict__ my, int n, int2* __restrict__ out) {
     int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    int sx = __float2int_rn(__fmul_rn(mx[i], 32.0f));
-    int sy = __float2int_rn(__fmul_rn(my[i], 32.0f));
+    int sx = map_fixed(mx[i]);
+    int sy = map_fixed(my[i]);
     int ix = min(max(sx >> 5, -32768), 32767), iy = min(max(sy >> 5, -32768), 32767);
     int2 o;
     o.x = (ix & 0xffff) | (iy << 16);

@@ -42,6 +42,33 @@ def test_remap(case):
     assert np.array_equal(cref.remap_bilinear(src, mx, my), cv2.remap(src, mx, my, cv2.INTER_LINEAR))
 
 
+@pytest.mark.parametrize("axis", ["x", "y", "both"])
+def test_remap_nonfinite_map_entries_sample_the_border(axis):
+    """cv2.remap(INTER_LINEAR) rounds a map entry times 32 with cvRound, which gives INT_MIN for NaN, +-inf and values
+    past the int range: the tap saturates to -32768 and the pixel is the constant border 0.  Entries of +-1e6 land
+    outside any image too.  build_rectmap_kernel (csrc/remap.cu) follows this rule; a cv2 that changes it fails here."""
+    rng = np.random.default_rng(17)
+    H, W = 23, 37
+    src = rng.integers(1, 256, (H, W, 3), dtype=np.uint8)  # no zero pixel: the border is the only source of 0
+    mx = (rng.random((H, W)) * (W - 1)).astype(np.float32)
+    my = (rng.random((H, W)) * (H - 1)).astype(np.float32)
+    inside = cv2.remap(src, mx, my, cv2.INTER_LINEAR)
+    assert inside.all()
+    bad = np.zeros((H, W), bool)
+    for k, v in enumerate((np.nan, np.inf, -np.inf, 3e9, -3e9, 1e6, -1e6)):
+        sel = np.zeros((H, W), bool)
+        sel.ravel()[rng.choice(H * W, 12, replace=False)] = True
+        sel &= ~bad
+        if axis in ("x", "both"):
+            mx[sel] = v
+        if axis in ("y", "both"):
+            my[sel] = v
+        bad |= sel
+    out = cv2.remap(src, mx, my, cv2.INTER_LINEAR)
+    assert (out[bad] == 0).all()
+    assert np.array_equal(out[~bad], inside[~bad])
+
+
 SGBM_CASES = [
     # (W, H, D, bs, minD-kind, params-kind, quant)
     (96, 48, 16, 3, "zero", "base", 0), (130, 50, 32, 5, "zero", "base", 16), (130, 50, 32, 5, "right", "mut", 16),
