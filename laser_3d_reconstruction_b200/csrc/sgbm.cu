@@ -10,10 +10,9 @@
 //
 // Kernels:
 //   sgbm_prefilter_kernel     x-Sobel clip + half-pixel min/max, as pixel-pair operand entries (2 planes x 16 B / pixel)
-//   sgbm_cost_dual_kernel     Birchfield-Tomasi pixel cost -> blockSize^2 box sum -> C (+P2), single-segment volumes at
-//                             block 5 / D 64, block 9 / D 128, block 11 / D 256 (one or both matchers of a frame)
-//   sgbm_cost_warp_kernel     the warp-decoupled single-volume form: SGBM_3WAY's striped volumes at block 5 / D 64 and
-//                             block 9 / D 128
+//   sgbm_cost_dual_kernel     Birchfield-Tomasi pixel cost -> blockSize^2 box sum -> C (+P2) at block 5 / D 64,
+//                             block 9 / D 128, block 11 / D 256: one volume (SGBM_3WAY's striped ones too, except at
+//                             block 11 / D 256) or both matchers' single-segment volumes of a frame
 //   sgbm_cost_kernel          the block-synchronous form: every other geometry, SGBM_3WAY's at block 11 / D 256 among them
 //   sgbm_scan_hpair_kernel    both horizontal paths of a row in one CTA
 //   sgbm_scan_kernel          one SGM path direction per launch, one warp per scan line, path state in registers,

@@ -6,16 +6,23 @@
 // Kernels:
 //   sgbm_prefilter_kernel     x-Sobel clip + half-pixel min/max, as pixel-pair operand entries (2 planes x 16 B / pixel)
 //   sgbm_cost_dual_kernel     Birchfield-Tomasi pixel cost -> blockSize^2 box sum -> C (+P2) of one or both matchers of a
-//                             frame: single-segment volumes at block 5 / D 64, block 9 / D 128, block 11 / D 256
-//   sgbm_cost_warp_kernel     the same sums for one volume, disparity pairs split over the warps, warp-private cost strips
-//                             and row-sum rings, TMA operand ring, no block barrier: SGBM_3WAY's striped volumes at
-//                             block 5 / D 64 and block 9 / D 128 (the dual kernel takes no segments)
+//                             frame at block 5 / D 64, block 9 / D 128, block 11 / D 256 (one volume: single-segment, or
+//                             SGBM_3WAY's striped at block 5 / D 64 and block 9 / D 128; both: single-segment)
 //   sgbm_cost_kernel          the block-synchronous form: every other geometry, SGBM_3WAY's at block 11 / D 256 among them
+#include <map>
+#include <mutex>
+
 #include "sgbm.cuh"
 
 namespace l3d {
 
 constexpr int MAXBAND = 64;
+// One band of a cost pass: volume rows vr0 .. vr0 + rows - 1 from image rows y0 .. y0 + rows - 1.  The vertical window
+// clamps to image rows clo .. H - 1, so the box sum restarts at the top of the band's segment (SGBM_3WAY stripe, else
+// the image).
+struct CostBand {
+    int vr0, y0, rows, clo;
+};
 // ------------------------------------------------------------------------------------------
 // prefilter: per pixel and channel (0 = clipped x-Sobel, 1 = intensity) the Birchfield-Tomasi
 // operands as signed 16-bit values, ready for packed s16x2 DPX arithmetic:
@@ -96,7 +103,7 @@ struct CostArgs {
     int nxg, cpg;  // phase B: column groups per CTA, columns per group
     unsigned* flags;  // bit 0 is set when a cost value reaches 32768 (OpenCV's int16 would wrap there; see make_geom)
     int nbands;
-    int band_vr0[MAXBAND], band_y0[MAXBAND], band_rows[MAXBAND], band_clo[MAXBAND], band_chi[MAXBAND];
+    CostBand band[MAXBAND];
 };
 
 constexpr int COST_THREADS = 512;
@@ -141,7 +148,7 @@ __global__ void __launch_bounds__(COST_THREADS, 1) sgbm_cost_kernel(const CostAr
     const int width1 = a.width1, W = a.W;
     const int tid = threadIdx.x;
     const int b = blockIdx.y, x0 = blockIdx.x * TX;
-    const int y0 = a.band_y0[b], rows = a.band_rows[b], clo = a.band_clo[b], chi = a.band_chi[b], vr0 = a.band_vr0[b];
+    const int y0 = a.band[b].y0, rows = a.band[b].rows, clo = a.band[b].clo, chi = a.H - 1, vr0 = a.band[b].vr0;
     const int xa = min(max(x0 - SW2, 0), width1 - 1);
     const int xb = min(max(x0 + TXH - 1 - SW2, 0), width1 - 1);
     const int xr_base = xa + a.minX1 - (a.minD + D - 1);  // lowest right pixel any pair reads
@@ -308,181 +315,26 @@ __global__ void __launch_bounds__(COST_THREADS, 1) sgbm_cost_kernel(const CostAr
 }
 
 // ------------------------------------------------------------------------------------------
-// cost volume, warp-decoupled form (numDisparities 64 / 128, 64-column tiles)
+// cost volume of one matcher, or of BOTH matchers of a frame from one pixel-cost pass, with staged rows
+// (block 5 / D 64, block 9 / D 128, block 11 / D 256)
 // ------------------------------------------------------------------------------------------
-// Same tile / band decomposition and the same arithmetic as sgbm_cost_kernel, but the disparity pairs are split
-// over the 16 warps (DPW = D/32 pairs each) and BOTH phases of a pair stay in one warp: the warp computes the pixel
-// costs of its pairs for all 64 tile columns (lane <-> columns lane and lane + 32), writes them to a private strip
-// of shared memory, and sums them itself (lane <-> pair x group of columns) against a private ring of row sums.
-// There is no block-wide barrier in the row loop: warps only meet at the mbarriers of the operand-table ring
-// (full: TMA bulk copies landed; empty: all 16 warps are done reading a stage) and drift apart by up to
-// CW_NS - 1 rows, so one warp's shared-memory latency is covered by another warp's arithmetic.  The left operands
-// come in with the same bulk copies (contiguous run of the tile's columns; replicate-clamped tile edges index the
-// run with a clamped column).  A warp stores DPW * 4 contiguous bytes per pixel; the 16 warps' pieces of a pixel's
-// vector meet in L2 before they reach HBM.
-constexpr int CW_NS = 4;        // operand-table stages
-constexpr int CW_TXH = 64;      // tile width incl. halo
-constexpr int CW_PDS = 88;      // pixel-cost strip stride per pair (== 24 mod 32: phase B's 32 lanes hit 32 banks)
-
-static size_t cost_warp_smem(int D, int bs) {
-    const int D2 = D / 2, TX = CW_TXH - (bs - 1);
-    return (size_t)CW_NS * (2 * (CW_TXH + D) + 2 * CW_TXH) * 16 + (size_t)D2 * CW_PDS * 4 + (size_t)bs * D2 * TX * 4 + 64;
-}
-
-template <int BS, int DD>
-__global__ void __launch_bounds__(COST_THREADS, 1) sgbm_cost_warp_kernel(const CostArgs a) {
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    constexpr int D = DD, D2 = DD / 2, SW2 = BS / 2, TXH = CW_TXH, TX = TXH - 2 * SW2;
-    constexpr int NW = COST_THREADS / 32, DPW = D2 / NW, NG = 32 / DPW, CPG = (TX + NG - 1) / NG;
-    constexpr int NEMAX = TXH + D;                      // right-operand entries per channel and stage
-    constexpr int STAGE_U4 = 2 * NEMAX + 2 * TXH;       // [R0 | R1 | L0 | L1]
-    static_assert(DPW >= 1 && 32 % DPW == 0 && CPG <= COST_MAXCPG, "tile geometry");
-    const int width1 = a.width1, W = a.W;
-    const int lane = threadIdx.x & 31;
-    const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);
-    const int b = blockIdx.y, x0 = blockIdx.x * TX;
-    const int y0 = a.band_y0[b], rows = a.band_rows[b], clo = a.band_clo[b], chi = a.band_chi[b], vr0 = a.band_vr0[b];
-    const int xa = min(max(x0 - SW2, 0), width1 - 1);
-    const int xb = min(max(x0 + TXH - 1 - SW2, 0), width1 - 1);
-    const int xr_base = xa + a.minX1 - (a.minD + D - 1);
-    const int nE = (xb - xa) + D - 1;
-    const size_t plane = (size_t)W * a.H;
-    // contiguous run of left columns this tile reads: tile columns [lc0, lc1) hold image columns x0 - SW2 + c unclamped
-    const int lc0 = max(0, SW2 - x0), lc1 = min(TXH, width1 - (x0 - SW2));
-    uint4* tabs = (uint4*)smem_raw;                                          // [CW_NS][STAGE_U4]
-    uint32_t* pdw = (uint32_t*)(tabs + CW_NS * STAGE_U4) + warp * DPW * CW_PDS;  // this warp's pixel-cost strip [DPW][CW_PDS]
-    uint32_t* ringw = (uint32_t*)(tabs + CW_NS * STAGE_U4) + D2 * CW_PDS + (size_t)warp * BS * DPW * TX;  // [BS][DPW][TX]
-    const uint32_t bars = (uint32_t)__cvta_generic_to_shared((uint32_t*)(tabs + CW_NS * STAGE_U4) + D2 * CW_PDS + (size_t)BS * D2 * TX);
-    // bars + 8 s: full[s], bars + 8 (CW_NS + s): empty[s]
-    const int nk = rows + BS - 1;
-    auto row_of = [&](int k) { return min(max(y0 - SW2 + k, clo), chi); };
-    auto issue_tables = [&](int k) {  // one thread: operand entries of band row k -> stage k % CW_NS
-        const int s = k % CW_NS;
-        const uint32_t bar = bars + 8 * s;
-        const uint32_t rbytes = (uint32_t)nE * 16u, lbytes = (uint32_t)(lc1 - lc0) * 16u;
-        const size_t ro = (size_t)row_of(k) * W;
-        const uint4* rsrc = a.Rdesc + ro + xr_base;
-        const uint4* lsrc = a.Ldesc + ro + (x0 - SW2 + lc0) + a.minX1;
-        uint4* dst = tabs + s * STAGE_U4;
-        cost_mbar_expect_tx(bar, 2 * rbytes + 2 * lbytes);
-        cost_bulk_g2s((uint32_t)__cvta_generic_to_shared(dst), rsrc, rbytes, bar);
-        cost_bulk_g2s((uint32_t)__cvta_generic_to_shared(dst + NEMAX), rsrc + plane, rbytes, bar);
-        cost_bulk_g2s((uint32_t)__cvta_generic_to_shared(dst + 2 * NEMAX + lc0), lsrc, lbytes, bar);
-        cost_bulk_g2s((uint32_t)__cvta_generic_to_shared(dst + 2 * NEMAX + TXH + lc0), lsrc + plane, lbytes, bar);
-    };
-    if (threadIdx.x == 0) {
-        for (int s = 0; s < CW_NS; s++) { cost_mbar_init(bars + 8 * s, 1); cost_mbar_init(bars + 8 * (CW_NS + s), NW); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        for (int k = 0; k < CW_NS - 1 && k < nk; k++) issue_tables(k);
-    }
-    __syncthreads();  // barrier init visible; the only block-wide barrier of the kernel
-
-    // phase A role: tile columns lane and lane + 32, pairs dp0 .. dp0 + DPW - 1
-    const int dp0 = warp * DPW;
-    int eoff[2], lcol[2];
-#pragma unroll
-    for (int hh = 0; hh < 2; hh++) {
-        const int c = lane + 32 * hh;
-        const int xc = min(max(x0 - SW2 + c, 0), width1 - 1);
-        eoff[hh] = xc - xa + D - 2 - 2 * dp0;               // entry of pair dp0; pair dp0 + i is 2 i entries lower
-        lcol[hh] = min(max(c, lc0), lc1 - 1);               // replicate clamp inside the staged run
-    }
-    // phase B role
-    const int dpi = lane % DPW, g = lane / DPW;
-    const int cb0 = g * CPG;
-    const int ncb = max(0, min(min(CPG, TX - cb0), width1 - (x0 + cb0)));
-    const uint32_t p2x2 = (uint32_t)a.P2 * 0x10001u;
-    uint32_t crun[CPG];
-#pragma unroll
-    for (int j = 0; j < CPG; j++) crun[j] = p2x2;
-    uint32_t ovf = 0;
-    uint32_t* Cdst = (uint32_t*)(a.C + ((ptrdiff_t)(vr0 - (BS - 1)) * width1 + x0 + cb0) * D) + dp0 + dpi;
-    const size_t crow = (size_t)width1 * D2;
-    const uint32_t* ppb = pdw + dpi * CW_PDS + cb0;
-    uint32_t* rpb = ringw + dpi * TX + cb0;
-    int slot = 0;
-
-    for (int k = 0; k < nk; k++) {
-        const int s = k % CW_NS;
-        // refill duty: rows' tables are issued CW_NS - 1 rows ahead by the warp whose turn it is
-        if (warp == (k & (NW - 1)) && k + CW_NS - 1 < nk) {
-            if (lane == 0) {
-                const int kk = k + CW_NS - 1, sk = kk % CW_NS;  // stage last read for row k - 1
-                if (k >= 1) cost_mbar_wait(bars + 8 * (CW_NS + sk), (uint32_t)(((k - 1) / CW_NS) & 1));
-                issue_tables(kk);
-            }
-            __syncwarp();
-        }
-        cost_mbar_wait(bars + 8 * s, (uint32_t)((k / CW_NS) & 1));
-        const uint4* T0 = tabs + s * STAGE_U4;
-        // ---- phase A
-#pragma unroll
-        for (int hh = 0; hh < 2; hh++) {
-            const uint4 l0 = T0[2 * NEMAX + lcol[hh]], l1 = T0[2 * NEMAX + TXH + lcol[hh]];
-            const uint32_t u0 = __byte_perm(l0.x, l0.x, 0x3232), nu0 = __byte_perm(l0.y, l0.y, 0x3232);
-            const uint32_t ul0 = __byte_perm(l0.z, l0.z, 0x3232), nuh0 = __byte_perm(l0.w, l0.w, 0x3232);
-            const uint32_t u1 = __byte_perm(l1.x, l1.x, 0x3232), nu1 = __byte_perm(l1.y, l1.y, 0x3232);
-            const uint32_t ul1 = __byte_perm(l1.z, l1.z, 0x3232), nuh1 = __byte_perm(l1.w, l1.w, 0x3232);
-            uint4 e0[DPW], e1[DPW];
-#pragma unroll
-            for (int i = 0; i < DPW; i++) { e0[i] = T0[eoff[hh] - 2 * i]; e1[i] = T0[NEMAX + eoff[hh] - 2 * i]; }
-            uint32_t c[DPW];
-#pragma unroll
-            for (int i = 0; i < DPW; i++) {
-                const uint32_t c0 = bt_pair(u0, nu0, ul0, nuh0, e0[i]);
-                const uint32_t c1 = bt_pair(u1, nu1, ul1, nuh1, e1[i]);
-                c[i] = c0 + ((c1 >> 2) & 0x3fff3fffu);
-            }
-#pragma unroll
-            for (int i = 0; i < DPW; i++) pdw[i * CW_PDS + lane + 32 * hh] = c[i];
-        }
-        __syncwarp();  // strip complete; every lane's table reads have returned
-        if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bars + 8 * (CW_NS + s)) : "memory");
-        // ---- phase B
-        if (ncb > 0) {
-            uint32_t* rp = rpb + (size_t)slot * DPW * TX;
-            const bool sub = k >= BS, emit = k >= BS - 1;
-            constexpr int NV = CPG + BS - 1;
-            uint32_t pv[NV], old[CPG], hs[CPG];
-#pragma unroll
-            for (int i = 0; i < NV; i++) pv[i] = ppb[i];
-#pragma unroll
-            for (int j = 0; j < CPG; j++) old[j] = (sub && j < ncb) ? rp[j] : 0u;
-            uint32_t h = 0;
-#pragma unroll
-            for (int i = 0; i < BS; i++) h += pv[i];
-#pragma unroll
-            for (int j = 0; j < CPG; j++) {
-                if (j > 0) h = h + pv[j + BS - 1] - pv[j - 1];
-                hs[j] = h;
-                crun[j] = crun[j] + h - old[j];
-            }
-#pragma unroll
-            for (int j = 0; j < CPG; j++) {
-                if (j < ncb) {
-                    rp[j] = hs[j];
-                    ovf |= crun[j];
-                    if (emit) Cdst[(size_t)j * D2] = crun[j];
-                }
-            }
-        }
-        __syncwarp();  // the strip is rewritten by the next row's phase A
-        Cdst += crow;
-        slot = slot + 1 == BS ? 0 : slot + 1;
-    }
-    if ((ovf & 0x80008000u) && a.flags) atomicOr(a.flags, 1u);
-}
-// ------------------------------------------------------------------------------------------
-// cost volumes of BOTH matchers of a frame from one pixel-cost pass (numDisparities 64 / 128)
-// ------------------------------------------------------------------------------------------
+// Same tile / band decomposition and the same arithmetic as sgbm_cost_kernel, but the disparity pairs are split over the
+// 16 warps (DPW = D/32 pairs each) and BOTH phases of a pair stay in one warp: the warp computes the pixel costs of its
+// pairs for all TXH tile columns (lane <-> columns lane + 32 h), writes them to a private strip of shared memory, and
+// sums them itself (lane <-> pair x group of columns) against a private ring of row sums.  There is no block-wide
+// barrier in the row loop: warps meet at the mbarriers of the operand-table ring (full: TMA bulk copies landed; empty:
+// all 16 warps are done reading a stage) and of the staged rows below, so one warp's shared-memory latency is covered
+// by another warp's arithmetic.  The left operands come in with the same bulk copies (contiguous run of the tile's
+// columns; replicate-clamped tile edges index the run with a clamped column).  Each CTA walks one band of a band table
+// (CostBand): a single-segment volume or the stripes of SGBM_3WAY, whose vertical windows restart at the stripe tops.
+//
 // The right matcher (minDisparity = -(D-1), views swapped: camera/single_usb_stereo_camera.py:277,325) evaluates the
 // same Birchfield-Tomasi pixel costs as the left one -- the BT cost is symmetric in its two pixels -- and the box sum
 // runs along x and y at a fixed disparity, so away from the replicate-clamped borders of the two width1 windows
 //     C_right[y][x'][D-1-k] = C_left[y][x' + k - (D-1)][k]        (x, x' in width1 coordinates, k = 0 .. D-1)
 // holds exactly, for x' in [SW2 + D-1, width1 - SW2) (derivation in DESIGN.md).  So:
-//   role-0 CTAs  compute a tile of the LEFT matcher's volume as sgbm_cost_warp_kernel does (same arithmetic, same
-//                warp-private strips and rings), stage every finished row [column][disparity] in shared memory, and
-//                all 16 warps then write the row out twice: as it is (coalesced 16-byte chunks, whole 256-byte
+//   role-0 CTAs  compute a tile of the LEFT matcher's volume, stage every finished row [column][disparity] in shared
+//                memory, and all 16 warps then write the row out twice: as it is (coalesced 16-byte chunks, whole 256-byte
 //                vectors) into C_left, and sheared into C_right for the columns RA <= x' < RB.  One right-volume word
 //                (disparity indices 2w, 2w+1 of column x') is the high half of the staged word (column A = x' - 2w,
 //                pair D/2-1-w) and the low half of the same pair one column to the left: two LDS + one PRMT.  The
@@ -503,6 +355,7 @@ struct DualArgs {
     int W, H, width1, P2;
     int viewL[2], minD[2], minX1[2];  // role r: which view is its left image, its minDisparity, its minX1
     int ntiles[2], nbands[2];
+    CostBand band[2][MAXBAND];  // role r: bands of every tile
     int stride0;                // role-0 tile origins: t * stride0; role-1 origins: x1[t]
     int x1[CD_MAXT1];
     int emit, RA, RB;           // role-0 tiles also write columns RA <= x' < RB of C[1]
@@ -556,9 +409,7 @@ __global__ void __launch_bounds__(COST_THREADS, 1) sgbm_cost_dual_kernel(const D
     const int nb = a.nbands[role];
     const int tile = cta / nb, b = cta - tile * nb;
     const int x0 = role ? a.x1[tile] : tile * a.stride0;
-    const int br = (a.H + nb - 1) / nb;
-    const int y0 = b * br, rows = min(br, a.H - y0);
-    if (rows <= 0) return;
+    const int y0 = a.band[role][b].y0, rows = a.band[role][b].rows, clo = a.band[role][b].clo, vr0 = a.band[role][b].vr0;
     const int chi = a.H - 1;
     const uint4* __restrict__ Ldesc = a.desc[a.viewL[role]];
     const uint4* __restrict__ Rdesc = a.desc[1 - a.viewL[role]];
@@ -583,7 +434,7 @@ __global__ void __launch_bounds__(COST_THREADS, 1) sgbm_cost_dual_kernel(const D
     // bars + 8 s: full[s]; + 8 (CD_NS + s): empty[s]; + 8 (2 CD_NS + s): row staged[s]; + 8 (2 CD_NS + 2 + s): row written out[s]
     const uint32_t bar_lsf = bars + 8 * (2 * CD_NS), bar_lse = bars + 8 * (2 * CD_NS + 2);
     const int nk = rows + BS - 1;
-    auto row_of = [&](int k) { return min(max(y0 - SW2 + k, 0), chi); };
+    auto row_of = [&](int k) { return min(max(y0 - SW2 + k, clo), chi); };
     auto issue_tables = [&](int k) {
         const int s = k % CD_NS;
         const uint32_t bar = bars + 8 * s;
@@ -634,9 +485,9 @@ __global__ void __launch_bounds__(COST_THREADS, 1) sgbm_cost_dual_kernel(const D
     uint32_t* Cown32 = (uint32_t*)a.C[role];
     uint32_t* Cother32 = (uint32_t*)a.C[1];
 
-    auto write_out = [&](int er) {  // emitted row er of the band (image row y0 + er), staged in Ls[er & 1]
+    auto write_out = [&](int er) {  // emitted row er of the band (volume row vr0 + er), staged in Ls[er & 1]
         const uint32_t* ls = Ls + (er & 1) * TX * CS;
-        const size_t rowbase = (size_t)(y0 + er) * width1;
+        const size_t rowbase = (size_t)(vr0 + er) * width1;
         if (CS % 4 == 0) {
             constexpr int CPC = D2 / 4;                    // 16-byte chunks per column
             for (int q = threadIdx.x; q < ncopy * CPC; q += COST_THREADS) {
@@ -766,77 +617,68 @@ int sgbm_prefilter(Lane& L, const uint8_t* img, int W, int H, int ftzero, uint4*
     return L3D_OK;
 }
 
-// bands: split each segment (SGBM_3WAY stripe, else the image) so that the grid is close to `want` CTAs per x tile
-static void cost_bands(const Geom& g, int H, int want, CostArgs& ca) {
-    int per_seg = std::max(1, std::min(want / g.nseg, MAXBAND / g.nseg));
-    ca.nbands = 0;
+// Splits every segment of g (SGBM_3WAY stripe, else the image) into n bands of ceil(rows / n) rows,
+// n = min(nmax, rows / (2 blockSize)) but at least 1.  Returns the number of bands.
+static int cost_bands(const Geom& g, int nmax, CostBand* band) {
+    int nb = 0;
     for (int s = 0; s < g.nseg; s++) {
-        int rows = g.seg_rows[s];
-        int nb = std::max(1, std::min(per_seg, rows / (2 * g.bs) > 0 ? rows / (2 * g.bs) : 1));
-        int br = cdiv(rows, nb);
-        for (int r0 = 0; r0 < rows; r0 += br) {
-            int i = ca.nbands++;
-            ca.band_vr0[i] = g.seg_vr0[s] + r0;
-            ca.band_y0[i] = g.seg_y0[s] + r0;
-            ca.band_rows[i] = std::min(br, rows - r0);
-            ca.band_clo[i] = g.seg_y0[s];  // the vertical box sum restarts at the segment top
-            ca.band_chi[i] = H - 1;
+        const int rows = g.seg_rows[s];
+        const int br = cdiv(rows, std::max(1, std::min(nmax, rows / (2 * g.bs))));
+        for (int r0 = 0; r0 < rows; r0 += br) band[nb++] = {g.seg_vr0[s] + r0, g.seg_y0[s] + r0, std::min(br, rows - r0), g.seg_y0[s]};
+    }
+    return nb;
+}
+
+// nmax of cost_bands for a grid close to one wave of CTAs (one CTA per SM: the row-sum ring takes most of the shared
+// memory) over xtiles column tiles
+static int cost_wave_bands(const Geom& g, int xtiles) {
+    const int want = std::max(1, NUM_SMS / xtiles);
+    return std::max(1, std::min(want / g.nseg, MAXBAND / g.nseg));
+}
+
+// Band split of a single-segment launch of the staged kernel: nt0 role-0 tiles and nt1 role-1 tiles, every CTA walks
+// (band rows + bs - 1) rows; one CTA per SM.  Picks the bands per tile of both roles that minimise the finish time of
+// a greedy assignment of the CTAs (in launch order: role 0 first) to the SMs.  The result depends on the arguments
+// alone and is computed once per process.
+static void cost_pick_bands(int H, int bs, int nt0, int nt1, int& b0_out, int& b1_out) {
+    static std::mutex mu;
+    static std::map<long long, std::pair<int, int>> cache;
+    const long long key = ((long long)H << 40) | ((long long)bs << 32) | ((long long)nt0 << 8) | nt1;
+    std::lock_guard<std::mutex> lk(mu);
+    auto it = cache.find(key);
+    if (it == cache.end()) {
+        // with role-1 tiles (both matchers' volumes), a role-0 row costs about 1.35 role-1 rows: it also writes the
+        // sheared copy
+        const double w0 = nt1 ? 1.35 : 1.0, w1 = 1.0;
+        const int maxb = std::max(1, std::min(MAXBAND, H / (2 * bs)));
+        double bestt = 1e30;
+        int b0b = 1, b1b = 1;
+        std::vector<double> sm(NUM_SMS);
+        for (int b0 = 1; b0 <= maxb; b0++) {
+            for (int b1 = 1; b1 <= (nt1 ? maxb : 1); b1++) {
+                const double t0 = w0 * (cdiv(H, b0) + bs - 1), t1 = w1 * (cdiv(H, b1) + bs - 1);
+                std::fill(sm.begin(), sm.end(), 0.0);
+                const int n0 = nt0 * b0, n1 = nt1 * b1;
+                if (n0 + n1 > 4096) continue;
+                // CTAs of equal length: fill round-robin onto the earliest-free SM
+                for (int i = 0; i < n0 + n1; i++) {
+                    int k = 0;
+                    for (int q = 1; q < NUM_SMS; q++) if (sm[q] < sm[k]) k = q;
+                    sm[k] += i < n0 ? t0 : t1;
+                }
+                double t = 0;
+                for (double v : sm) t = std::max(t, v);
+                // inside the frame pipeline other kernels fill idle SMs, so total work (halo rows of short bands) counts too
+                t += 0.3 * (n0 * t0 + n1 * t1) / NUM_SMS + 1e-3 * (b0 + b1);
+                if (t < bestt) { bestt = t; b0b = b0; b1b = b1; }
+            }
         }
+        it = cache.emplace(key, std::make_pair(b0b, b1b)).first;
     }
+    b0_out = it->second.first; b1_out = it->second.second;
 }
 
-static int cost_single_staged(Lane& L, const Geom& g, const uint4* dL, const uint4* dR, int16_t* C);
-static bool cost_dual_cfg(int bs, int D);
-
-int sgbm_cost_single(Lane& L, const Geom& g, const uint4* dL, const uint4* dR, int16_t* C) {
-    const int W = g.W, H = g.H;
-    CostArgs ca;
-    ca.Ldesc = dL; ca.Rdesc = dR; ca.C = C;
-    ca.W = W; ca.H = H; ca.minD = g.minD; ca.D = g.D; ca.minX1 = g.minX1; ca.width1 = g.width1;
-    ca.SW2 = g.SW2; ca.bs = g.bs; ca.P2 = g.P2; ca.flags = L.flags;
-    const int D2 = g.D / 2;
-    auto cost_smem = [&](int txh) {
-        int tx = txh - 2 * g.SW2;
-        return (size_t)2 * 2 * (txh + g.D) * 16 + (size_t)2 * D2 * (txh + 1) * 4 + (size_t)g.bs * tx * D2 * 4 + 16;
-    };
-    ca.nxg = std::max(1, COST_THREADS / D2);
-    int TXH = 64;
-    while (TXH > 2 * g.SW2 + 1 &&
-           (cost_smem(TXH) > 200 * 1024 || cdiv(TXH - 2 * g.SW2, ca.nxg) > COST_MAXCPG)) TXH /= 2;
-    L3D_ARG(L, TXH > 2 * g.SW2 && COST_THREADS % TXH == 0 && cost_smem(TXH) <= 200 * 1024 &&
-                   cdiv(TXH - 2 * g.SW2, ca.nxg) <= COST_MAXCPG,
-            "sgbm: blockSize / numDisparities combination exceeds the cost kernel's shared-memory tile");
-    ca.TXH = TXH; ca.TX = TXH - 2 * g.SW2;
-    ca.cpg = cdiv(ca.TX, ca.nxg);
-    size_t smem = cost_smem(TXH);
-    if (g.nseg == 1 && cost_dual_cfg(g.bs, g.D)) return cost_single_staged(L, g, dL, dR, C);
-    // from here on: SGBM_3WAY's striped volumes (nseg > 1) and the geometries the staged kernel is not instantiated for
-    const bool warp_form = (g.D == 128 && g.bs == 9) || (g.D == 64 && g.bs == 5);
-    if (warp_form) {
-        // warp-decoupled form: 64-column tiles
-        ca.TXH = CW_TXH; ca.TX = CW_TXH - 2 * g.SW2;
-        smem = cost_warp_smem(g.D, g.bs);
-    }
-    // the grid is close to one wave of CTAs (one CTA per SM: the row-sum ring takes most of the shared memory)
-    const int xtiles = cdiv(g.width1, ca.TX);
-    cost_bands(g, H, std::max(1, NUM_SMS / xtiles), ca);
-    const int dpa_step = COST_THREADS / TXH;
-    const int nit = (D2 % dpa_step == 0) ? D2 / dpa_step : 0;
-#define COST_CASE(KERN)                                                                                          \
-    {                                                                                                            \
-        L3D_CHECK(L, cudaFuncSetAttribute(KERN, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));       \
-        L3D_LAUNCH(L, KERN, dim3(xtiles, ca.nbands), COST_THREADS, smem, ca);                                    \
-    }
-    // specialised for the configurations of BASELINE.json (c1-c2: D 64 / block 5, c3: D 128 / block 9, c4: D 256 / block 11)
-    if (warp_form && g.D == 128) COST_CASE((sgbm_cost_warp_kernel<9, 128>))
-    else if (warp_form) COST_CASE((sgbm_cost_warp_kernel<5, 64>))
-    else if (nit == 8 && g.bs == 11 && g.D == 256 && TXH == 32) COST_CASE((sgbm_cost_kernel<8, 11, 256, 32>))
-    else COST_CASE((sgbm_cost_kernel<0, 0, 0, 0>))
-#undef COST_CASE
-    return L3D_OK;
-}
-
-// the (blockSize, numDisparities) pairs the dual kernel is instantiated for
+// the (blockSize, numDisparities) pairs the staged kernel is instantiated for
 static bool cost_dual_cfg(int bs, int D) { return (bs == 9 && D == 128) || (bs == 5 && D == 64) || (bs == 11 && D == 256); }
 
 template <int BS, int DD>
@@ -858,54 +700,56 @@ static int launch_cost_dual_any(Lane& L, int bs, int D, const DualArgs& da) {
 
 static int cost_dual_tx(int bs, int D) { return (D > 128 ? 32 : 64) - 2 * (bs / 2); }
 
-// Band split of a launch: nt0 tiles whose CTAs cost w0 per row and nt1 tiles at w1 per row, every CTA walks
-// (band rows + bs - 1) rows; one CTA per SM.  Picks the bands per tile of both roles that minimise the finish time of
-// a greedy assignment of the CTAs (in launch order: role 0 first) to the SMs.
-static void cost_pick_bands(int H, int bs, int nt0, double w0, int nt1, double w1, int& b0_out, int& b1_out) {
-    const int maxb = std::max(1, std::min(64, H / (2 * bs)));
-    double bestt = 1e30;
-    b0_out = b1_out = 1;
-    std::vector<double> sm(NUM_SMS);
-    for (int b0 = 1; b0 <= maxb; b0++) {
-        for (int b1 = 1; b1 <= (nt1 ? maxb : 1); b1++) {
-            const double t0 = w0 * (cdiv(H, b0) + bs - 1), t1 = w1 * (cdiv(H, b1) + bs - 1);
-            std::fill(sm.begin(), sm.end(), 0.0);
-            const int n0 = nt0 * b0, n1 = nt1 * b1;
-            if (n0 + n1 > 4096) continue;
-            // CTAs of equal length: fill round-robin onto the earliest-free SM
-            for (int i = 0; i < n0 + n1; i++) {
-                int k = 0;
-                for (int q = 1; q < NUM_SMS; q++) if (sm[q] < sm[k]) k = q;
-                sm[k] += i < n0 ? t0 : t1;
-            }
-            double t = 0;
-            for (double v : sm) t = std::max(t, v);
-            // inside the frame pipeline other kernels fill idle SMs, so total work (halo rows of short bands) counts too
-            t += 0.3 * (n0 * t0 + n1 * t1) / NUM_SMS + 1e-3 * (b0 + b1);
-            if (t < bestt) { bestt = t; b0_out = b0; b1_out = b1; }
-        }
+int sgbm_cost_single(Lane& L, const Geom& g, const uint4* dL, const uint4* dR, int16_t* C) {
+    // SGBM_3WAY's striped volumes at block 11 / D 256 stay on the block-synchronous kernel's specialisation below: the
+    // staged kernel's cost pass is about 6 % slower there in the frame pipeline (tools/kernel_times.py, 1920x1080, one
+    // B200 at 1000 W)
+    if (cost_dual_cfg(g.bs, g.D) && (g.nseg == 1 || g.D != 256)) {
+        // the staged kernel, role 0 only: nothing is emitted into a second volume
+        DualArgs da = {};
+        da.desc[0] = dL; da.desc[1] = dR; da.C[0] = C;
+        da.W = g.W; da.H = g.H; da.width1 = g.width1; da.P2 = g.P2;
+        da.viewL[0] = 0; da.minD[0] = g.minD; da.minX1[0] = g.minX1;
+        const int TX = cost_dual_tx(g.bs, g.D);
+        da.stride0 = TX; da.ntiles[0] = cdiv(g.width1, TX);
+        int nb = cost_wave_bands(g, da.ntiles[0]), nb1;
+        if (g.nseg == 1) cost_pick_bands(g.H, g.bs, da.ntiles[0], 0, nb, nb1);
+        da.nbands[0] = cost_bands(g, nb, da.band[0]);
+        da.flags = L.flags;
+        return launch_cost_dual_any(L, g.bs, g.D, da);
     }
-}
-
-// one volume through the staged-row kernel (role 0 only, nothing emitted into a second volume)
-static int cost_single_staged(Lane& L, const Geom& g, const uint4* dL, const uint4* dR, int16_t* C) {
-    DualArgs da = {};
-    da.desc[0] = dL; da.desc[1] = dR; da.C[0] = C; da.C[1] = nullptr;
-    da.W = g.W; da.H = g.H; da.width1 = g.width1; da.P2 = g.P2;
-    da.viewL[0] = 0; da.minD[0] = g.minD; da.minX1[0] = g.minX1;
-    const int TX = cost_dual_tx(g.bs, g.D);
-    da.stride0 = TX; da.ntiles[0] = cdiv(g.width1, TX); da.ntiles[1] = 0; da.nbands[1] = 1;
-    static std::map<long long, int> cache;  // (H, bs, tiles) -> bands
-    const long long key = ((long long)g.H << 32) | ((long long)g.bs << 24) | da.ntiles[0];
-    auto it = cache.find(key);
-    if (it == cache.end()) {
-        int b0, b1;
-        cost_pick_bands(g.H, g.bs, da.ntiles[0], 1.0, 0, 0.0, b0, b1);
-        it = cache.emplace(key, b0).first;
+    CostArgs ca;
+    ca.Ldesc = dL; ca.Rdesc = dR; ca.C = C;
+    ca.W = g.W; ca.H = g.H; ca.minD = g.minD; ca.D = g.D; ca.minX1 = g.minX1; ca.width1 = g.width1;
+    ca.SW2 = g.SW2; ca.bs = g.bs; ca.P2 = g.P2; ca.flags = L.flags;
+    const int D2 = g.D / 2;
+    auto cost_smem = [&](int txh) {
+        int tx = txh - 2 * g.SW2;
+        return (size_t)2 * 2 * (txh + g.D) * 16 + (size_t)2 * D2 * (txh + 1) * 4 + (size_t)g.bs * tx * D2 * 4 + 16;
+    };
+    ca.nxg = std::max(1, COST_THREADS / D2);
+    int TXH = 64;
+    while (TXH > 2 * g.SW2 + 1 &&
+           (cost_smem(TXH) > 200 * 1024 || cdiv(TXH - 2 * g.SW2, ca.nxg) > COST_MAXCPG)) TXH /= 2;
+    L3D_ARG(L, TXH > 2 * g.SW2 && COST_THREADS % TXH == 0 && cost_smem(TXH) <= 200 * 1024 &&
+                   cdiv(TXH - 2 * g.SW2, ca.nxg) <= COST_MAXCPG,
+            "sgbm: blockSize / numDisparities combination exceeds the cost kernel's shared-memory tile");
+    ca.TXH = TXH; ca.TX = TXH - 2 * g.SW2;
+    ca.cpg = cdiv(ca.TX, ca.nxg);
+    const int xtiles = cdiv(g.width1, ca.TX);
+    ca.nbands = cost_bands(g, cost_wave_bands(g, xtiles), ca.band);
+    const int dpa_step = COST_THREADS / TXH;
+    const int nit = (D2 % dpa_step == 0) ? D2 / dpa_step : 0;
+#define COST_CASE(KERN)                                                                                          \
+    {                                                                                                            \
+        L3D_CHECK(L, cudaFuncSetAttribute(KERN, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));       \
+        L3D_LAUNCH(L, KERN, dim3(xtiles, ca.nbands), COST_THREADS, cost_smem(TXH), ca);                          \
     }
-    da.nbands[0] = it->second;
-    da.emit = 0; da.RA = da.RB = 0; da.flags = L.flags;
-    return launch_cost_dual_any(L, g.bs, g.D, da);
+    // specialised for SGBM_3WAY at the configuration of c4 (D 256 / block 11)
+    if (nit == 8 && g.bs == 11 && g.D == 256 && TXH == 32) COST_CASE((sgbm_cost_kernel<8, 11, 256, 32>))
+    else COST_CASE((sgbm_cost_kernel<0, 0, 0, 0>))
+#undef COST_CASE
+    return L3D_OK;
 }
 
 bool sgbm_cost_dual_ok(const Geom& gl, const Geom& gr) {
@@ -939,16 +783,10 @@ int sgbm_cost_dual(Lane& L, const Geom& gl, const Geom& gr, const uint4* dLv, co
         da.x1[nt1++] = da.RB;
     }
     da.ntiles[1] = nt1; da.flags = L.flags;
-    // a role-0 row costs about 1.35 role-1 rows (it also writes the sheared copy)
-    static std::map<long long, std::pair<int, int>> cache;  // (H, bs, tiles) -> bands of both roles
-    const long long key = ((long long)H << 40) | ((long long)gl.bs << 32) | ((long long)da.ntiles[0] << 8) | nt1;
-    auto it = cache.find(key);
-    if (it == cache.end()) {
-        int b0, b1;
-        cost_pick_bands(H, gl.bs, da.ntiles[0], 1.35, nt1, 1.0, b0, b1);
-        it = cache.emplace(key, std::make_pair(b0, b1)).first;
-    }
-    da.nbands[0] = it->second.first; da.nbands[1] = it->second.second;
+    int b0, b1;
+    cost_pick_bands(H, gl.bs, da.ntiles[0], nt1, b0, b1);
+    da.nbands[0] = cost_bands(gl, b0, da.band[0]);
+    da.nbands[1] = cost_bands(gr, b1, da.band[1]);
     if (getenv("L3D_DEBUG_CLUSTERS"))
         fprintf(stderr, "[l3d] cost dual: %d x %d + %d x %d CTAs, RA %d RB %d\n", da.ntiles[0], da.nbands[0], nt1, da.nbands[1], da.RA, da.RB);
     return launch_cost_dual_any(L, gl.bs, D, da);

@@ -2,6 +2,7 @@
 reference calls -- and against the oracle restatement for intermediates cv2 never exposes.
 Bit-exact for integer stages; stated tolerances for WLS (unpinned), Steger centres and 3D points."""
 import ctypes as C
+import math
 
 import cv2
 import numpy as np
@@ -327,6 +328,49 @@ def test_sgbm_3way_tiny_images(ctx, bs, H):
             eq(ctx.sgbm_compute(p, lg, rg), want, "3way tiny %s" % ((bs, H, D, uq),))
             disp, raw = ctx.sgbm_compute(p, lg, rg, want_raw=True)
             eq(disp, want, "3way tiny (raw read back) %s" % ((bs, H, D, uq),))
+
+
+def stripes_3way(H, bs):
+    """OpenCV's SGBM_3WAY stripes (make_geom): 4 stripes of ceil(H / 4) rows, each starting `overlap` rows early, clamped
+    at row 0.  -> [(first image row, rows)] in volume-row order."""
+    stripe = -(-H // 4)
+    overlap = bs // 2 + 1 + math.ceil(0.1 * stripe)
+    out = []
+    for s in range(4):
+        y0, y1 = max(s * stripe - overlap, 0), min((s + 1) * stripe, H)
+        if y1 > y0:
+            out.append((y0, y1 - y0))
+    return out
+
+
+@pytest.mark.parametrize("H", [5, 12, 20, 28, 300])
+@pytest.mark.parametrize("bs,D", [(5, 64), (9, 128), (11, 256)])
+def test_sgbm_3way_striped_volumes(ctx, bs, D, H):
+    """SGBM_3WAY at the (blockSize, numDisparities) pairs the cost kernels are specialised for, from images of a few rows
+    (shifted stripe rows) to a few hundred, three or more column tiles wide, in both matcher roles.  The striped cost
+    volume must equal the full-image volume of the oracle wherever a stripe's vertical window is not cut at its top:
+    every row of a stripe that starts at image row 0, and rows y >= y0 + bs // 2 of the others."""
+    W = D + 150
+    lg, rg = gray_pair(W, H, D, 13)
+    _, mut, right = ref_ops.sgbm_param_sets(D, bs, 2)
+    vols = []
+    for kw, a, b in ((mut, lg, rg), (right, rg, lg)):
+        tag = "3way bs%d D%d H%d minD%d" % (bs, D, H, kw["minDisparity"])
+        p = N.SgbmParams(**kw)
+        disp, raw, Cg, _ = ctx.sgbm_compute(p, a, b, want_raw=True, want_volumes=True)
+        eq(disp, cv2.StereoSGBM_create(**kw).compute(a, b), tag + " disp vs cv2")
+        eq(raw, cref.sgbm_compute(a, b, want_raw=True, **kw)[1], tag + " raw")
+        _, oC, _ = cref.sgbm_compute(a, b, want_volumes=True, **dict(kw, mode=1))
+        vr0 = 0
+        for y0, rows in stripes_3way(H, bs):
+            first = 0 if y0 == 0 else min(bs // 2, rows)
+            eq(Cg[vr0 + first:vr0 + rows], oC[y0 + first:y0 + rows], tag + " C volume, stripe from row %d" % y0)
+            vr0 += rows
+        assert vr0 == len(Cg), tag + " volume rows"
+        vols.append(Cg)
+    _, _, Cl, Cr = ctx.sgbm_compute_pair(N.SgbmParams(**mut), N.SgbmParams(**right), lg, rg, want_volumes=True)
+    eq(Cl, vols[0], "3way bs%d D%d H%d pair: left volume" % (bs, D, H))
+    eq(Cr, vols[1], "3way bs%d D%d H%d pair: right volume" % (bs, D, H))
 
 
 @pytest.mark.parametrize("H", [1, 2, 3, 5, 8])
